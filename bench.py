@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the reference path on the host CPU cores
+    python bench.py ... --dump-outputs DIR                   # also writes the last timed step's logits to DIR/logits.npy
 
 A "step" is one forward of PointNet2SemSeg (model/pointnet2.py:131-162: 4 SA + 4 FP + head) over one batch
 of `--batch` synthetic scenes per GPU (weak scaling: per-GPU work is fixed).  One JSON line is printed by
@@ -96,6 +97,18 @@ class ClockSampler:
         if not sm:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": float(max(mx)), "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, logits):
+    """Writes the logits of one step (B, N, C) as out_dir/logits.npy in float32; above DUMP_LIMIT_BYTES only the first
+    scenes that fit are kept (4 KB left for the .npy header)."""
+    logits = np.ascontiguousarray(logits, dtype=np.float32)
+    keep = (DUMP_LIMIT_BYTES - 4096) // logits[0].nbytes
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), logits[:keep])
 
 
 def build_model(device):
@@ -579,14 +592,16 @@ def run_ours(args):
         for i in range(args.steps):
             x = devs[i % n_rot]
             if pipe is not None:
-                pipe.submit(x[:, :3], x[:, 3:])
+                last = pipe.submit(x[:, :3], x[:, 3:])[0]
             else:
-                step(i)
+                last = step(i)
         if pipe is not None:
             pipe.join()
         b.record()
         barrier()
         clocks.end()
+        # a static graph output: copied now, before the legs below replay the same graphs
+        last_logits = last.float().cpu().numpy() if args.dump_outputs else None
         total_ms = a.elapsed_time(b)
         launches = _lib.launch_count() - launches0
         if graphed is not None:
@@ -777,6 +792,8 @@ def run_ours(args):
                                               "conv/BN on all host threads" % (B, cpu_steps)}
         if extra:
             line["extra"] = extra
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_logits)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -796,7 +813,15 @@ def main():
     ap.add_argument("--tc-max-ctas", type=int, default=0, help="developer knob: cap resident CTAs/SM of the tensor-core MLP kernel")
     ap.add_argument("--no-graph", action="store_true", help="launch the forward eagerly instead of replaying a CUDA graph")
     ap.add_argument("--no-extras", action="store_true", help="skip the op rooflines / ref_gpu / cpu_baseline legs (for ncu runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the (B, N, 21) fp32 logits of the headline leg's last step as DIR/logits.npy "
+                         "(rank 0; at most 64 MB: the first scenes of a larger batch); inputs and weights are seeded, so two "
+                         "builds given the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,6 +6,7 @@ nvcc cross-compiles without a GPU; the .so travels with the tree (git-ignored, n
 """
 import hashlib
 import os
+import shutil
 import subprocess
 import sys
 from concurrent.futures import ThreadPoolExecutor
@@ -17,6 +18,11 @@ HEADERS = ["common.cuh", "row_mlp_tile.cuh", os.path.join(ROOT, "include", "pn2_
 OUT = os.path.join(HERE, "libpn2_b200.so")
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-I", os.path.join(ROOT, "include"), "-I", HERE]
+
+
+def _nvcc():
+    """nvcc on PATH, else under CUDA_HOME (default /usr/local/cuda), so a login without the CUDA bin directory builds too."""
+    return shutil.which("nvcc") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc")
 
 
 def _digest(paths):
@@ -41,7 +47,7 @@ def build(force=False, verbose=False):
         want = _digest([src]) + hdr_digest
         if not force and os.path.exists(obj) and os.path.exists(stamp) and open(stamp).read() == want:
             return obj, False
-        cmd = ["nvcc"] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
+        cmd = [_nvcc()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("nvcc failed for %s:\n%s\n%s" % (src, r.stdout, r.stderr))
@@ -55,7 +61,7 @@ def build(force=False, verbose=False):
         results = list(ex.map(compile_one, srcs))
     objs = [o for o, _ in results]
     if force or any(changed for _, changed in results) or not os.path.exists(OUT):
-        subprocess.check_call(["nvcc", "-shared", "-Wno-deprecated-gpu-targets", "-o", OUT] + objs + ["-lcudart"])
+        subprocess.check_call([_nvcc(), "-shared", "-Wno-deprecated-gpu-targets", "-o", OUT] + objs + ["-lcudart"])
     return OUT
 
 

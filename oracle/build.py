@@ -9,10 +9,12 @@
 The reference sources are never copied into this repository; --ref is a no-op when
 /root/reference is absent (the GPU box uses the prebuilt oracle/_ref/ref_cuda.so).
 """
+import hashlib
 import os
 import subprocess
 import sys
 import sysconfig
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF_SRC = "/root/reference/utils/src"
@@ -26,17 +28,33 @@ def _newer(target, deps):
 
 
 def build_oracle(force=False):
-    out_dir = os.path.join(HERE, "_build")
-    os.makedirs(out_dir, exist_ok=True)
+    """Rebuilds only when the source or the flags change (a content stamp, not mtimes, so a copied tree stays valid).
+    When the tree is read-only and holds no current build, the library goes to a fresh temporary directory."""
     src = os.path.join(HERE, "pn2_oracle.c")
-    out = os.path.join(out_dir, "liboracle.so")
-    if not force and _newer(out, [src]):
-        return out
     # -ffp-contract=off: the only fused operations are the explicit fmaf() calls.
     # -mfma so fmaf() is one instruction; x86-64-v3 class hosts only.
-    cmd = ["gcc", "-O2", "-std=c11", "-ffp-contract=off", "-mfma", "-mavx2", "-fopenmp", "-shared", "-fPIC",
-           src, "-o", out, "-lm"]
-    subprocess.check_call(cmd)
+    flags = ["-O2", "-std=c11", "-ffp-contract=off", "-mfma", "-mavx2", "-fopenmp", "-shared", "-fPIC"]
+    with open(src, "rb") as f:
+        h = hashlib.sha256(f.read())
+    h.update(" ".join(flags).encode())
+    want = h.hexdigest()
+    out_dir = os.path.join(HERE, "_build")
+    out = os.path.join(out_dir, "liboracle.so")
+    stamp = out + ".sha"
+    if not force and os.path.exists(out) and os.path.exists(stamp) and open(stamp).read() == want:
+        return out
+    try:
+        os.makedirs(out_dir, exist_ok=True)
+        writable = os.access(out_dir, os.W_OK)
+    except OSError:
+        writable = False
+    if not writable:
+        out_dir = tempfile.mkdtemp(prefix="pn2_oracle_")
+        out = os.path.join(out_dir, "liboracle.so")
+        stamp = out + ".sha"
+    subprocess.check_call(["gcc"] + flags + [src, "-o", out, "-lm"])
+    with open(stamp, "w") as f:
+        f.write(want)
     return out
 
 

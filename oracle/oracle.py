@@ -29,7 +29,7 @@ def lib():
         spec = importlib.util.spec_from_file_location("_oracle_build", os.path.join(_HERE, "build.py"))
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
-        path = mod.build_oracle()  # rebuilds only when pn2_oracle.c is newer than the library
+        path = mod.build_oracle()  # rebuilds only when pn2_oracle.c or its flags changed
         _LIB = ctypes.CDLL(path)
         _LIB.orc_project_point.restype = ctypes.c_int32
         _LIB.orc_opt_n_threads.restype = ctypes.c_int
