@@ -305,6 +305,10 @@ void pn2_debug_set_lift_mode(int mode);
 /* Worker warps per 128-row tile of the tensor-core MLP kernel: 4 (up to 4 CTAs per SM), 8 (two warps per TMEM lane
  * quarter splitting the columns, up to 2 CTAs per SM) or 0 = chosen by launch size (default).  Results are identical. */
 void pn2_debug_set_tc_workers(int n);
+/* What the last pn2_sa_mlp_max_bf16 / pn2_fp_mlp_bf16 call on this thread launched: the kernel build (*name, e.g.
+ * "bf16_x4_sa", "f32_w8_fp"; "" when the call launched nothing), its grid and threads per CTA.  Any pointer may be
+ * NULL.  Returns 1 if that call launched a kernel, else 0.  Recording changes no launch. */
+int pn2_debug_last_tc_launch(const char **name, int *grid, int *threads);
 /* Kernel choice of pn2_three_interpolate: 0 automatic, 1 tiled kernels only, 32 the lane-along-channel kernel wherever it
  * applies (+ 256 / 4096 / 512: 256 / 768 / 1024 threads per CTA instead of 512; + 1024: no stores, + 2048: no row reads --
  * bisect probes, results are then meaningless).  scripts/interp_sweep.py. */

@@ -1320,10 +1320,11 @@ Plan make_plan_capped(const pn2_mlp *mlp, int nblk_cap) {
 int g_tc_max_ctas = 8;  // developer knob (pn2_debug_set_tc_max_ctas)
 int g_tc_workers = 0;   // worker warps per tile: 0 = by launch size, 4, or 8 (pn2_debug_set_tc_workers)
 
+// CTAs of this plan that shared memory and TMEM let reside on one SM.  The developer cap (g_tc_max_ctas) is applied at
+// launch only: make_plan compares these counts, and the packed weight image it describes must not depend on a knob.
 int ctas_per_sm(const Plan &P) {
     int per_sm = (int)((TC_SMEM_LIMIT + 1024) / (P.smem_bytes + 1024));  // + 1 KB per CTA reserved by the system
     if (per_sm > 512 / P.tmem_cols) per_sm = 512 / P.tmem_cols;
-    if (per_sm > g_tc_max_ctas) per_sm = g_tc_max_ctas;
     return per_sm < 1 ? 1 : per_sm;
 }
 
@@ -1384,6 +1385,30 @@ int check_mlp_tc(const char *op, const pn2_mlp *mlp, int c0) {
 long long *take_tc_dbg();
 namespace {
 
+// What the last pn2_*_bf16 call on this thread launched (developer hook pn2_debug_last_tc_launch); name "" = nothing.
+struct TcLaunchRecord {
+    const char *name;
+    int grid, threads;
+};
+thread_local TcLaunchRecord g_tc_last = {"", 0, 0};
+
+const char *tc_build_name(void (*kernel)(TcParams)) {
+    static const struct {
+        void (*fn)(TcParams);
+        const char *name;
+    } builds[] = {
+        {row_mlp_tc_kernel_f32_sa, "f32_sa"},          {row_mlp_tc_kernel_f32_fp, "f32_fp"},
+        {row_mlp_tc_kernel_bf16_sa, "bf16_sa"},        {row_mlp_tc_kernel_bf16_fp, "bf16_fp"},
+        {row_mlp_tc_kernel_bf16_wide_sa, "bf16_wide_sa"}, {row_mlp_tc_kernel_bf16_wide_fp, "bf16_wide_fp"},
+        {row_mlp_tc_kernel_bf16_x4_sa, "bf16_x4_sa"},  {row_mlp_tc_kernel_f32_w8_sa, "f32_w8_sa"},
+        {row_mlp_tc_kernel_f32_w8_fp, "f32_w8_fp"},    {row_mlp_tc_kernel_bf16_w8_sa, "bf16_w8_sa"},
+        {row_mlp_tc_kernel_bf16_w8_fp, "bf16_w8_fp"},
+    };
+    for (const auto &b : builds)
+        if (b.fn == kernel) return b.name;
+    return "?";
+}
+
 int launch_tc(TcParams &p, const Plan &P, const void *packed, long long tiles, cudaStream_t s) {
     p.dbg = take_tc_dbg();
     PN2_REQUIRE(tiles * TC_ROWS <= 2147483647ll, "row_mlp_tc: more than 2^31 rows in one launch");
@@ -1406,6 +1431,7 @@ int launch_tc(TcParams &p, const Plan &P, const void *packed, long long tiles, c
     const bool sa = p.mode == MODE_SA;
     // persistent grid: as many CTAs as can be resident (shared memory, 512 TMEM columns, registers), at most one per tile
     int per_sm = ctas_per_sm(P);
+    if (per_sm > g_tc_max_ctas) per_sm = g_tc_max_ctas;
     // register budget of the bf16-input builds: the SA build fits 80 registers (4 CTAs/SM: sa2 39.3 -> 35.3 us), the FP
     // build (three-row interpolating gather) needs 96 (at 80 it spills 164 bytes: fp1+head 107 -> 115 us)
     if (p.in_bf16 && per_sm > (sa ? 4 : 3)) per_sm = sa ? 4 : 3;
@@ -1436,6 +1462,7 @@ int launch_tc(TcParams &p, const Plan &P, const void *packed, long long tiles, c
     if (grid > tiles) grid = tiles;
     kernel<<<(unsigned)grid, threads, P.smem_bytes, s>>>(p);
     PN2_LAUNCH_OK("row_mlp_tc_kernel");
+    g_tc_last = {tc_build_name(kernel), (int)grid, threads};
     return PN2_OK;
 }
 
@@ -1444,6 +1471,13 @@ int launch_tc(TcParams &p, const Plan &P, const void *packed, long long tiles, c
 
 extern "C" void pn2_debug_set_tc_max_ctas(int n) { pn2::g_tc_max_ctas = n < 1 ? 1 : n; }
 extern "C" void pn2_debug_set_tc_workers(int n) { pn2::g_tc_workers = (n == 8 || n == 4) ? n : 0; }
+extern "C" int pn2_debug_last_tc_launch(const char **name, int *grid, int *threads) {
+    const pn2::TcLaunchRecord &r = pn2::g_tc_last;
+    if (name) *name = r.name;
+    if (grid) *grid = r.grid;
+    if (threads) *threads = r.threads;
+    return r.grid > 0;
+}
 
 extern "C" int pn2_mlp_bf16_supported(const pn2_mlp *mlp) {
     if (!mlp || mlp->num_layers < 1 || mlp->num_layers > PN2_MAX_LAYERS) return 0;
@@ -1479,6 +1513,7 @@ extern "C" int pn2_sa_mlp_max_bf16(int b, int n, int m, int k, int d, const floa
                                    const float *new_xyz, const int32_t *idx, const pn2_mlp *mlp, const void *packed,
                                    float *out, int out_stride, int out_offset, int flags, void *stream) {
     using namespace pn2;
+    g_tc_last = {"", 0, 0};
     PN2_REQUIRE(b >= 0 && n >= 1 && m >= 0 && k >= 1 && d >= 0, "sa_mlp_max_bf16: bad dims b=%d n=%d m=%d k=%d d=%d", b, n, m, k, d);
     if (int st = check_mlp_tc("sa_mlp_max_bf16", mlp, 3 + d)) return st;
     if (b == 0 || m == 0) return PN2_OK;
@@ -1510,6 +1545,7 @@ extern "C" int pn2_fp_mlp_bf16(int b, int n, int m, int d1, int d2, const float 
                                const int32_t *idx, const float *weight, const pn2_mlp *mlp, const void *packed,
                                const int32_t *row_perm, float *out, int flags, void *stream) {
     using namespace pn2;
+    g_tc_last = {"", 0, 0};
     PN2_REQUIRE(b >= 0 && n >= 0 && m >= 1 && d1 >= 0 && d2 >= 1, "fp_mlp_bf16: bad dims b=%d n=%d m=%d d1=%d d2=%d", b, n, m, d1, d2);
     if (int st = check_mlp_tc("fp_mlp_bf16", mlp, d1 + d2)) return st;
     if (b == 0 || n == 0) return PN2_OK;
