@@ -116,6 +116,20 @@ int pn2_lift_views_poses(int b, int n, int v, int c, int h, int w, const float *
                          const float *c2w, const float *cam_corners, const float *intr, float depth_min, float depth_max,
                          float accuracy, int reduce, float *out, int32_t *pix, int32_t *count, void *stream);
 
+/* Backward of pn2_lift_views / pn2_lift_views_poses with respect to feats: the gradient torch autograd gives for the
+ * reference's composition (Projection per view, then the view reduction), deterministic.
+ *   feats (B,V,C,H,W) as given to the forward; pix (B,V,N) int32 as the forward wrote it; grad_out (B,C,N)
+ *   -> grad_feats (B,V,C,H,W), WRITTEN IN FULL (zero where no point contributes; no pre-zeroing).
+ *   PN2_REDUCE_MAX: grad_out[b,c,i] goes to the pixel of the first view (in view order) holding the maximum of channel c,
+ *     invisible views taking part with 0 (torch's max pooling takes a new maximum only on a strict >); dropped when that
+ *     view does not see the point.
+ *   PN2_REDUCE_FIRST: the whole column goes to the first view that sees the point with a column that is not all zero;
+ *     without one, to view V-1 if it sees the point (the reference's fill loop assigns from V-1 last), else dropped.
+ * Contributions to one element are summed in ascending point index in fp32, without atomics: bit-identical from run to
+ * run and under CUDA-graph replay.  Temporary storage comes from the stream-ordered allocator; no host synchronisation. */
+int pn2_lift_views_grad(int b, int n, int v, int c, int h, int w, const float *feats, const int32_t *pix, int reduce,
+                        const float *grad_out, float *grad_feats, void *stream);
+
 /* Best-view selection of the ScanNet loader (data_utils/ScanNetDataLoader.py:87-105 -> utils/projection.py:132-164):
  * number of the n points inside the frustum of each of num_poses cameras, evaluated in fp64 as the reference does.
  * corner2/corner4 (P,3), normals (P,6,3) as for pn2_lift_views; counts (P) int32 must be pre-zeroed. */

@@ -28,6 +28,14 @@ struct Scratch {
     cudaError_t alloc(size_t bytes) { return scratch_alloc(&ptr, bytes, stream); }
 };
 
+// Stable inversion of a key list (scatter_det.cu): keys_in (total) with values in [0, nkeys), pos_in (total) the payload
+// of each key -> pos (total) = the payloads in ascending key order, equal keys in their input order, and seg_start
+// (nkeys + 1): seg_start[k] = first slot of pos whose key is >= k.  One device radix sort; `scratch` holds
+// segment_sort_scratch_bytes(total, nkeys) bytes.  No host synchronisation.
+size_t segment_sort_scratch_bytes(long long total, long long nkeys);
+int segment_sort(long long total, long long nkeys, const uint32_t *keys_in, const int32_t *pos_in, void *scratch, int32_t *seg_start,
+                 int32_t *pos, cudaStream_t s);
+
 #define PN2_REQUIRE(cond, ...)                                             \
     do {                                                                   \
         if (!(cond)) return pn2::set_error(PN2_ERR_INVALID_ARGUMENT, __VA_ARGS__); \

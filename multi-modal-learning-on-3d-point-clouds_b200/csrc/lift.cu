@@ -620,6 +620,160 @@ frustum_count_kernel(int n, int np, const float *__restrict__ points, const floa
     if (threadIdx.x < pc && cnt[threadIdx.x]) atomicAdd(counts + p0 + threadIdx.x, cnt[threadIdx.x]);
 }
 
+// ---- backward of the lifting with respect to the feature maps (pn2_lift_views_grad) --------------------------------
+// The gradient torch autograd computes for the reference's composition: per view Projection (a scatter of the maps onto
+// the points, zero for points that are not lifted; its backward is the transposed scatter), then the view reduction:
+//   max   (F.max_pool1d over the stacked views, invisible views = 0): grad_out[b, c, i] goes to the FIRST view holding the
+//         maximum of channel c (the pooling takes a new maximum only on a strict >), if that view sees the point;
+//   first (in-place fill loop, model/pointnet2multiview.py:93-98): the whole column goes to the first visible view whose
+//         C-channel column is not all zero, else to view V-1 (the loop's last assignment) if it sees the point.
+// Deterministic by construction: the (view, pixel) keys of all contributions are inverted once per call (segment_sort,
+// stable: ascending point index inside a segment), then every output element sums its segment in that order, fp32, with
+// no atomics.  Every element of grad_feats is written.
+//   lift_grad_keys_kernel  key per contribution: cloud * (V*HW + 1) + view * HW + pixel, or the cloud's last bucket (V*HW)
+//                          for a point the view does not see / whose gradient is dropped; payload = the point index.
+//                          max: one key per (view, point); first: one per point (the selected view, nz flags as in the forward)
+//   lift_grad_kernel       one CTA per (cloud, 4 channels), output-stationary: a thread owns (view, pixel) outputs and
+//                          walks their segments.  grad_out rows of the 4 channels are staged point-major (one float4 per
+//                          point) and, for max, the feature slab of all views pixel-major as in lift_gather_pm_kernel, from
+//                          which the per-channel winner of every contribution is recomputed.  Either falls back to global
+//                          reads when it does not fit shared memory (large maps / clouds).  Writes are coalesced along pixels.
+__global__ void __launch_bounds__(256)
+lift_grad_keys_kernel(long long total, int n, int nv, int hw, int first, const int32_t *__restrict__ pix,
+                      const unsigned char *__restrict__ nz, uint32_t *__restrict__ keys, int32_t *__restrict__ pos) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e >= total) return;
+    const int nout = nv * hw;
+    if (first) {  // e = b * n + i
+        const long long b = e / n;
+        const int i = (int)(e - b * n);
+        const int32_t *pb = pix + (size_t)b * nv * n + i;
+        int j = nv - 1;  // no view with a non-zero column: the fill loop's last assignment is view V-1
+        for (int u = 0; u < nv; ++u) {
+            const int p = pb[(size_t)u * n];
+            if (p >= 0 && nz[((size_t)b * nv + u) * hw + p]) {
+                j = u;
+                break;
+            }
+        }
+        const int p = pb[(size_t)j * n];
+        keys[e] = (uint32_t)(b * (nout + 1) + (p >= 0 ? j * hw + p : nout));
+        pos[e] = i;
+    } else {  // e = (b * nv + u) * n + i
+        const long long bu = e / n;
+        const int i = (int)(e - bu * n);
+        const long long b = bu / nv;
+        const int u = (int)(bu - b * nv);
+        const int p = pix[e];
+        keys[e] = (uint32_t)(b * (nout + 1) + (p >= 0 ? u * hw + p : nout));
+        pos[e] = i;
+    }
+}
+
+// four channels of one (view, pixel) / one point, zero beyond the last channel; `stride` floats between channels
+__device__ __forceinline__ float4 load_ch4(const float *__restrict__ src, size_t stride, int cc) {
+    float4 x = make_float4(__ldg(src), 0.f, 0.f, 0.f);
+    if (cc > 1) x.y = __ldg(src + stride);
+    if (cc > 2) x.z = __ldg(src + 2 * stride);
+    if (cc > 3) x.w = __ldg(src + 3 * stride);
+    return x;
+}
+
+__device__ __forceinline__ void cp_async_ch4(float *dst, const float *src, size_t stride, int cc) {
+    cp_async4(dst, src);
+    if (cc > 1) cp_async4(dst + 1, src + stride); else dst[1] = 0.f;
+    if (cc > 2) cp_async4(dst + 2, src + 2 * stride); else dst[2] = 0.f;
+    if (cc > 3) cp_async4(dst + 3, src + 3 * stride); else dst[3] = 0.f;
+}
+
+constexpr int LGR_THREADS = 512;
+
+template <bool kFirst, bool kSlab, bool kGrad>
+__global__ void __launch_bounds__(LGR_THREADS)
+lift_grad_kernel(int n, int nv, int c, int hw, const float *__restrict__ feats, const int32_t *__restrict__ pix,
+                 const int32_t *__restrict__ seg_start, const int32_t *__restrict__ pos, const float *__restrict__ grad_out,
+                 float *__restrict__ grad_feats) {
+    extern __shared__ __align__(16) float4 sm4[];
+    const int b = blockIdx.y;
+    const int c0 = blockIdx.x * 4;
+    const int cc = min(4, c - c0);
+    const int nout = nv * hw;
+    float4 *slab = sm4;                        // [nv][hw], kSlab
+    float4 *gs = sm4 + (kSlab ? nout : 0);     // [n], kGrad
+    const float *fb = feats + ((size_t)b * nv * c + c0) * hw;  // view u, channel c0 + q: fb + (u * c + q) * hw
+    const float *gb = grad_out + ((size_t)b * c + c0) * n;     // channel c0 + q, point i: gb + q * n + i
+    // fills: asynchronous 4-byte copies (every load of the CTA in flight at once), channel rows read coalesced
+    if (kSlab)
+        for (int e = threadIdx.x; e < nout; e += LGR_THREADS) {
+            const int u = e / hw, p = e - u * hw;
+            cp_async_ch4(reinterpret_cast<float *>(slab + e), fb + (size_t)u * c * hw + p, hw, cc);
+        }
+    if (kGrad)
+        for (int i = threadIdx.x; i < n; i += LGR_THREADS) cp_async_ch4(reinterpret_cast<float *>(gs + i), gb + i, n, cc);
+    if (kSlab || kGrad) {
+        asm volatile("cp.async.wait_all;" ::: "memory");
+        __syncthreads();
+    }
+    const int32_t *sb = seg_start + (size_t)b * (nout + 1);
+    const int32_t *pb = pix + (size_t)b * nv * n;
+    for (int o = threadIdx.x; o < nout; o += LGR_THREADS) {
+        const int vv = o / hw, p = o - vv * hw;
+        const int s0 = sb[o], s1 = sb[o + 1];
+        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int s = s0; s < s1; ++s) {
+            const int i = __ldg(pos + s);
+            const float4 g = kGrad ? gs[i] : load_ch4(gb + i, n, cc);
+            if (kFirst) {
+                acc.x = __fadd_rn(acc.x, g.x);
+                acc.y = __fadd_rn(acc.y, g.y);
+                acc.z = __fadd_rn(acc.z, g.z);
+                acc.w = __fadd_rn(acc.w, g.w);
+                continue;
+            }
+            // winner of each channel: the first view holding the maximum, invisible views taking part with 0.  The pixel
+            // indices of all views are loaded before the first use (one dependent round trip per contribution, not V-1).
+            int pu[LV_MAXV];
+#pragma unroll
+            for (int u = 0; u < LV_MAXV; ++u) pu[u] = u < nv && u != vv ? __ldg(pb + (size_t)u * n + i) : p;
+            float4 best = make_float4(0.f, 0.f, 0.f, 0.f);
+            int wx = 0, wy = 0, wz = 0, ww = 0;
+#pragma unroll
+            for (int u = 0; u < LV_MAXV; ++u) {
+                if (u >= nv) break;
+                float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (pu[u] >= 0) x = kSlab ? slab[(size_t)u * hw + pu[u]] : load_ch4(fb + (size_t)u * c * hw + pu[u], hw, cc);
+                if (u == 0) {
+                    best = x;
+                    continue;
+                }
+                if (x.x > best.x) { best.x = x.x; wx = u; }
+                if (x.y > best.y) { best.y = x.y; wy = u; }
+                if (x.z > best.z) { best.z = x.z; wz = u; }
+                if (x.w > best.w) { best.w = x.w; ww = u; }
+            }
+            if (wx == vv) acc.x = __fadd_rn(acc.x, g.x);
+            if (wy == vv) acc.y = __fadd_rn(acc.y, g.y);
+            if (wz == vv) acc.z = __fadd_rn(acc.z, g.z);
+            if (ww == vv) acc.w = __fadd_rn(acc.w, g.w);
+        }
+        float *dst = grad_feats + (((size_t)b * nv + vv) * c + c0) * hw + p;
+        __stcs(dst, acc.x);
+        if (cc > 1) __stcs(dst + hw, acc.y);
+        if (cc > 2) __stcs(dst + 2 * (size_t)hw, acc.z);
+        if (cc > 3) __stcs(dst + 3 * (size_t)hw, acc.w);
+    }
+}
+
+template <bool kFirst, bool kSlab, bool kGrad>
+int launch_lift_grad_t(int b, int n, int nv, int c, int hw, const float *feats, const int32_t *pix, const int32_t *seg_start,
+                       const int32_t *pos, const float *grad_out, float *grad_feats, size_t smem, cudaStream_t s) {
+    PN2_CUDA(cudaFuncSetAttribute(lift_grad_kernel<kFirst, kSlab, kGrad>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    lift_grad_kernel<kFirst, kSlab, kGrad><<<dim3(ceil_div(c, 4), b), LGR_THREADS, smem, s>>>(n, nv, c, hw, feats, pix, seg_start, pos,
+                                                                                            grad_out, grad_feats);
+    PN2_LAUNCH_OK("lift_grad_kernel");
+    return PN2_OK;
+}
+
 }  // namespace
 }  // namespace pn2
 
@@ -737,4 +891,60 @@ extern "C" int pn2_lift_views_poses(int b, int n, int v, int c, int h, int w, co
                                     int32_t *count, void *stream) {
     return lift_views_impl(b, n, v, c, h, w, points, feats, depth, nullptr, nullptr, nullptr, nullptr, c2w, cam_corners, intr, depth_min,
                            depth_max, accuracy, reduce, out, pix, count, stream);
+}
+
+extern "C" int pn2_lift_views_grad(int b, int n, int v, int c, int h, int w, const float *feats, const int32_t *pix, int reduce,
+                                   const float *grad_out, float *grad_feats, void *stream) {
+    using namespace pn2;
+    PN2_REQUIRE(b >= 0 && n >= 0 && v >= 1 && c >= 0 && h >= 1 && w >= 1, "lift_views_grad: bad dims");
+    if (v > LV_MAXV) return set_error(PN2_ERR_UNSUPPORTED, "lift_views_grad: at most %d views per cloud (got %d)", LV_MAXV, v);
+    PN2_REQUIRE(reduce == PN2_REDUCE_MAX || reduce == PN2_REDUCE_FIRST, "lift_views_grad: unknown reduce %d", reduce);
+    if (b == 0 || c == 0) return PN2_OK;
+    PN2_REQUIRE(grad_feats && (n == 0 || (feats && pix && grad_out)), "lift_views_grad: null pointer");
+    PN2_REQUIRE(b <= 65535 && ceil_div(c, 4) <= 65535 && (reduce != PN2_REDUCE_FIRST || b * v <= 65535),
+                "lift_views_grad: b, c/4 and (for reduce first) b*v must be <= 65535");
+    const int hw = h * w;
+    const long long nkeys = (long long)b * ((long long)v * hw + 1);
+    PN2_REQUIRE(nkeys < (1ll << 31) && (long long)b * v * n < (1ll << 31) && (long long)b * v * c * hw < (1ll << 31),
+                "lift_views_grad: more than 2^31 elements");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (n == 0) {  // no point: nothing reaches the maps
+        PN2_CUDA(cudaMemsetAsync(grad_feats, 0, (size_t)b * v * c * hw * sizeof(float), s));
+        return PN2_OK;
+    }
+    const bool first = reduce == PN2_REDUCE_FIRST;
+    const long long total = first ? (long long)b * n : (long long)b * v * n;  // one contribution per point / per (view, point)
+    const size_t key_bytes = ((size_t)total * sizeof(uint32_t) + 255) / 256 * 256;
+    const size_t seg_bytes = ((size_t)(nkeys + 1) * sizeof(int32_t) + 255) / 256 * 256;
+    const size_t nz_bytes = first ? ((size_t)b * v * hw + 255) / 256 * 256 : 0;
+    Scratch scratch_mem(s);  // [keys | payloads in | payloads sorted | segment starts | nz flags | segment_sort scratch]
+    PN2_CUDA(scratch_mem.alloc(3 * key_bytes + seg_bytes + nz_bytes + segment_sort_scratch_bytes(total, nkeys)));
+    unsigned char *cur = (unsigned char *)scratch_mem.ptr;
+    uint32_t *keys = (uint32_t *)cur;
+    int32_t *pos_in = (int32_t *)(cur + key_bytes);
+    int32_t *pos = (int32_t *)(cur + 2 * key_bytes);
+    int32_t *seg_start = (int32_t *)(cur + 3 * key_bytes);
+    unsigned char *nz = cur + 3 * key_bytes + seg_bytes;
+    void *sort_scratch = cur + 3 * key_bytes + seg_bytes + nz_bytes;
+    if (first) {
+        lift_nonzero_kernel<<<dim3(ceil_div(hw, 256), b * v), 256, 0, s>>>(c, hw, feats, nz);
+        PN2_LAUNCH_OK("lift_nonzero_kernel");
+    }
+    lift_grad_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(total, n, v, hw, first ? 1 : 0, pix, nz, keys, pos_in);
+    PN2_LAUNCH_OK("lift_grad_keys_kernel");
+    const int st = segment_sort(total, nkeys, keys, pos_in, sort_scratch, seg_start, pos, s);
+    if (st != PN2_OK) return st;
+    // shared memory: the feature slab of all views (max only), then the grad_out rows, each only while it fits
+    const size_t budget = 200 * 1024;
+    const size_t slab_bytes = !first && (size_t)v * hw * sizeof(float4) <= budget ? (size_t)v * hw * sizeof(float4) : 0;
+    const size_t grad_bytes = slab_bytes + (size_t)n * sizeof(float4) <= budget ? (size_t)n * sizeof(float4) : 0;
+    const size_t smem = slab_bytes + grad_bytes;
+    if (first)
+        return grad_bytes ? launch_lift_grad_t<true, false, true>(b, n, v, c, hw, feats, pix, seg_start, pos, grad_out, grad_feats, smem, s)
+                          : launch_lift_grad_t<true, false, false>(b, n, v, c, hw, feats, pix, seg_start, pos, grad_out, grad_feats, smem, s);
+    if (slab_bytes)
+        return grad_bytes ? launch_lift_grad_t<false, true, true>(b, n, v, c, hw, feats, pix, seg_start, pos, grad_out, grad_feats, smem, s)
+                          : launch_lift_grad_t<false, true, false>(b, n, v, c, hw, feats, pix, seg_start, pos, grad_out, grad_feats, smem, s);
+    return grad_bytes ? launch_lift_grad_t<false, false, true>(b, n, v, c, hw, feats, pix, seg_start, pos, grad_out, grad_feats, smem, s)
+                      : launch_lift_grad_t<false, false, false>(b, n, v, c, hw, feats, pix, seg_start, pos, grad_out, grad_feats, smem, s);
 }

@@ -76,6 +76,34 @@ scatter_det_kernel(int c, int n, long long J, int div, const float *__restrict__
 }
 
 }  // namespace
+
+size_t segment_sort_scratch_bytes(long long total, long long nkeys) {
+    int end_bit = 1;
+    while ((1ll << end_bit) < nkeys) ++end_bit;
+    size_t tmp_bytes = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const uint32_t *)nullptr, (uint32_t *)nullptr, (const int32_t *)nullptr,
+                                    (int32_t *)nullptr, (int)total, 0, end_bit);
+    return ((size_t)total * sizeof(uint32_t) + 255) / 256 * 256 + tmp_bytes;
+}
+
+int segment_sort(long long total, long long nkeys, const uint32_t *keys_in, const int32_t *pos_in, void *scratch, int32_t *seg_start,
+                 int32_t *pos, cudaStream_t s) {
+    int end_bit = 1;
+    while ((1ll << end_bit) < nkeys) ++end_bit;
+    size_t tmp_bytes = 0;
+    PN2_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const uint32_t *)nullptr, (uint32_t *)nullptr, (const int32_t *)nullptr,
+                                             (int32_t *)nullptr, (int)total, 0, end_bit, s));
+    const size_t key_bytes = ((size_t)total * sizeof(uint32_t) + 255) / 256 * 256;
+    uint32_t *keys_out = (uint32_t *)scratch;
+    // LSD radix sort is stable: equal keys keep ascending source position
+    PN2_CUDA(cub::DeviceRadixSort::SortPairs((unsigned char *)scratch + key_bytes, tmp_bytes, keys_in, keys_out, pos_in, pos, (int)total, 0,
+                                             end_bit, s));
+    const int blocks = (int)((total + 255) / 256 < 2048 ? (total + 255) / 256 : 2048);
+    seg_start_kernel<<<blocks, 256, 0, s>>>(total, nkeys, keys_out, seg_start);
+    PN2_LAUNCH_OK("seg_start_kernel");
+    return PN2_OK;
+}
+
 }  // namespace pn2
 
 extern "C" int pn2_inverse_index(int b, int n, long long j, const int32_t *idx, int32_t *seg_start, int32_t *pos, void *stream) {
@@ -90,25 +118,16 @@ extern "C" int pn2_inverse_index(int b, int n, long long j, const int32_t *idx, 
         PN2_CUDA(cudaMemsetAsync(seg_start, 0, (size_t)(nkeys + 1) * sizeof(int32_t), s));
         return PN2_OK;
     }
-    int end_bit = 1;
-    while ((1ll << end_bit) < nkeys) ++end_bit;
-    size_t tmp_bytes = 0;
-    PN2_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const uint32_t *)nullptr, (uint32_t *)nullptr, (const int32_t *)nullptr,
-                                             (int32_t *)nullptr, (int)total, 0, end_bit, s));
     const size_t key_bytes = ((size_t)total * sizeof(uint32_t) + 255) / 256 * 256;
-    Scratch scratch_mem(s);  // [keys in | keys out | positions in | cub temp], released on every return below
-    PN2_CUDA(scratch_mem.alloc(3 * key_bytes + tmp_bytes));
+    Scratch scratch_mem(s);  // [keys in | positions in | segment_sort scratch], released on every return below
+    PN2_CUDA(scratch_mem.alloc(2 * key_bytes + segment_sort_scratch_bytes(total, nkeys)));
     unsigned char *scratch = (unsigned char *)scratch_mem.ptr;
-    uint32_t *keys_in = (uint32_t *)scratch, *keys_out = (uint32_t *)(scratch + key_bytes);
-    int32_t *pos_in = (int32_t *)(scratch + 2 * key_bytes);
+    uint32_t *keys_in = (uint32_t *)scratch;
+    int32_t *pos_in = (int32_t *)(scratch + key_bytes);
     const int blocks = (int)((total + 255) / 256 < 2048 ? (total + 255) / 256 : 2048);
     inv_keys_kernel<<<blocks, 256, 0, s>>>(total, j, n, idx, keys_in, pos_in);
     PN2_LAUNCH_OK("inv_keys_kernel");
-    // LSD radix sort is stable: equal keys keep ascending source position
-    PN2_CUDA(cub::DeviceRadixSort::SortPairs(scratch + 3 * key_bytes, tmp_bytes, keys_in, keys_out, pos_in, pos, (int)total, 0, end_bit, s));
-    seg_start_kernel<<<blocks, 256, 0, s>>>(total, nkeys, keys_out, seg_start);
-    PN2_LAUNCH_OK("seg_start_kernel");
-    return PN2_OK;
+    return segment_sort(total, nkeys, keys_in, pos_in, scratch + 2 * key_bytes, seg_start, pos, s);
 }
 
 extern "C" int pn2_scatter_rows_det(int b, int c, int n, long long j, int div, const float *grad_out, const int32_t *seg_start,

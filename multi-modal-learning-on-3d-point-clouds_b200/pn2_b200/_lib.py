@@ -51,6 +51,7 @@ _SIGNATURES = {
     "pn2_scatter_rows_det": [_c_int, _c_int, _c_int, ctypes.c_longlong, _c_int, _vp, _vp, _vp, _vp, _vp, _vp],
     "pn2_lift_views": [_c_int] * 6 + [_vp] * 7 + [ctypes.POINTER(_c_float)] + [_c_float] * 3 + [_c_int] + [_vp] * 4,
     "pn2_lift_views_poses": [_c_int] * 6 + [_vp] * 4 + [ctypes.POINTER(_c_float)] * 2 + [_c_float] * 3 + [_c_int] + [_vp] * 4,
+    "pn2_lift_views_grad": [_c_int] * 6 + [_vp, _vp, _c_int, _vp, _vp, _vp],
     "pn2_frustum_count": [_c_int, _c_int, _vp, _vp, _vp, _vp, _vp, _vp],
     "pn2_sa_mlp_max": [_c_int] * 5 + [_vp] * 4 + [_c_int, ctypes.POINTER(Pn2Mlp), _vp, _c_int, _c_int, _vp],
     "pn2_fp_mlp": [_c_int] * 5 + [_vp] * 4 + [ctypes.POINTER(Pn2Mlp), _vp, _vp],

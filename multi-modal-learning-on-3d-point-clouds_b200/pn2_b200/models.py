@@ -445,7 +445,9 @@ class _MultiviewStackBase(nn.Module):
         return l1_xyz_geo, l1_points, l2_xyz, l2_points, l2_points_feat
 
     def forward_views(self, xyz, feats, depth, camera_to_world, intrinsic, depth_min, depth_max, image_dims, accuracy):
-        """Lifting + point branch: feats (B, V, 128, H, W) are the 2-D feature maps (ENet output in the reference)."""
+        """Lifting + point branch: feats (B, V, 128, H, W) are the 2-D feature maps (ENet output in the reference).
+        lift_views is differentiable with respect to feats, so a trainable 2-D stage in front (the reference's
+        enet_trainable) receives its gradient through this call."""
         from .projection import lift_views
         points = xyz.permute(0, 2, 1).contiguous()
         image_features = lift_views(points, feats, depth, camera_to_world, intrinsic, depth_min, depth_max, image_dims,

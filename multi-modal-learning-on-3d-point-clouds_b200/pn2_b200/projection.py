@@ -18,6 +18,7 @@ import ctypes
 
 import torch
 from torch.autograd import Function
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from ._lib import ptr
@@ -95,7 +96,18 @@ def lift_views(points, feats, depth, camera_to_world, intrinsic, depth_min, dept
     count (B, V) int32].  view_parameters = (w2c (B,V,4,4), corner2 (B,V,3), corner4 (B,V,3), normals (B,V,6,3)) replaces
     the internal `view_params(camera_to_world, ...)` call, for callers that already hold them (camera_to_world is then
     unused and may be None).
+
+    Differentiable with respect to feats: when grad mode is on and feats.requires_grad, the output carries a grad_fn whose
+    backward (pn2_lift_views_grad) is the gradient of the reference's composition -- Projection per view, then the view
+    reduction -- computed in a fixed order (bit-reproducible).  points, depth and poses get no gradient (the lifting is
+    piecewise constant in them); pix and count are not differentiable.  Without a gradient the call is the plain forward.
     """
+    if feats.requires_grad and torch.is_grad_enabled():
+        def run(f):  # called by the Function with grad mode off: the plain forward below, asked for pix
+            return lift_views(points, f, depth, camera_to_world, intrinsic, depth_min, depth_max, image_dims, accuracy,
+                              reduce=reduce, return_pixels=True, view_parameters=view_parameters)
+        res = _LiftViews.apply(feats, run, reduce)
+        return res if return_pixels else res[0]
     _lib.require_cuda(points, feats, depth)
     B, N, _ = points.shape
     _, V, C, H, W = feats.shape
@@ -131,6 +143,44 @@ def lift_views(points, feats, depth, camera_to_world, intrinsic, depth_min, dept
     if return_pixels:
         return out, pix, count
     return out
+
+
+def lift_views_grad(feats, pix, grad_out, reduce="max"):
+    """Backward of lift_views with respect to the feature maps (pn2_lift_views_grad): feats (B, V, C, H, W) as given to
+    the forward, pix (B, V, N) int32 as it returned them, grad_out (B, C, N) -> grad_feats (B, V, C, H, W).  Every
+    contribution to one element is summed in ascending point index, in fp32: the result is bit-reproducible."""
+    feats, grad_out = _lib.check_f32(feats, "feats"), _lib.check_f32(grad_out, "grad_out")
+    pix = _lib.check_i32(pix, "pix")
+    B, V, C, H, W = feats.shape
+    N = pix.shape[-1]
+    if tuple(pix.shape) != (B, V, N) or tuple(grad_out.shape) != (B, C, N):
+        raise _lib.Pn2Error("lift_views_grad: pix must be (B, V, N) and grad_out (B, C, N) for feats (B, V, C, H, W) = %s"
+                            % (tuple(feats.shape),))
+    grad = torch.empty((B, V, C, H, W), dtype=torch.float32, device=feats.device)
+    red = _lib.REDUCE_FIRST if reduce == "first" else _lib.REDUCE_MAX
+    with torch.cuda.device(feats.device):
+        _lib.call("pn2_lift_views_grad", B, N, V, C, H, W, ptr(feats), ptr(pix), red, ptr(grad_out), ptr(grad),
+                  _lib.stream_ptr(feats.device))
+    return grad
+
+
+class _LiftViews(Function):
+    """lift_views under autograd: the forward always asks the kernels for pix (what the backward needs); the backward is
+    pn2_lift_views_grad.  Only feats is differentiable."""
+
+    @staticmethod
+    def forward(ctx, feats, run, reduce):
+        out, pix, count = run(feats)
+        ctx.save_for_backward(feats, pix)
+        ctx.reduce = reduce
+        ctx.mark_non_differentiable(pix, count)
+        return out, pix, count
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out, *_):
+        feats, pix = ctx.saved_tensors
+        return lift_views_grad(feats, pix, grad_out, ctx.reduce), None, None
 
 
 def frustum_counts(points, camera_to_world, intrinsic, depth_min, depth_max, image_dims, view_parameters=None):
