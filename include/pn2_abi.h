@@ -308,14 +308,13 @@ enum { PN2_FPS_AUTO = 0, PN2_FPS_ONE_CTA = 1, PN2_FPS_CLUSTER = 2 };
 int pn2_set_fps_policy(int policy);
 
 /* ---- developer hooks (tests / profiling; not part of the operator surface) ---- */
-/* Same switch as pn2_set_fps_policy, without the return value (kept for the profiling scripts). */
+/* pn2_set_fps_policy without the return value (bench.py and the profiling scripts): an unknown value is refused and
+ * leaves the policy unchanged. */
 void pn2_debug_set_fps_mode(int mode);
 /* The next pn2_*_bf16 launch on this thread records clock64() phase stamps of CTA 0 into buf (>= 512 int64, device; MMA issuer stamps from [256]). */
 void pn2_debug_set_tc_timestamps(long long *buf);
 /* Caps the resident CTAs per SM of the tensor-core MLP kernel (bench.py --tc-max-ctas; default 8 = no cap). */
 void pn2_debug_set_tc_max_ctas(int n);
-/* Lifting gather kernel: 0 automatic (pixel-major slab when n % 4 == 0), 1 = the channel-major slab kernel only. */
-void pn2_debug_set_lift_mode(int mode);
 /* Worker warps per 128-row tile of the tensor-core MLP kernel: 4 (up to 4 CTAs per SM), 8 (two warps per TMEM lane
  * quarter splitting the columns, up to 2 CTAs per SM) or 0 = chosen by launch size (default).  Results are identical. */
 void pn2_debug_set_tc_workers(int n);
@@ -324,8 +323,8 @@ void pn2_debug_set_tc_workers(int n);
  * NULL.  Returns 1 if that call launched a kernel, else 0.  Recording changes no launch. */
 int pn2_debug_last_tc_launch(const char **name, int *grid, int *threads);
 /* Kernel choice of pn2_three_interpolate: 0 automatic, 1 tiled kernels only, 32 the lane-along-channel kernel wherever it
- * applies (+ 256 / 4096 / 512: 256 / 768 / 1024 threads per CTA instead of 512; + 1024: no stores, + 2048: no row reads --
- * bisect probes, results are then meaningless).  scripts/interp_sweep.py. */
+ * applies with 512 threads per CTA, 32 | 256 the same with 256 threads per CTA; any other value is automatic.
+ * scripts/interp_sweep.py. */
 void pn2_debug_set_interp_mode(int mode);
 
 #ifdef __cplusplus

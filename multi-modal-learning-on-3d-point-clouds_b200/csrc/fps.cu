@@ -55,26 +55,6 @@ __device__ __forceinline__ void update_min(const float (&x)[P], const float (&y)
     }
 }
 
-// The same update that also returns max_i tm[i] (values only): pairs of running minima go through FMNMX3.
-template <int P>
-__device__ __forceinline__ float update_min_max(const float (&x)[P], const float (&y)[P], const float (&z)[P], float (&tm)[P],
-                                                float cx, float cy, float cz) {
-    static_assert(P % 2 == 0, "pairs");
-    const float2 nx = make_float2(-cx, -cx), ny = make_float2(-cy, -cy), nz = make_float2(-cz, -cz);
-    float best = 0.f;  // running minima are >= 0
-#pragma unroll
-    for (int i = 0; i < P; i += 2) {
-        const float2 dx = __fadd2_rn(make_float2(x[i], x[i + 1]), nx);
-        const float2 dy = __fadd2_rn(make_float2(y[i], y[i + 1]), ny);
-        const float2 dz = __fadd2_rn(make_float2(z[i], z[i + 1]), nz);
-        const float2 d = __ffma2_rn(dz, dz, __ffma2_rn(dx, dx, __fmul2_rn(dy, dy)));
-        tm[i] = fminf(d.x, tm[i]);
-        tm[i + 1] = fminf(d.y, tm[i + 1]);
-        best = fmaxf(fmaxf(best, tm[i]), tm[i + 1]);
-    }
-    return best;
-}
-
 template <int T>
 struct Log2 {
     static constexpr int value = 1 + Log2<T / 2>::value;
@@ -161,34 +141,25 @@ fps_reg_kernel(int n, int m, const float *__restrict__ xyz_all, int32_t *__restr
     }
 }
 
-// One CTA per cloud with FEWER THREADS than the reference block size (bs = 1024): T = 1024 / SUB threads own
-// P = SUB * Q points each (Q = capacity / 1024).  The fixed per-warp cost of a round (two CREDUX pairs, slot exchange,
-// barrier, decode) is paid by T/32 warps instead of 32, so a round issues ~30 % fewer instructions and the CTA holds
-// fewer registers -- the variant for several batches in flight, where SM time, not latency, is what FPS costs.
-// Thread t owns k = t + T*(SUB*q + s), q < Q, s < SUB.  Its tie key is (bitrev10(k mod 1024) << QB) | q with
-// bitrev10(t + T*s) = bitrev10(t) + bitrev_{log2 SUB}(s), so the in-thread tie order is "s in bit-reversed order, then
-// q ascending": the points are held in that order (slot j = bitrev(s)*Q + q) and the first strict maximum in ascending
-// j is the reference's winner.
-//
-// kValueFirst (developer mode 6, NOT the default): the round reduces the VALUE of the maximum only (one FMNMX3 per pair of
-// points in the update, one CREDUX per warp, one shared-memory hop); which point holds it is worked out afterwards by the
-// few threads whose own maximum equals it -- first slot in tie order, then an atomic minimum of the tie keys in shared
-// memory -- instead of carrying (value, slot) pairs through a 31-step select tree in every thread.  Fewer instructions
-// for seven of the eight warps (the round issues 2.7 instructions per cycle and SM: 2256 warp instructions in 1038 cycles
-// at 32 points per thread), but one more block barrier in the serial tail of the round; measured (32 clouds, bit-identical
-// results): 0.571 vs 0.529 us per round at 8192 points, 0.414 vs 0.324 at 4096, 0.345 vs 0.240 at 2048, 0.321 vs 0.209 at
-// 1024 -- the dependent chain (tree, CREDUX pair, barrier, CREDUX pair, decode, coordinate fetch), not issue, is what a
-// round costs.
-template <int T, int Q, bool kValueFirst>
-__global__ void __launch_bounds__(T, 1)
+// One CTA per cloud with FEWER THREADS than the reference block size (bs = 1024): T = 256 threads own P = 4Q points
+// each (Q = capacity / 1024).  The fixed per-warp cost of a round (two CREDUX pairs, slot exchange, barrier, decode) is
+// paid by 8 warps instead of 32, so a round issues ~30 % fewer instructions and the CTA holds fewer registers -- the
+// variant for several batches in flight, where SM time, not latency, is what FPS costs.
+// Thread t owns k = t + 256*(4q + s), q < Q, s < 4.  Its tie key is (bitrev10(k mod 1024) << QB) | q with
+// bitrev10(t + 256 s) = bitrev10(t) + bitrev2(s), so the in-thread tie order is "s in bit-reversed order, then q
+// ascending": the points are held in that order (slot j = bitrev2(s)*Q + q) and the first strict maximum in ascending j
+// is the reference's winner.
+// A value-first round (reduce only the maximum's value, then the threads holding it resolve the tie key by an atomic
+// minimum in shared memory) was slower: 0.571 vs 0.529 us per round at 8192 points (32 clouds) -- it saves issue slots
+// but adds a block barrier to the round's dependent chain, and that chain, not issue, is what a round costs.
+template <int Q>
+__global__ void __launch_bounds__(256, 1)
 fps_few_kernel(int n, int m, const float *__restrict__ xyz_all, int32_t *__restrict__ idx_all,
                float *__restrict__ new_xyz_all) {
-    constexpr int SUB = 1024 / T, LS = Log2<SUB>::value, P = SUB * Q, NW = T / 32;
+    constexpr int T = 256, SUB = 4, LS = 2, P = SUB * Q, NW = T / 32;
     extern __shared__ float smem[];
     float *sx = smem, *sy = smem + 1024 * Q, *sz = smem + 2 * 1024 * Q;
     __shared__ unsigned long long slot[2][32];
-    __shared__ uint32_t slotv[2][32];
-    __shared__ uint32_t win[2];
 
     const float *xyz = xyz_all + (size_t)blockIdx.x * n * 3;
     int32_t *idx = idx_all + (size_t)blockIdx.x * m;
@@ -198,7 +169,7 @@ fps_few_kernel(int n, int m, const float *__restrict__ xyz_all, int32_t *__restr
 #pragma unroll
     for (int j = 0; j < P; ++j) {
         const int sr = j / Q, q = j % Q;                               // sr = bit-reversed s
-        const int sb = (int)(__brev((unsigned)sr) >> (32 - (LS > 0 ? LS : 1))) & (SUB - 1);
+        const int sb = (int)(__brev((unsigned)sr) >> (32 - LS));
         const int k = t + T * (SUB * q + sb);
         const bool ok = k < n;
         x[j] = ok ? xyz[3 * k + 0] : 0.f;
@@ -212,47 +183,11 @@ fps_few_kernel(int n, int m, const float *__restrict__ xyz_all, int32_t *__restr
     const uint32_t rank0 = __brev((uint32_t)t) >> 22;  // bitrev10(t); t < T so its low log2(SUB) bits are free
     const uint32_t inv_base = 0xFFFFFFFFu - (rank0 << QB);
     float *new_xyz = new_xyz_all ? new_xyz_all + (size_t)blockIdx.x * m * 3 : nullptr;
-    if (t == 0) {
-        idx[0] = 0;
-        win[0] = win[1] = 0xFFFFFFFFu;
-    }
+    if (t == 0) idx[0] = 0;
     __syncthreads();
     float x1 = sx[0], y1 = sy[0], z1 = sz[0];
     if (t == 0 && new_xyz) {
         new_xyz[0] = x1; new_xyz[1] = y1; new_xyz[2] = z1;
-    }
-
-    if constexpr (kValueFirst && P % 2 == 0) {
-        for (int r = 1; r < m; ++r) {
-            const float lm = update_min_max<P>(x, y, z, tm, x1, y1, z1);
-            const uint32_t hi = __float_as_uint(lm);  // non-negative floats order like their bit patterns
-            const uint32_t wh = __reduce_max_sync(0xffffffffu, hi);
-            if (lane == 0) slotv[r & 1][warp] = wh;
-            __syncthreads();
-            if (t == 0) win[(r + 1) & 1] = 0xFFFFFFFFu;  // next round's cell; its last readers are past this barrier
-            const uint32_t M = __reduce_max_sync(0xffffffffu, lane < NW ? slotv[r & 1][lane] : 0u);
-            if (hi == M) {
-                // this thread holds a point at the maximum: its first such slot in tie order, then the smallest tie key wins
-                int bj = P - 1;
-#pragma unroll
-                for (int j = P - 2; j >= 0; --j) bj = (__float_as_uint(tm[j]) == M) ? j : bj;
-                const uint32_t key = (rank0 << QB) + ((((uint32_t)bj / Q) << QB) | ((uint32_t)bj % Q));
-                atomicMin(&win[r & 1], key);
-            }
-            __syncthreads();
-            const uint32_t tie = win[r & 1];
-            const int k = (int)(tie & QMASK) * 1024 + (int)(__brev(tie >> QB) >> 22);
-            x1 = sx[k];
-            y1 = sy[k];
-            z1 = sz[k];
-            if (t == 0) {
-                idx[r] = k;
-                if (new_xyz) {
-                    new_xyz[3 * r] = x1; new_xyz[3 * r + 1] = y1; new_xyz[3 * r + 2] = z1;
-                }
-            }
-        }
-        return;
     }
 
     for (int r = 1; r < m; ++r) {
@@ -797,18 +732,11 @@ int launch_reg(int b, int n, int m, const float *xyz, int32_t *idx, float *new_x
     return PN2_OK;
 }
 
-int fps_force_mode();
-
-template <int T, int Q>
+template <int Q>
 int launch_few(int b, int n, int m, const float *xyz, int32_t *idx, float *new_xyz, cudaStream_t s) {
     const size_t smem = (size_t)3 * 1024 * Q * sizeof(float);
-    if (fps_force_mode() == 6) {  // developer mode 6: the value-first round (measured slower, see the kernel's comment)
-        PN2_CUDA(cudaFuncSetAttribute(fps_few_kernel<T, Q, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        fps_few_kernel<T, Q, true><<<b, T, smem, s>>>(n, m, xyz, idx, new_xyz);
-    } else {
-        PN2_CUDA(cudaFuncSetAttribute(fps_few_kernel<T, Q, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        fps_few_kernel<T, Q, false><<<b, T, smem, s>>>(n, m, xyz, idx, new_xyz);
-    }
+    PN2_CUDA(cudaFuncSetAttribute(fps_few_kernel<Q>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fps_few_kernel<Q><<<b, 256, smem, s>>>(n, m, xyz, idx, new_xyz);
     PN2_LAUNCH_OK("fps_few_kernel");
     return PN2_OK;
 }
@@ -852,19 +780,18 @@ int launch_reg_small(int b, int n, int m, const float *xyz, int32_t *idx, float 
 }  // namespace
 }  // namespace pn2
 
-// 0 = automatic, 1 = one CTA per cloud, 2 = cluster kernel; 3 / 4 = developer variants (see fps_impl)
-static int g_fps_mode = 0;
-extern "C" void pn2_debug_set_fps_mode(int mode) { g_fps_mode = mode; }
+// PN2_FPS_AUTO / PN2_FPS_ONE_CTA / PN2_FPS_CLUSTER (see fps_impl)
+static int g_fps_policy = PN2_FPS_AUTO;
 extern "C" int pn2_set_fps_policy(int policy) {
     if (policy < PN2_FPS_AUTO || policy > PN2_FPS_CLUSTER) return -1;
-    const int prev = g_fps_mode;
-    g_fps_mode = policy;
+    const int prev = g_fps_policy;
+    g_fps_policy = policy;
     return prev;
 }
+extern "C" void pn2_debug_set_fps_mode(int mode) { pn2_set_fps_policy(mode); }
 
 namespace pn2 {
 namespace {
-int fps_force_mode() { return g_fps_mode; }
 int fps_impl(int b, int n, int m, const float *xyz, float *temp, int32_t *idx, float *new_xyz, void *stream) {
     PN2_REQUIRE(b >= 0 && n >= 1, "fps: need b >= 0 and n >= 1 (got b=%d n=%d)", b, n);
     if (b == 0 || m <= 0) return PN2_OK;  // the reference kernel returns at once for m <= 0 (sampling_gpu.cu:101)
@@ -887,16 +814,15 @@ int fps_impl(int b, int n, int m, const float *xyz, float *temp, int32_t *idx, f
         case 512: return launch_reg_small<512>(b, n, m, xyz, idx, new_xyz, s);
         default: break;
     }
-    if (n == 1024 && fps_force_mode() != 4) return launch_few<256, 1>(b, n, m, xyz, idx, new_xyz, s);  // 4 points per thread
+    if (n == 1024) return launch_few<1>(b, n, m, xyz, idx, new_xyz, s);  // 4 points per thread
     if (n <= 1024) return launch_reg<1024, 1>(b, n, m, xyz, idx, new_xyz, s);
     // 1024 < n <= 8192.  One CTA per cloud = the 256-thread kernel (fps_few_kernel): 0.12 / 0.17 / 0.54 ms for
     // 2048->512 / 4096->512 / 8192->1024, faster than both alternatives up to 4096 points.  At 4096 < n <= 8192 the
     // 4-CTA cluster is 17 % faster (0.45 ms) but occupies four SMs per cloud: chosen automatically only while the
     // clouds alone cannot fill the GPU; PN2_FPS_ONE_CTA keeps one SM per cloud (several batches in flight).
-    // Developer modes: 3 = 512-thread variant, 4 = the 1024-thread kernel (one point rank per thread).
-    const int mode = fps_force_mode();
+    const int policy = g_fps_policy;
     const bool cluster_ok = (long long)b * 4 <= sm_count();
-    const bool use_cluster = n > 8192 || mode == PN2_FPS_CLUSTER || (mode == PN2_FPS_AUTO && n > 4096 && cluster_ok);
+    const bool use_cluster = n > 8192 || policy == PN2_FPS_CLUSTER || (policy == PN2_FPS_AUTO && n > 4096 && cluster_ok);
     if (use_cluster) {
         // large sweeps: 8 CTAs per cloud (half the points per thread) while the clusters still fit the GPU in one wave
         if (n <= 2048) return launch_cluster<2>(b, n, m, xyz, idx, new_xyz, s);
@@ -912,23 +838,13 @@ int fps_impl(int b, int n, int m, const float *xyz, float *temp, int32_t *idx, f
         // than the halved per-thread work saves: 16 sweeps x 34720 points 1789 -> 1483 sweeps/s, so 4 CTAs stay the default;
         // 512-thread CTAs -- 18 points per thread -- were no faster either: 0.80 vs 0.74 us per round.)
         if (n <= 65536) return launch_cluster<32, 8>(b, n, m, xyz, idx, new_xyz, s);
-    } else if (mode == 4) {
-        if (n <= 2048) return launch_reg<1024, 2>(b, n, m, xyz, idx, new_xyz, s);
-        if (n <= 4096) return launch_reg<1024, 4>(b, n, m, xyz, idx, new_xyz, s);
-        return launch_reg<1024, 8>(b, n, m, xyz, idx, new_xyz, s);
-    } else if (mode == 3 && n > 4096) {
-        return launch_few<512, 8>(b, n, m, xyz, idx, new_xyz, s);
     } else {
-        if (n <= 2048) return launch_few<256, 2>(b, n, m, xyz, idx, new_xyz, s);
-        if (mode == 7) {  // developer mode 7: the index-interleaved kernel at every size (what the slab kernel replaced)
-            if (n <= 4096) return launch_few<256, 4>(b, n, m, xyz, idx, new_xyz, s);
-            return launch_few<256, 8>(b, n, m, xyz, idx, new_xyz, s);
-        }
+        if (n <= 2048) return launch_few<2>(b, n, m, xyz, idx, new_xyz, s);
         // spatial slabs per warp + skipped rounds: pays once enough points are picked for the running minima to fall
         // below the slab distances (a few hundred picks)
         // (at 4096 points the slab kernel's set-up and per-round test cost more than the skipped rounds save)
-        if (n <= 4096) return launch_few<256, 4>(b, n, m, xyz, idx, new_xyz, s);
-        return m >= 128 ? launch_slab<8>(b, n, m, xyz, idx, new_xyz, s) : launch_few<256, 8>(b, n, m, xyz, idx, new_xyz, s);
+        if (n <= 4096) return launch_few<4>(b, n, m, xyz, idx, new_xyz, s);
+        return m >= 128 ? launch_slab<8>(b, n, m, xyz, idx, new_xyz, s) : launch_few<8>(b, n, m, xyz, idx, new_xyz, s);
     }
     if (!temp)
         return set_error(PN2_ERR_INVALID_ARGUMENT, "fps: n=%d exceeds the on-chip kernels; pass the (B,N) temp scratch", n);

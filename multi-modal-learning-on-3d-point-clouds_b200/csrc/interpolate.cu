@@ -334,8 +334,9 @@ int launch_interp_smem(int b, int c, int m, int n, const float *points, const in
 // quarter hold contiguous bytes of a channel row; a quarter then writes two whole lines (stores: 20 -> 8 us of the fp1 shape).
 // Persistent CTAs: the (cloud, channel tile, granule) space is cut into gridDim.x contiguous ranges, so a CTA stages at
 // most two tiles more than it has whole (cloud, tile) pairs and there is no partial last wave.
-// `probe` (developer bisect, pn2_debug_set_interp_mode bits 10 / 11): 1 = no stores, 2 = no row reads.  At the fp1 shape
-// (45 us): stores 8 us, row reads 6 us, the rest (stage 2 x 128 KB per CTA, ring, arithmetic, shuffles) 31 us.
+// Time split at the fp1 shape (45 us), measured by switching the stores or the row reads off: stores 8 us, row reads 6 us,
+// the rest (stage 2 x 128 KB per CTA, ring, arithmetic, shuffles) 31 us.  768- and 1024-thread CTAs (80 / 64 registers)
+// were slower: 59.4 / 65.5 us against 49.2 at 512 threads (before the shuffle exchange; profiles/README.md).
 
 // Transposing stage: tile4[k][q ^ ((k >> 2) & (LPR - 1))] = channels q + LPR * {0,1,2,3} of coarse point k (zero beyond nc).
 // Vector form: an item = four consecutive points of four channel rows (four coalesced 128-bit loads) -> four swizzled
@@ -345,7 +346,7 @@ __device__ __forceinline__ void lac_stage_tile(float4 *tile4, const float *__res
     if ((m & 3) == 0 && ((uintptr_t)f & 15) == 0) {
         const int m4 = m >> 2;
         const int items = LPR * m4;
-        constexpr int NB = T >= 768 ? 2 : 4;  // items per thread and batch
+        constexpr int NB = 4;  // items per thread and batch
         for (int base = 0; base < items; base += NB * T) {
             float4 r[NB][4];
             int cqs[NB], is[NB];
@@ -389,7 +390,7 @@ template <int CC, int T>
 __global__ void __launch_bounds__(T, T <= 256 ? 2 : 1)
 three_interpolate_lac_kernel(int c, int m, int n, int chunks, int gpp, long long total_gran,
                              const float *__restrict__ points, const int32_t *__restrict__ idx,
-                             const float *__restrict__ weight, float *__restrict__ out, int probe) {
+                             const float *__restrict__ weight, float *__restrict__ out) {
     constexpr int LPR = CC / 4;    // lanes per coarse row = lanes per group
     constexpr int PPI = 32 / LPR;  // groups per warp
     constexpr int GRAN = LC_GRAN;  // points per warp granule
@@ -464,14 +465,9 @@ three_interpolate_lac_kernel(int c, int m, int n, int chunks, int gpp, long long
                     for (int s = 0; s < 8; ++s) {
                         const int k0 = ri[3 * (q0 + s)], k1 = ri[3 * (q0 + s) + 1], k2 = ri[3 * (q0 + s) + 2];
                         const float w0 = rw[3 * (q0 + s)], w1 = rw[3 * (q0 + s) + 1], w2 = rw[3 * (q0 + s) + 2];
-                        float4 a0, a1, a2;
-                        if (probe & 2) {
-                            a0 = a1 = a2 = make_float4(__int_as_float(k0), __int_as_float(k1), __int_as_float(k2), w0);
-                        } else {
-                            a0 = *reinterpret_cast<const float4 *>(tile_bytes + row_off(k0));
-                            a1 = *reinterpret_cast<const float4 *>(tile_bytes + row_off(k1));
-                            a2 = *reinterpret_cast<const float4 *>(tile_bytes + row_off(k2));
-                        }
+                        const float4 a0 = *reinterpret_cast<const float4 *>(tile_bytes + row_off(k0));
+                        const float4 a1 = *reinterpret_cast<const float4 *>(tile_bytes + row_off(k1));
+                        const float4 a2 = *reinterpret_cast<const float4 *>(tile_bytes + row_off(k2));
                         // the reference's contraction (K8): fma(w2, f2, fma(w0, f0, rn(w1 * f1)))
                         acc[0][s] = __fmaf_rn(w2, a2.x, __fmaf_rn(w0, a0.x, __fmul_rn(w1, a1.x)));
                         acc[1][s] = __fmaf_rn(w2, a2.y, __fmaf_rn(w0, a0.y, __fmul_rn(w1, a1.y)));
@@ -494,7 +490,7 @@ three_interpolate_lac_kernel(int c, int m, int n, int chunks, int gpp, long long
 #pragma unroll
                     for (int s = 0; s < 8; ++s) v[s] = __shfl_sync(0xffffffffu, acc[u][s], src);
                     const int ch = LPR * u + 2 * Q + (l >> 2);
-                    if (ch < nc && prun < n && (!(probe & 1) || v[0] + v[7] == 12345.678f))
+                    if (ch < nc && prun < n)
                         asm volatile("st.global.cs.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(ob + (size_t)ch * n + prun), "f"(v[0]),
                                      "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7])
                                      : "memory");
@@ -506,8 +502,7 @@ three_interpolate_lac_kernel(int c, int m, int n, int chunks, int gpp, long long
 }
 
 int g_interp_mode = 0;  // developer knob (pn2_debug_set_interp_mode): 0 auto, 1 tiled kernels only, 32 the lane-along-channel
-                        // kernel wherever it applies (+ 256: 256-thread CTAs, two per SM; + 4096 / 512: 768 / 1024 threads;
-                        // + 1024 / 2048: probe bits)
+                        // kernel wherever it applies (32 | 256: 256-thread CTAs, two per SM); any other value = auto
 
 inline size_t lac_smem_bytes(int m, int cc, int threads) {
     return (size_t)m * cc * 4 + (size_t)(threads / 32) * LC_DEPTH * LC_GRAN * 24;
@@ -523,7 +518,7 @@ int launch_interp_lac(int b, int c, int m, int n, const float *points, const int
     const size_t smem = lac_smem_bytes(m, CC, T);
     const int grid = (int)std::min<long long>((long long)(T <= 256 ? 2 : 1) * sm_count(), std::max<long long>(1, total / (T / 32)));
     PN2_CUDA(cudaFuncSetAttribute(three_interpolate_lac_kernel<CC, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    three_interpolate_lac_kernel<CC, T><<<grid, T, smem, s>>>(c, m, n, chunks, gpp, total, points, idx, weight, out, (g_interp_mode >> 10) & 3);
+    three_interpolate_lac_kernel<CC, T><<<grid, T, smem, s>>>(c, m, n, chunks, gpp, total, points, idx, weight, out);
     PN2_LAUNCH_OK("three_interpolate");
     return PN2_OK;
 }
@@ -596,14 +591,11 @@ extern "C" int pn2_three_interpolate(int b, int c, int m, int n, const float *po
         // 16-byte aligned idx / weight.  Measured (scripts/interp_sweep.py, profiles/r1_interp_sweep_lac.jsonl): fp1 shape (b 32,
         // c 128, m 1024, n 8192) 57 -> 45 us = 53 % of HBM, 20-40 % faster at m <= 256; no gain with too little work per SM.
         cudaStream_t st = (cudaStream_t)stream;
-        const bool forced = (g_interp_mode & 255) == 32;
-        const int threads = forced ? ((g_interp_mode & 256) ? 256 : (g_interp_mode & 512) ? 1024 : (g_interp_mode & 4096) ? 768 : 512)
-                                   : (lac_fits(m, 32, 256) ? 256 : 512);
+        const bool forced = g_interp_mode == 32 || g_interp_mode == (32 | 256);
+        const int threads = forced ? (g_interp_mode == 32 ? 512 : 256) : (lac_fits(m, 32, 256) ? 256 : 512);
         const long long granules = (long long)b * ceil_div(c, 32) * ceil_div(n, LC_GRAN);
         const bool wanted = forced || (c >= 32 && n >= 2 * m && (m <= 512 || granules >= 16ll * sm_count()));
         if (wanted && lac_fits(m, 32, threads)) {
-            if (threads == 1024) return launch_interp_lac<32, 1024>(b, c, m, n, points, idx, weight, out, st);
-            if (threads == 768) return launch_interp_lac<32, 768>(b, c, m, n, points, idx, weight, out, st);
             if (threads == 512) return launch_interp_lac<32, 512>(b, c, m, n, points, idx, weight, out, st);
             return launch_interp_lac<32, 256>(b, c, m, n, points, idx, weight, out, st);
         }

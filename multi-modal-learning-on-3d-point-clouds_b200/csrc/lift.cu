@@ -329,7 +329,6 @@ lift_project_kernel(int n, int nv, int h, int w, const float *__restrict__ point
 }
 
 constexpr int LG_THREADS = 512;
-int g_lift_mode = 0;  // developer knob (pn2_debug_set_lift_mode): 1 = channel-major slab kernel only
 
 template <int CH>
 __global__ void __launch_bounds__(LG_THREADS)
@@ -777,8 +776,6 @@ int launch_lift_grad_t(int b, int n, int nv, int c, int hw, const float *feats, 
 }  // namespace
 }  // namespace pn2
 
-extern "C" void pn2_debug_set_lift_mode(int mode) { pn2::g_lift_mode = mode; }
-
 extern "C" int pn2_frustum_count(int n, int num_poses, const float *points, const float *corner2, const float *corner4,
                                  const float *normals, int32_t *counts, void *stream) {
     using namespace pn2;
@@ -831,7 +828,7 @@ static int lift_views_impl(int b, int n, int v, int c, int h, int w, const float
         const bool first = reduce == PN2_REDUCE_FIRST && c > 0;
         // the pixel-major gather reads 16-bit pixel indices (half the index traffic: every 4-channel CTA re-reads them)
         const bool pm_ok = c > 0 && (n & 3) == 0 && (((uintptr_t)out) & 15) == 0 && (size_t)v * hw * 16 <= 200 * 1024 && hw < 32768 &&
-                           ceil_div(c, 4) <= 65535 && g_lift_mode != 1;
+                           ceil_div(c, 4) <= 65535;
         const bool need32 = !pix && !pm_ok;
         const size_t pix_bytes = need32 ? ((size_t)b * v * n * sizeof(int32_t) + 255) / 256 * 256 : 0;
         const size_t pix16_bytes = pm_ok ? ((size_t)b * v * n * sizeof(int16_t) + 255) / 256 * 256 : 0;

@@ -18,8 +18,6 @@
 // BatchNorm is folded into (W, bias) by the caller (eval mode), see pn2_b200/pointnet_util.py.
 //
 // fp32 FFMA throughout (the 1e-5 parity path).  The bf16 tcgen05 variant lives in row_mlp_tc.cu.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "row_mlp_tile.cuh"
 
@@ -290,12 +288,10 @@ int launch(const RowMlpParams &p, const Layout &L, long long tiles, cudaStream_t
 // would leave SMs idle.
 int dispatch(RowMlpParams &p, const pn2_mlp *mlp, int c0, long long total_rows, int min_tr, cudaStream_t s) {
     const int cands[4] = {128, 64, 32, 16};
-    static const int forced = getenv("PN2_DEV_ROW_TILE") ? atoi(getenv("PN2_DEV_ROW_TILE")) : 0;  // developer timing only
     int chosen = -1;
     for (int i = 0; i < 4; ++i) {
         const int tr = cands[i];
         if (tr < min_tr || tr % min_tr) continue;
-        if (forced && tr > forced && tr / 2 >= min_tr) continue;
         if (make_layout(tr, c0, mlp).bytes > SMEM_LIMIT) continue;
         chosen = tr;
         const long long tiles = (total_rows + tr - 1) / tr;

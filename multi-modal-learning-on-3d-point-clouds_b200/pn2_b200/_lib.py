@@ -84,7 +84,6 @@ _OTHER = {
     "pn2_debug_set_tc_max_ctas": ([_c_int], None),
     "pn2_debug_set_tc_workers": ([_c_int], None),
     "pn2_debug_last_tc_launch": ([ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(_c_int), ctypes.POINTER(_c_int)], _c_int),
-    "pn2_debug_set_lift_mode": ([_c_int], None),
     "pn2_debug_set_interp_mode": ([_c_int], None),
     "pn2_mlp_pack_bf16_size": ([ctypes.POINTER(Pn2Mlp)], ctypes.c_longlong),
 }
@@ -114,8 +113,6 @@ def load():
             fn = getattr(lib, name)
             fn.argtypes = argtypes
             fn.restype = restype
-        if os.environ.get("PN2_TC_WORKERS"):  # developer knob: worker warps per tile of the tensor-core MLP kernel
-            lib.pn2_debug_set_tc_workers(int(os.environ["PN2_TC_WORKERS"]))
         _lib = lib
     return _lib
 

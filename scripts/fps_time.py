@@ -1,5 +1,6 @@
-"""FPS round time per kernel choice: mode 1 = one 256-thread CTA per cloud (spatial slabs per warp, skipped rounds), 7 = the
-index-interleaved single-CTA kernel it replaced, 2 = 4-CTA cluster with DSMEM exchange.  CUDA events, L2 flushed, median of 7."""
+"""FPS round time per kernel policy: mode 1 = one 256-thread CTA per cloud (spatial slabs per warp with skipped rounds
+above 4096 points, the index-interleaved kernel up to 4096), 2 = 4-CTA cluster with DSMEM exchange.  CUDA events, L2
+flushed, median of 7."""
 import json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "multi-modal-learning-on-3d-point-clouds_b200"))
@@ -13,7 +14,7 @@ B = int(sys.argv[1]) if len(sys.argv) > 1 else 32
 for (N, M) in ((8192, 1024), (4096, 1024), (2048, 512), (1024, 256)):
     xyz = torch.from_numpy(np.stack([scenes.scannet_scene(10 + b, N)[0] for b in range(B)])).to(dev)
     row = {"B": B, "N": N, "M": M}
-    for mode in (1, 7, 2):
+    for mode in (1, 2):
         lib.pn2_debug_set_fps_mode(mode)
         for _ in range(2):
             fps_gather_cl(xyz, M)

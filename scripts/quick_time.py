@@ -42,7 +42,7 @@ def main():
         x = xyz[:, :n].contiguous()
         print("fps %d->%d: med %.3f ms min %.3f" % ((n, m) + timeit(lambda: fps_gather_cl(x, m))))
     from pn2_b200 import _lib as L
-    for mode in (1, 2, 3, 4):
+    for mode in (1, 2):
         L.load().pn2_debug_set_fps_mode(mode)
         print("fps 8192->1024 mode %d: med %.3f ms min %.3f" % ((mode,) + timeit(lambda: fps_gather_cl(xyz, 1024))))
         x4, x2 = xyz[:, :4096].contiguous(), xyz[:, :2048].contiguous()

@@ -73,6 +73,10 @@ def test_fps_policy_switch_returns_previous_value():
     assert lib.pn2_set_fps_policy(2) == 1
     assert lib.pn2_set_fps_policy(7) == -1          # unknown policy: refused, state unchanged
     assert lib.pn2_set_fps_policy(0) == 2
+    lib.pn2_debug_set_fps_mode(2)                   # the developer switch sets the same policy
+    assert lib.pn2_set_fps_policy(1) == 2
+    lib.pn2_debug_set_fps_mode(6)                   # unknown value: refused, policy unchanged
+    assert lib.pn2_set_fps_policy(0) == 1
     from pn2_b200.pointnet_util import fps_policy
     with fps_policy("throughput"):
         assert lib.pn2_set_fps_policy(1) == 1
