@@ -200,6 +200,42 @@ int pn2_train_linear_bwd(long long rows, int cin, int cout, const float *x, cons
                          const float *wt, const float *g, const float *z, const float *scale, const float *shift,
                          const float *ca, const float *cb, const float *cc, float *g_in, float *dw, void *stream);
 
+/* ---- first and last layer of a whole training-mode SA scale / FP block: the grouped or interpolated operand is read
+ * where it lies and never materialised, the pooled output is written without the (rows,c) activation. ----
+ * Row source of the first layer (fp32, channel-last, contiguous):
+ *   PN2_ROWS_GROUPED (SA): xyz (b,n,3), feat (b,n,d) or NULL (d == 0), new_xyz (b,m,3), idx (b,m,k) in [0,n);
+ *     row (bb*m + s)*k + j = [xyz[p] - new_xyz[s] | feat[p]] (PN2_ORDER_XYZ_FIRST) or [feat[p] | xyz[p] - new_xyz[s]]
+ *     (PN2_ORDER_FEAT_FIRST), p = idx[bb,s,j]; the centring is one fp32 subtraction.  rows = b*m*k, cin = 3 + d.
+ *   PN2_ROWS_INTERP (FP): skip (b,n,d_skip) or NULL (d_skip == 0), feat (b,m,d), idx / weight (b,n,3);
+ *     row bb*n + i = [skip[i] | fma(w2,f[i2],fma(w0,f[i0],w1*f[i1]))] (three_interpolate's order); with m == 1 idx and
+ *     weight are NULL and the one coarse row is repeated.  rows = b*n, cin = d_skip + d. */
+#define PN2_ROWS_GROUPED 1
+#define PN2_ROWS_INTERP 2
+typedef struct pn2_rows {
+    int kind;
+    int order; /* PN2_ROWS_GROUPED: PN2_ORDER_XYZ_FIRST or PN2_ORDER_FEAT_FIRST */
+    int b, n, m, k, d, d_skip;
+    const float *xyz, *new_xyz, *feat, *skip;
+    const int32_t *idx;
+    const float *weight;
+} pn2_rows;
+/* pn2_train_linear_fwd with the first layer's operand read from `src` (no act_in). */
+int pn2_train_linear_fwd_rows(long long rows, int cin, int cout, const pn2_rows *src, const float *w, const float *bias,
+                              float *z, double *stats, void *stream);
+/* pn2_train_linear_bwd of the first layer with x read from `src`.  g_in (rows, cin) (NULL = not needed); for
+ * PN2_ROWS_INTERP the first d_skip columns go to g_skip (rows, d_skip) and g_in holds the d interpolated columns
+ * (rows, d); either may be NULL. */
+int pn2_train_linear_bwd_rows(long long rows, int cin, int cout, const pn2_rows *src, const float *wt, const float *g,
+                              const float *z, const float *scale, const float *shift, const float *ca, const float *cb,
+                              const float *cc, float *g_in, float *g_skip, float *dw, void *stream);
+/* Last layer + max over the k rows of each of `groups` groups: a = relu(scale z + shift) (as pn2_train_bn_relu), z (groups*k, c);
+ * out[gr*out_stride + out_offset + ch] = max_j a, arg (groups, c) uint8 = the first j holding it.  k <= 256. */
+int pn2_train_bn_relu_max(long long groups, int k, int c, const float *z, const float *scale, const float *shift, float *out,
+                          int out_stride, int out_offset, uint8_t *arg, void *stream);
+/* Backward of the pooling: g (groups*k, c) written in full, g = gp[gr*gp_stride + gp_offset + ch] on row j == arg, 0 elsewhere. */
+int pn2_train_max_bwd(long long groups, int k, int c, const float *gp, int gp_stride, int gp_offset, const uint8_t *arg,
+                      float *g, void *stream);
+
 /* ---- the same two blocks on the tcgen05 tensor cores: bf16 operands, fp32 accumulation in TMEM ----
  * Outputs agree with the fp32 entry points within bf16 rounding (2e-2 relative).  Weights are packed once
  * (bf16, pre-swizzled UMMA tiles) with pn2_mlp_pack_bf16; biases are still read from `mlp`.
@@ -268,6 +304,11 @@ int pn2_three_nn_grid(int b, int n, int m, const float *unknown, const float *kn
 int pn2_inverse_index(int b, int n, long long j, const int32_t *idx, int32_t *seg_start, int32_t *pos, void *stream);
 int pn2_scatter_rows_det(int b, int c, int n, long long j, int div, const float *grad_out, const int32_t *seg_start,
                          const int32_t *pos, const float *weight, float *grad_points, void *stream);
+/* Channel-last pn2_scatter_rows_det over row matrices, WRITTEN in full (no pre-zeroing; 0 where no row refers to a point):
+ *   grad_points[bb,k,c] = sum over the p of (bb,k), ascending, of weight[bb,p] * g_in[(bb*(j/div) + p/div)*row_stride + col_offset + c]
+ *   for c < d, grad_points (b,n,d).  SA grouping: j = m*nsample, div = 1, weight NULL; three_interpolate: j = 3*n_fine, div = 3. */
+int pn2_scatter_rows_det_cl(int b, int d, int n, long long j, int div, const float *g_in, int row_stride, int col_offset,
+                            const int32_t *seg_start, const int32_t *pos, const float *weight, float *grad_points, void *stream);
 
 /* ---- evaluation voxelisation (SURVEY 8f N3) ----
  * utils/pc_util.py:39-51 point_cloud_label_to_surface_voxel_label_fast, as the evaluation loops call it per scene

@@ -75,6 +75,32 @@ scatter_det_kernel(int c, int n, long long J, int div, const float *__restrict__
         if (q < cc) dst[(size_t)q * n] += acc[q];
 }
 
+// Channel-last variant over row matrices: thread <-> (destination point, channel), lanes along channels, so each
+// contribution is a contiguous slice of one row of g_in; same per-element order and arithmetic as scatter_det_kernel.
+// Every element of grad_points is written (0 for a point no row refers to).
+__global__ void __launch_bounds__(256)
+scatter_det_cl_kernel(long long total, int d, int n, long long J, int div, const float *__restrict__ g_in, int row_stride,
+                      int col_offset, const int32_t *__restrict__ seg_start, const int32_t *__restrict__ pos,
+                      const float *__restrict__ weight, float *__restrict__ grad_points) {
+    const long long rows_per_cloud = J / div;
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+        const long long key = e / d;  // b * n + k
+        const int ch = (int)(e - key * d);
+        const long long b = key / n;
+        const int s0 = __ldg(seg_start + key), s1 = __ldg(seg_start + key + 1);
+        const float *g = g_in + b * rows_per_cloud * row_stride + col_offset + ch;
+        const float *w = weight ? weight + b * J : nullptr;
+        float acc = 0.f;
+        for (int s = s0; s < s1; ++s) {
+            const int p = __ldg(pos + s);
+            const int row = div == 1 ? p : p / div;
+            const float go = __ldg(g + (long long)row * row_stride);
+            acc = __fadd_rn(acc, w ? __fmul_rn(go, __ldg(w + p)) : go);
+        }
+        grad_points[e] = acc;
+    }
+}
+
 }  // namespace
 
 size_t segment_sort_scratch_bytes(long long total, long long nkeys) {
@@ -142,5 +168,24 @@ extern "C" int pn2_scatter_rows_det(int b, int c, int n, long long j, int div, c
     dim3 grid((unsigned)((n + DET_THREADS - 1) / DET_THREADS), (unsigned)((c + DET_CH - 1) / DET_CH), (unsigned)b);
     scatter_det_kernel<<<grid, DET_THREADS, 0, (cudaStream_t)stream>>>(c, n, j, div, grad_out, seg_start, pos, weight, grad_points);
     PN2_LAUNCH_OK("scatter_det_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_scatter_rows_det_cl(int b, int d, int n, long long j, int div, const float *g_in, int row_stride, int col_offset,
+                                       const int32_t *seg_start, const int32_t *pos, const float *weight, float *grad_points, void *stream) {
+    using namespace pn2;
+    PN2_REQUIRE(b >= 0 && d >= 0 && n >= 1 && j >= 0 && (div == 1 || div == 3), "scatter_rows_det_cl: bad dims b=%d d=%d n=%d j=%lld div=%d",
+                b, d, n, j, div);
+    PN2_REQUIRE(j % div == 0, "scatter_rows_det_cl: j=%lld is not a multiple of div=%d", j, div);
+    PN2_REQUIRE(col_offset >= 0 && row_stride >= col_offset + d, "scatter_rows_det_cl: row_stride=%d col_offset=%d d=%d", row_stride,
+                col_offset, d);
+    PN2_REQUIRE((long long)b * n < (1ll << 31) && (long long)b * j < (1ll << 31), "scatter_rows_det_cl: more than 2^31 keys");
+    if (b == 0 || d == 0) return PN2_OK;
+    PN2_REQUIRE(seg_start && grad_points && (j == 0 || (g_in && pos)), "scatter_rows_det_cl: null pointer");
+    const long long total = (long long)b * n * d;
+    const unsigned grid = (unsigned)((total + 255) / 256 < 8ll * sm_count() ? (total + 255) / 256 : 8ll * sm_count());
+    scatter_det_cl_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(total, d, n, j, div, g_in, row_stride, col_offset, seg_start, pos, weight,
+                                                                   grad_points);
+    PN2_LAUNCH_OK("scatter_det_cl_kernel");
     return PN2_OK;
 }

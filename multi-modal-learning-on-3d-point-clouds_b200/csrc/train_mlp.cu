@@ -20,6 +20,8 @@
 //
 // All four are the same register-tiled SIMT GEMM (128 x NT output tile, 256 threads, k-chunks of 16 double buffered in
 // shared memory, FFMA): the 1e-5 parity path.  Widths are arbitrary (16 .. 1536 in the MSG stack).
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace pn2 {
@@ -143,6 +145,119 @@ struct DzIn {  // dz = ca * g * [scale z + shift > 0] + cb + cc * z, built from 
     }
 };
 
+// First-layer operands of a whole SA scale / FP block (pn2_rows), read where they lie: the grouped / interpolated row
+// matrix of the reference's composition is never materialised.  Same raw() / finish() split as ActIn.
+struct GroupIn {  // row (bb*m + s)*k + j: xyz columns [xc0, xc0 + 3) = xyz[p] - new_xyz[s], feature columns [fc0, fc0 + d) = feat[p]
+    const float *xyz, *new_xyz, *feat;
+    const int32_t *idx;
+    long long rows;
+    int c, n, m, k, d, xc0, fc0;
+    // feature rows are float4-loadable (d % 4 == 0, 16-byte aligned).  Only PN2_ORDER_FEAT_FIRST (MSG, fc0 = 0) puts a
+    // 4-aligned k-chunk on 4-aligned feature columns; with xyz first (SSG, fc0 = 3) every feature element is a scalar load,
+    // as the materialised (rows, 3 + d) operand of the composition was
+    bool vec;
+    struct Raw {
+        float4 v, ctr;  // finish() = v - ctr (ctr = 0 outside the xyz columns)
+    };
+    __device__ __forceinline__ Raw raw(long long r, int kc) const {
+        Raw q;
+        q.v = q.ctr = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (r >= rows) return q;
+        const int row = (int)r, bs = row / k;
+        const long long pt = (long long)(bs / m) * n + __ldg(idx + row);
+        if (vec && kc >= fc0 && kc + 3 < fc0 + d && ((kc - fc0) & 3) == 0) {
+            q.v = __ldg(reinterpret_cast<const float4 *>(feat + pt * d + (kc - fc0)));
+            return q;
+        }
+        float v[4], t[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const int col = kc + e;
+            v[e] = t[e] = 0.f;
+            if (col >= c) continue;
+            if (col >= xc0 && col < xc0 + 3) {
+                v[e] = __ldg(xyz + pt * 3 + (col - xc0));
+                t[e] = __ldg(new_xyz + (long long)bs * 3 + (col - xc0));
+            } else {
+                v[e] = __ldg(feat + pt * d + (col - fc0));
+            }
+        }
+        q.v = make_float4(v[0], v[1], v[2], v[3]);
+        q.ctr = make_float4(t[0], t[1], t[2], t[3]);
+        return q;
+    }
+    __device__ __forceinline__ float4 finish(const Raw &q, long long, int) const {
+        // the centring of sample_and_group: one fp32 subtraction (x - 0 == x bit for bit in the feature columns)
+        return make_float4(__fsub_rn(q.v.x, q.ctr.x), __fsub_rn(q.v.y, q.ctr.y), __fsub_rn(q.v.z, q.ctr.z), __fsub_rn(q.v.w, q.ctr.w));
+    }
+};
+
+struct InterpIn {  // row bb*n + i: columns [0, ds) = skip[i], [ds, ds + d) = three_interpolate(feat, idx[i], weight[i])
+    const float *skip, *feat, *weight;
+    const int32_t *idx;  // NULL: m == 1, the one coarse row repeated
+    long long rows;
+    int c, n, m, d, ds;
+    bool vec_skip, vec_feat;  // float4-loadable rows
+    struct Raw {
+        float4 a0, a1, a2;  // a1 holds the final value of skip / repeated / out-of-range columns
+    };
+    __device__ __forceinline__ bool direct(long long r, int col) const { return r >= rows || col >= c || col < ds || !idx; }
+    __device__ __forceinline__ Raw raw(long long r, int kc) const {
+        Raw q;
+        q.a0 = q.a1 = q.a2 = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (r >= rows) return q;
+        const long long cloud = r / n;
+        int i0 = 0, i1 = 0, i2 = 0;
+        if (idx && kc + 3 >= ds) {
+            i0 = __ldg(idx + r * 3); i1 = __ldg(idx + r * 3 + 1); i2 = __ldg(idx + r * 3 + 2);
+        }
+        const float *f0 = feat + (cloud * m + i0) * d - ds, *f1 = feat + (cloud * m + i1) * d - ds, *f2 = feat + (cloud * m + i2) * d - ds;
+        if (vec_skip && kc + 3 < ds) {
+            q.a1 = __ldg(reinterpret_cast<const float4 *>(skip + r * ds + kc));
+            return q;
+        }
+        if (vec_feat && kc >= ds && kc + 3 < c && ((kc - ds) & 3) == 0) {
+            q.a1 = __ldg(reinterpret_cast<const float4 *>(f1 + kc));
+            if (idx) {
+                q.a0 = __ldg(reinterpret_cast<const float4 *>(f0 + kc));
+                q.a2 = __ldg(reinterpret_cast<const float4 *>(f2 + kc));
+            }
+            return q;
+        }
+        float a0[4], a1[4], a2[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const int col = kc + e;
+            a0[e] = a1[e] = a2[e] = 0.f;
+            if (col >= c) continue;
+            if (col < ds) {
+                a1[e] = __ldg(skip + r * ds + col);
+            } else {
+                a1[e] = __ldg(f1 + col);
+                if (idx) { a0[e] = __ldg(f0 + col); a2[e] = __ldg(f2 + col); }
+            }
+        }
+        q.a0 = make_float4(a0[0], a0[1], a0[2], a0[3]);
+        q.a1 = make_float4(a1[0], a1[1], a1[2], a1[3]);
+        q.a2 = make_float4(a2[0], a2[1], a2[2], a2[3]);
+        return q;
+    }
+    // the weights are read here, not in raw(): the row's idx load above already brought their cache line on chip, and
+    // three more live registers per staged operand made the widest weight-gradient tile spill
+    __device__ __forceinline__ float one(float w0, float w1, float w2, float a0, float a1, float a2, long long r, int col) const {
+        // three_interpolate's order (interpolate.cu)
+        return direct(r, col) ? a1 : __fmaf_rn(w2, a2, __fmaf_rn(w0, a0, __fmul_rn(w1, a1)));
+    }
+    __device__ __forceinline__ float4 finish(const Raw &q, long long r, int kc) const {
+        float w0 = 0.f, w1 = 0.f, w2 = 0.f;
+        if (r < rows && idx && kc + 3 >= ds) {
+            w0 = __ldg(weight + r * 3); w1 = __ldg(weight + r * 3 + 1); w2 = __ldg(weight + r * 3 + 2);
+        }
+        return make_float4(one(w0, w1, w2, q.a0.x, q.a1.x, q.a2.x, r, kc), one(w0, w1, w2, q.a0.y, q.a1.y, q.a2.y, r, kc + 1),
+                           one(w0, w1, w2, q.a0.z, q.a1.z, q.a2.z, r, kc + 2), one(w0, w1, w2, q.a0.w, q.a1.w, q.a2.w, r, kc + 3));
+    }
+};
+
 struct WeightIn {  // w (n_total, k_total) row-major: 4 consecutive k of output column n
     const float *w;
     int n_total, k_total;
@@ -215,9 +330,9 @@ __device__ __forceinline__ void gemm_rows(const LA &la, const WeightIn &lb, long
 }
 
 // ---- forward: z = act_in(x) W^T + b, per-channel sum / sum of squares of z ---------------------------------------------------
-template <int NT>
+template <int NT, class LX>
 __global__ void __launch_bounds__(TG_THREADS, 2)
-train_linear_fwd_kernel(ActIn xin, WeightIn w, const float *__restrict__ bias, float *__restrict__ z, double *__restrict__ stats,
+train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, float *__restrict__ z, double *__restrict__ stats,
                         long long tiles) {
     using S = TileShape<NT>;
     extern __shared__ __align__(16) float smem[];
@@ -319,9 +434,11 @@ train_bn_bwd_reduce_kernel(long long rows, int c, const float *__restrict__ g, c
 }
 
 // ---- backward, input gradient: g_in = dz W  (W^T given as wt (cin, cout) row-major) -------------------------------------------
-template <int NT>
+// SPLIT (first layer of an FP block): columns < split go to g_skip (rows, split), the others to g_in (rows, cin - split);
+// either may be NULL
+template <int NT, bool SPLIT>
 __global__ void __launch_bounds__(TG_THREADS, 2)
-train_linear_bwd_input_kernel(DzIn dz, WeightIn wt, float *__restrict__ g_in, long long tiles) {
+train_linear_bwd_input_kernel(DzIn dz, WeightIn wt, float *__restrict__ g_in, float *__restrict__ g_skip, int split, long long tiles) {
     using S = TileShape<NT>;
     extern __shared__ __align__(16) float smem[];
     const int cin = wt.n_total, cout = wt.k_total;
@@ -338,7 +455,18 @@ train_linear_bwd_input_kernel(DzIn dz, WeightIn wt, float *__restrict__ g_in, lo
         for (int i = 0; i < S::TM; ++i) {
             const long long r = m0 + ty * S::TM + i;
             if (r >= dz.rows) continue;
-            if (col + 3 < cin && (cin & 3) == 0) {
+            if constexpr (SPLIT) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const int cj = col + j;
+                    if (cj >= cin) continue;
+                    if (cj < split) {
+                        if (g_skip) g_skip[r * split + cj] = acc[i][j];
+                    } else if (g_in) {
+                        g_in[r * (cin - split) + (cj - split)] = acc[i][j];
+                    }
+                }
+            } else if (col + 3 < cin && (cin & 3) == 0) {
                 *reinterpret_cast<float4 *>(g_in + r * cin + col) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
             } else {
 #pragma unroll
@@ -352,9 +480,9 @@ train_linear_bwd_input_kernel(DzIn dz, WeightIn wt, float *__restrict__ g_in, lo
 // ---- backward, weight gradient: dW[co][ci] += sum_r dz[r][co] act_in(x)[r][ci] over a row range per CTA -----------------------
 // Both operands are contiguous along their channel (row-major activations), so the k-chunk (16 rows) is staged as it lies:
 // As[k][co], Bs[k][ci].  Output tile 128 (co) x NT (ci); the CTA walks its rows once per output tile.
-template <int NT, int MT>
+template <int NT, int MT, class LX>
 __global__ void __launch_bounds__(TG_THREADS, 2)
-train_linear_bwd_weight_kernel(DzIn dz, ActIn xin, float *__restrict__ dw, long long rows_per_cta) {
+train_linear_bwd_weight_kernel(DzIn dz, LX xin, float *__restrict__ dw, long long rows_per_cta) {
     using S = TileShape<NT, MT>;
     extern __shared__ __align__(16) float smem[];
     float *As = smem, *Bs = smem + 2 * TG_KC * S::AS;
@@ -376,7 +504,7 @@ train_linear_bwd_weight_kernel(DzIn dz, ActIn xin, float *__restrict__ dw, long 
                 for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
             constexpr int AQ = (MT * 4 + TG_THREADS - 1) / TG_THREADS;
             DzIn::Raw ra[AQ];
-            ActIn::Raw rb[BQ];
+            typename LX::Raw rb[BQ];
             // A chunk: 16 rows x MT co = MT * 4 float4: q -> (k = q / (MT / 4), co4 = q % (MT / 4));  B chunk: 16 rows x NT ci
             // rows past the CTA's range are read as rows past the end of the matrix (zeros)
             auto load = [&](long long r0) {  // long-latency loads only (see ActIn::raw)
@@ -456,6 +584,45 @@ train_bn_relu_scalar_kernel(long long total, int c, const float *__restrict__ z,
     }
 }
 
+// ---- last layer of an SA scale: BatchNorm + ReLU + max over the k rows of a group, the winning row kept for the backward ------
+// thread <-> (group, channel), lanes along channels: every z row is read coalesced; the (rows, c) activation is never written
+__global__ void __launch_bounds__(256)
+train_bn_relu_max_kernel(long long groups, int k, int c, const float *__restrict__ z, const float *__restrict__ scale,
+                         const float *__restrict__ shift, float *__restrict__ out, int out_stride, int out_offset,
+                         uint8_t *__restrict__ arg) {
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < groups * c; e += (long long)gridDim.x * 256) {
+        const long long gr = e / c;
+        const int ch = (int)(e - gr * c);
+        const float sc = __ldg(scale + ch), sh = __ldg(shift + ch);
+        const float *zr = z + gr * k * c + ch;
+        float best = fmaxf(fmaf(__ldg(zr), sc, sh), 0.f);
+        int bj = 0;
+        for (int j = 1; j < k; ++j) {
+            const float a = fmaxf(fmaf(__ldg(zr + (long long)j * c), sc, sh), 0.f);
+            if (a > best) {  // strict: the first maximum wins, as torch.max(dim) reports it
+                best = a;
+                bj = j;
+            }
+        }
+        out[gr * out_stride + out_offset + ch] = best;
+        arg[e] = (uint8_t)bj;
+    }
+}
+
+// ---- its backward: the pooled gradient on the winning row, 0 on the others; every element of g is written --------------------
+__global__ void __launch_bounds__(256)
+train_max_bwd_kernel(long long groups, int k, int c, const float *__restrict__ gp, int gp_stride, int gp_offset,
+                     const uint8_t *__restrict__ arg, float *__restrict__ g) {
+    const long long total = groups * k * c;
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < total; e += (long long)gridDim.x * 256) {
+        const long long row = e / c;
+        const int ch = (int)(e - row * c);
+        const long long gr = row / k;
+        const int j = (int)(row - gr * k);
+        g[e] = __ldg(arg + gr * c + ch) == j ? __ldg(gp + gr * gp_stride + gp_offset + ch) : 0.f;
+    }
+}
+
 // ---- per-channel coefficient kernels (one tiny launch instead of ~15 elementwise torch launches per layer and direction) ----
 // forward: (sum z, sum z^2) -> mean, biased var, rstd (fp64 -> fp32 where stored), scale = gamma rstd, shift = beta - mean scale;
 // running statistics updated like torch.nn.BatchNorm in training mode (momentum, UNBIASED variance).
@@ -504,20 +671,11 @@ int pick_nt(int n) { return n <= 32 ? 32 : (n <= 64 ? 64 : 128); }
 template <int NT>
 size_t tile_smem() { return TileShape<NT>::smem_floats * sizeof(float); }
 
-}  // namespace
-}  // namespace pn2
 
-using namespace pn2;
-
-extern "C" int pn2_train_linear_fwd(long long rows, int cin, int cout, const float *x, const float *in_scale, const float *in_shift,
-                                    const float *w, const float *bias, float *z, double *stats, void *stream) {
-    PN2_REQUIRE(rows >= 0 && cin >= 1 && cout >= 1, "train_linear_fwd: bad dims rows=%lld cin=%d cout=%d", rows, cin, cout);
-    if (rows == 0) return PN2_OK;
-    PN2_REQUIRE(x && w && bias && z && stats && ((in_scale == nullptr) == (in_shift == nullptr)), "train_linear_fwd: null pointer");
-    PN2_REQUIRE((((uintptr_t)x | (uintptr_t)w | (uintptr_t)z | (uintptr_t)in_scale | (uintptr_t)in_shift) & 15) == 0, "train_linear_fwd: 16-byte alignment");
-    cudaStream_t s = (cudaStream_t)stream;
-    ActIn a = {x, in_scale, in_shift, rows, cin};
-    WeightIn b = {w, cout, cin};
+template <class LX>
+int launch_fwd(const LX &a, const WeightIn &b, const float *bias, float *z, double *stats, cudaStream_t s) {
+    const long long rows = a.rows;
+    const int cout = b.n_total;
     const long long tiles = (rows + TG_M - 1) / TG_M;
     const int nt = pick_nt(cout);
     const long long work = tiles * ((cout + nt - 1) / nt);
@@ -531,6 +689,112 @@ extern "C" int pn2_train_linear_fwd(long long rows, int cin, int cout, const flo
     }
     PN2_LAUNCH_OK("train_linear_fwd_kernel");
     return PN2_OK;
+}
+
+// g_in = dz W (split: see train_linear_bwd_input_kernel), then dW += dz^T x
+template <class LX>
+int launch_bwd(const DzIn &dz, const LX &a, const float *wt, float *g_in, float *g_skip, int split, float *dw, cudaStream_t s) {
+    const long long rows = dz.rows;
+    const int cin = a.c, cout = dz.c;
+    const long long tiles = (rows + TG_M - 1) / TG_M;
+    if (g_in || g_skip) {
+        WeightIn b = {wt, cin, cout};
+        const int nt = pick_nt(cin);
+        const long long work = tiles * ((cin + nt - 1) / nt);
+        const unsigned grid = (unsigned)(work < 2ll * sm_count() ? work : 2ll * sm_count());
+#define PN2_BI(NTV, SPL) train_linear_bwd_input_kernel<NTV, SPL><<<grid, TG_THREADS, tile_smem<NTV>(), s>>>(dz, b, g_in, g_skip, split, tiles)
+        if (split > 0) {
+            if (nt == 32) PN2_BI(32, true); else if (nt == 64) PN2_BI(64, true); else PN2_BI(128, true);
+        } else {
+            if (nt == 32) PN2_BI(32, false); else if (nt == 64) PN2_BI(64, false); else PN2_BI(128, false);
+        }
+#undef PN2_BI
+        PN2_LAUNCH_OK("train_linear_bwd_input_kernel");
+    }
+    {
+        // grid = (row ranges, output tiles): about four CTAs per SM in total, at least 128 rows per range (the partial sums
+        // go to dW with atomics)
+        // output tile (cout x cin) = mt x nt: no padded FMAs for narrow layers.  The interpolated operand stages three source
+        // rows per element: its 128 x 128 tile spilled (412 bytes), so it stays at 64 input channels per tile.
+        constexpr bool wide_ok = !std::is_same<LX, InterpIn>::value;
+        const int nt = wide_ok ? pick_nt(cin) : min(pick_nt(cin), 64), mt = pick_nt(cout);
+        const long long out_tiles = (long long)((cout + mt - 1) / mt) * ((cin + nt - 1) / nt);
+        PN2_REQUIRE(out_tiles <= 65535, "train_linear_bwd: too many output tiles");
+        long long ranges = (4ll * sm_count() + out_tiles - 1) / out_tiles;
+        long long per = (rows + ranges - 1) / ranges;
+        if (per < 128) per = 128;
+        per = (per + TG_KC - 1) / TG_KC * TG_KC;
+        ranges = (rows + per - 1) / per;
+        const dim3 grid((unsigned)ranges, (unsigned)out_tiles);
+#define PN2_WG(NTV, MTV) train_linear_bwd_weight_kernel<NTV, MTV><<<grid, TG_THREADS, TileShape<NTV, MTV>::smem_floats * sizeof(float), s>>>(dz, a, dw, per)
+        if (mt == 32) {
+            if (nt == 32) PN2_WG(32, 32); else if (nt == 64) PN2_WG(64, 32); else if constexpr (wide_ok) PN2_WG(128, 32);
+        } else if (mt == 64) {
+            if (nt == 32) PN2_WG(32, 64); else if (nt == 64) PN2_WG(64, 64); else if constexpr (wide_ok) PN2_WG(128, 64);
+        } else {
+            if (nt == 32) PN2_WG(32, 128); else if (nt == 64) PN2_WG(64, 128); else if constexpr (wide_ok) PN2_WG(128, 128);
+        }
+#undef PN2_WG
+        PN2_LAUNCH_OK("train_linear_bwd_weight_kernel");
+    }
+    return PN2_OK;
+}
+
+bool aligned16(const void *p) { return ((uintptr_t)p & 15) == 0; }
+
+// Validates a pn2_rows against (rows, cin) and builds its loader.  Returns PN2_OK or the error status.
+int rows_loader(const char *who, long long rows, int cin, const pn2_rows *src, GroupIn &gi, InterpIn &ii) {
+    PN2_REQUIRE(src, "%s: null row source", who);
+    PN2_REQUIRE(src->kind == PN2_ROWS_GROUPED || src->kind == PN2_ROWS_INTERP, "%s: unknown row source kind %d", who, src->kind);
+    PN2_REQUIRE(rows < (1ll << 31), "%s: more than 2^31 rows", who);
+    const pn2_rows &r = *src;
+    if (r.kind == PN2_ROWS_GROUPED) {
+        PN2_REQUIRE(r.b >= 1 && r.n >= 1 && r.m >= 1 && r.k >= 1 && r.d >= 0 && (r.order == PN2_ORDER_XYZ_FIRST || r.order == PN2_ORDER_FEAT_FIRST),
+                    "%s: bad grouped source b=%d n=%d m=%d k=%d d=%d order=%d", who, r.b, r.n, r.m, r.k, r.d, r.order);
+        PN2_REQUIRE(rows == (long long)r.b * r.m * r.k && cin == 3 + r.d, "%s: rows=%lld cin=%d do not match the grouped source", who, rows, cin);
+        PN2_REQUIRE(r.xyz && r.new_xyz && r.idx && ((r.feat == nullptr) == (r.d == 0)), "%s: null pointer", who);
+        const bool xyz_first = r.order == PN2_ORDER_XYZ_FIRST;
+        gi = {r.xyz, r.new_xyz, r.feat, r.idx, rows, cin, r.n, r.m, r.k, r.d, xyz_first ? 0 : r.d, xyz_first ? 3 : 0,
+              r.d > 0 && (r.d & 3) == 0 && aligned16(r.feat)};
+    } else {
+        PN2_REQUIRE(r.b >= 1 && r.n >= 1 && r.m >= 1 && r.d >= 1 && r.d_skip >= 0, "%s: bad interpolated source b=%d n=%d m=%d d=%d d_skip=%d",
+                    who, r.b, r.n, r.m, r.d, r.d_skip);
+        PN2_REQUIRE(rows == (long long)r.b * r.n && cin == r.d_skip + r.d, "%s: rows=%lld cin=%d do not match the interpolated source", who,
+                    rows, cin);
+        PN2_REQUIRE(r.feat && ((r.skip == nullptr) == (r.d_skip == 0)) && (r.m == 1 || (r.idx && r.weight)), "%s: null pointer", who);
+        ii = {r.skip, r.feat, r.weight, r.m == 1 ? nullptr : r.idx, rows, cin, r.n, r.m, r.d, r.d_skip,
+              r.d_skip > 0 && (r.d_skip & 3) == 0 && aligned16(r.skip), (r.d & 3) == 0 && aligned16(r.feat)};
+    }
+    return PN2_OK;
+}
+
+}  // namespace
+}  // namespace pn2
+
+using namespace pn2;
+
+extern "C" int pn2_train_linear_fwd(long long rows, int cin, int cout, const float *x, const float *in_scale, const float *in_shift,
+                                    const float *w, const float *bias, float *z, double *stats, void *stream) {
+    PN2_REQUIRE(rows >= 0 && cin >= 1 && cout >= 1, "train_linear_fwd: bad dims rows=%lld cin=%d cout=%d", rows, cin, cout);
+    if (rows == 0) return PN2_OK;
+    PN2_REQUIRE(x && w && bias && z && stats && ((in_scale == nullptr) == (in_shift == nullptr)), "train_linear_fwd: null pointer");
+    PN2_REQUIRE((((uintptr_t)x | (uintptr_t)w | (uintptr_t)z | (uintptr_t)in_scale | (uintptr_t)in_shift) & 15) == 0, "train_linear_fwd: 16-byte alignment");
+    ActIn a = {x, in_scale, in_shift, rows, cin};
+    return launch_fwd(a, WeightIn{w, cout, cin}, bias, z, stats, (cudaStream_t)stream);
+}
+
+extern "C" int pn2_train_linear_fwd_rows(long long rows, int cin, int cout, const pn2_rows *src, const float *w, const float *bias,
+                                         float *z, double *stats, void *stream) {
+    PN2_REQUIRE(rows >= 0 && cin >= 1 && cout >= 1, "train_linear_fwd_rows: bad dims rows=%lld cin=%d cout=%d", rows, cin, cout);
+    if (rows == 0) return PN2_OK;
+    GroupIn gi;
+    InterpIn ii;
+    if (int st = rows_loader("train_linear_fwd_rows", rows, cin, src, gi, ii)) return st;
+    PN2_REQUIRE(w && bias && z && stats, "train_linear_fwd_rows: null pointer");
+    PN2_REQUIRE((((uintptr_t)w | (uintptr_t)z) & 15) == 0, "train_linear_fwd_rows: 16-byte alignment");
+    const WeightIn b = {w, cout, cin};
+    cudaStream_t s = (cudaStream_t)stream;
+    return src->kind == PN2_ROWS_GROUPED ? launch_fwd(gi, b, bias, z, stats, s) : launch_fwd(ii, b, bias, z, stats, s);
 }
 
 extern "C" int pn2_train_bn_bwd_reduce(long long rows, int c, const float *g, const float *z, const float *scale, const float *shift,
@@ -557,44 +821,30 @@ extern "C" int pn2_train_linear_bwd(long long rows, int cin, int cout, const flo
                 "train_linear_bwd: 16-byte alignment");
     PN2_REQUIRE((cout & 3) != 0 || (((uintptr_t)scale | (uintptr_t)shift | (uintptr_t)ca | (uintptr_t)cb | (uintptr_t)cc) & 15) == 0,
                 "train_linear_bwd: 16-byte alignment of the per-channel vectors");
-    cudaStream_t s = (cudaStream_t)stream;
     DzIn dz = {g, z, scale, shift, ca, cb, cc, rows, cout};
     ActIn a = {x, in_scale, in_shift, rows, cin};
-    const long long tiles = (rows + TG_M - 1) / TG_M;
-    if (g_in) {
-        WeightIn b = {wt, cin, cout};
-        const int nt = pick_nt(cin);
-        const long long work = tiles * ((cin + nt - 1) / nt);
-        const unsigned grid = (unsigned)(work < 2ll * sm_count() ? work : 2ll * sm_count());
-        if (nt == 32) train_linear_bwd_input_kernel<32><<<grid, TG_THREADS, tile_smem<32>(), s>>>(dz, b, g_in, tiles);
-        else if (nt == 64) train_linear_bwd_input_kernel<64><<<grid, TG_THREADS, tile_smem<64>(), s>>>(dz, b, g_in, tiles);
-        else train_linear_bwd_input_kernel<128><<<grid, TG_THREADS, tile_smem<128>(), s>>>(dz, b, g_in, tiles);
-        PN2_LAUNCH_OK("train_linear_bwd_input_kernel");
-    }
-    {
-        // grid = (row ranges, output tiles): about four CTAs per SM in total, at least 128 rows per range (the partial sums
-        // go to dW with atomics)
-        const int nt = pick_nt(cin), mt = pick_nt(cout);  // output tile (cout x cin) = mt x nt: no padded FMAs for narrow layers
-        const long long out_tiles = (long long)((cout + mt - 1) / mt) * ((cin + nt - 1) / nt);
-        PN2_REQUIRE(out_tiles <= 65535, "train_linear_bwd: too many output tiles");
-        long long ranges = (4ll * sm_count() + out_tiles - 1) / out_tiles;
-        long long per = (rows + ranges - 1) / ranges;
-        if (per < 128) per = 128;
-        per = (per + TG_KC - 1) / TG_KC * TG_KC;
-        ranges = (rows + per - 1) / per;
-        const dim3 grid((unsigned)ranges, (unsigned)out_tiles);
-#define PN2_WG(NTV, MTV) train_linear_bwd_weight_kernel<NTV, MTV><<<grid, TG_THREADS, TileShape<NTV, MTV>::smem_floats * sizeof(float), s>>>(dz, a, dw, per)
-        if (mt == 32) {
-            if (nt == 32) PN2_WG(32, 32); else if (nt == 64) PN2_WG(64, 32); else PN2_WG(128, 32);
-        } else if (mt == 64) {
-            if (nt == 32) PN2_WG(32, 64); else if (nt == 64) PN2_WG(64, 64); else PN2_WG(128, 64);
-        } else {
-            if (nt == 32) PN2_WG(32, 128); else if (nt == 64) PN2_WG(64, 128); else PN2_WG(128, 128);
-        }
-#undef PN2_WG
-        PN2_LAUNCH_OK("train_linear_bwd_weight_kernel");
-    }
-    return PN2_OK;
+    return launch_bwd(dz, a, wt, g_in, nullptr, 0, dw, (cudaStream_t)stream);
+}
+
+extern "C" int pn2_train_linear_bwd_rows(long long rows, int cin, int cout, const pn2_rows *src, const float *wt, const float *g,
+                                         const float *z, const float *scale, const float *shift, const float *ca, const float *cb,
+                                         const float *cc, float *g_in, float *g_skip, float *dw, void *stream) {
+    PN2_REQUIRE(rows >= 0 && cin >= 1 && cout >= 1, "train_linear_bwd_rows: bad dims rows=%lld cin=%d cout=%d", rows, cin, cout);
+    if (rows == 0) return PN2_OK;
+    GroupIn gi;
+    InterpIn ii;
+    if (int st = rows_loader("train_linear_bwd_rows", rows, cin, src, gi, ii)) return st;
+    PN2_REQUIRE(wt && g && z && scale && shift && ca && cb && cc && dw, "train_linear_bwd_rows: null pointer");
+    PN2_REQUIRE(g_skip == nullptr || (src->kind == PN2_ROWS_INTERP && src->d_skip > 0),
+                "train_linear_bwd_rows: g_skip needs an interpolated source with skip columns (d_skip > 0)");
+    PN2_REQUIRE((((uintptr_t)wt | (uintptr_t)g | (uintptr_t)z | (uintptr_t)g_in) & 15) == 0, "train_linear_bwd_rows: 16-byte alignment");
+    PN2_REQUIRE((cout & 3) != 0 || (((uintptr_t)scale | (uintptr_t)shift | (uintptr_t)ca | (uintptr_t)cb | (uintptr_t)cc) & 15) == 0,
+                "train_linear_bwd_rows: 16-byte alignment of the per-channel vectors");
+    DzIn dz = {g, z, scale, shift, ca, cb, cc, rows, cout};
+    cudaStream_t s = (cudaStream_t)stream;
+    if (src->kind == PN2_ROWS_GROUPED) return launch_bwd(dz, gi, wt, g_in, nullptr, 0, dw, s);
+    // an FP block's skip columns come first: split them off into g_skip (without skip columns g_in is (rows, cin))
+    return launch_bwd(dz, ii, wt, g_in, g_skip, src->d_skip, dw, s);
 }
 
 extern "C" int pn2_train_bn_relu(long long rows, int c, const float *z, const float *scale, const float *shift, float *a, void *stream) {
@@ -633,5 +883,31 @@ extern "C" int pn2_train_bn_bwd_coeffs(long long rows, int c, const double *sums
     PN2_REQUIRE(sums && mean_rstd && gamma && coef && dgamma && dbeta, "train_bn_bwd_coeffs: null pointer");
     train_bn_bwd_coeffs_kernel<<<(c + 127) / 128, 128, 0, (cudaStream_t)stream>>>(c, (double)rows, sums, mean_rstd, gamma, coef, dgamma, dbeta);
     PN2_LAUNCH_OK("train_bn_bwd_coeffs_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_train_bn_relu_max(long long groups, int k, int c, const float *z, const float *scale, const float *shift, float *out,
+                                     int out_stride, int out_offset, uint8_t *arg, void *stream) {
+    PN2_REQUIRE(groups >= 0 && k >= 1 && k <= 256 && c >= 1, "train_bn_relu_max: bad dims groups=%lld k=%d c=%d (k <= 256)", groups, k, c);
+    PN2_REQUIRE(out_offset >= 0 && out_stride >= out_offset + c, "train_bn_relu_max: out_stride=%d out_offset=%d c=%d", out_stride, out_offset, c);
+    if (groups == 0) return PN2_OK;
+    PN2_REQUIRE(z && scale && shift && out && arg, "train_bn_relu_max: null pointer");
+    const long long total = groups * c;
+    const unsigned grid = (unsigned)((total + 255) / 256 < 8ll * sm_count() ? (total + 255) / 256 : 8ll * sm_count());
+    train_bn_relu_max_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(groups, k, c, z, scale, shift, out, out_stride, out_offset, arg);
+    PN2_LAUNCH_OK("train_bn_relu_max_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_train_max_bwd(long long groups, int k, int c, const float *gp, int gp_stride, int gp_offset, const uint8_t *arg,
+                                 float *g, void *stream) {
+    PN2_REQUIRE(groups >= 0 && k >= 1 && k <= 256 && c >= 1, "train_max_bwd: bad dims groups=%lld k=%d c=%d (k <= 256)", groups, k, c);
+    PN2_REQUIRE(gp_offset >= 0 && gp_stride >= gp_offset + c, "train_max_bwd: gp_stride=%d gp_offset=%d c=%d", gp_stride, gp_offset, c);
+    if (groups == 0) return PN2_OK;
+    PN2_REQUIRE(gp && arg && g, "train_max_bwd: null pointer");
+    const long long total = groups * k * c;
+    const unsigned grid = (unsigned)((total + 255) / 256 < 8ll * sm_count() ? (total + 255) / 256 : 8ll * sm_count());
+    train_max_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(groups, k, c, gp, gp_stride, gp_offset, arg, g);
+    PN2_LAUNCH_OK("train_max_bwd_kernel");
     return PN2_OK;
 }

@@ -15,6 +15,7 @@ LIB_PATH = os.path.join(CSRC, "libpn2_b200.so")
 PN2_MAX_LAYERS = 6
 REDUCE_MAX, REDUCE_FIRST = 0, 1
 ORDER_XYZ_FIRST, ORDER_FEAT_FIRST = 0, 1
+ROWS_GROUPED, ROWS_INTERP = 1, 2
 FLAG_IN_BF16, FLAG_SKIP_BF16, FLAG_OUT_BF16, FLAG_OUT_ARGMAX = 1, 2, 4, 8
 
 _c_int, _c_float, _vp = ctypes.c_int, ctypes.c_float, ctypes.c_void_p
@@ -29,6 +30,15 @@ class Pn2Mlp(ctypes.Structure):
                 ("weight", _vp * PN2_MAX_LAYERS),
                 ("bias", _vp * PN2_MAX_LAYERS)]
 
+
+class Pn2Rows(ctypes.Structure):
+    """struct pn2_rows (include/pn2_abi.h)"""
+    _fields_ = [("kind", _c_int), ("order", _c_int),
+                ("b", _c_int), ("n", _c_int), ("m", _c_int), ("k", _c_int), ("d", _c_int), ("d_skip", _c_int),
+                ("xyz", _vp), ("new_xyz", _vp), ("feat", _vp), ("skip", _vp), ("idx", _vp), ("weight", _vp)]
+
+
+_ROWS = ctypes.POINTER(Pn2Rows)
 
 # name -> argtypes; every function returns int (pn2_status) unless listed in _OTHER
 _SIGNATURES = {
@@ -49,6 +59,7 @@ _SIGNATURES = {
     "pn2_label_counts": [_c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "pn2_inverse_index": [_c_int, _c_int, ctypes.c_longlong, _vp, _vp, _vp, _vp],
     "pn2_scatter_rows_det": [_c_int, _c_int, _c_int, ctypes.c_longlong, _c_int, _vp, _vp, _vp, _vp, _vp, _vp],
+    "pn2_scatter_rows_det_cl": [_c_int, _c_int, _c_int, ctypes.c_longlong, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp],
     "pn2_lift_views": [_c_int] * 6 + [_vp] * 7 + [ctypes.POINTER(_c_float)] + [_c_float] * 3 + [_c_int] + [_vp] * 4,
     "pn2_lift_views_poses": [_c_int] * 6 + [_vp] * 4 + [ctypes.POINTER(_c_float)] * 2 + [_c_float] * 3 + [_c_int] + [_vp] * 4,
     "pn2_lift_views_grad": [_c_int] * 6 + [_vp, _vp, _c_int, _vp, _vp, _vp],
@@ -69,6 +80,10 @@ _SIGNATURES = {
     "pn2_train_bn_relu": [ctypes.c_longlong, _c_int] + [_vp] * 5,
     "pn2_train_bn_bwd_reduce": [ctypes.c_longlong, _c_int] + [_vp] * 6,
     "pn2_train_linear_bwd": [ctypes.c_longlong, _c_int, _c_int] + [_vp] * 14,
+    "pn2_train_linear_fwd_rows": [ctypes.c_longlong, _c_int, _c_int, _ROWS] + [_vp] * 5,
+    "pn2_train_linear_bwd_rows": [ctypes.c_longlong, _c_int, _c_int, _ROWS] + [_vp] * 12,
+    "pn2_train_bn_relu_max": [ctypes.c_longlong, _c_int, _c_int] + [_vp] * 4 + [_c_int, _c_int, _vp, _vp],
+    "pn2_train_max_bwd": [ctypes.c_longlong, _c_int, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
 }
 _OTHER = {
     "pn2_last_error": ([], ctypes.c_char_p),

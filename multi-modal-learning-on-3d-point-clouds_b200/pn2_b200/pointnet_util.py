@@ -13,8 +13,11 @@ Two execution paths per module:
     grouping, centring, concat, every 1x1 conv with its eval BatchNorm folded in, ReLU and the max
     over nsample never leave shared memory (csrc/row_mlp.cu).  Activations are channel-last inside;
     `forward_cl` exposes that layout so a whole network can stay in it (pn2_b200/models.py).
-  * training (batch statistics / autograd): the reference's own composition of operators -- our
-    kernels for the geometry, torch.nn for conv/BN -- with identical semantics.
+  * training (batch statistics / autograd): one autograd Function per SA scale / FP block (pn2_b200/train_mlp.py):
+    the first layer reads the grouped / interpolated rows where they lie, the last one pools, the backward scatters the
+    input gradients without atomics; with deterministic algorithms, set_fused_training(False) or coordinates that need a
+    gradient, the reference's own composition of operators -- our kernels for the geometry, torch.nn for conv/BN.  Both
+    with identical semantics.
 """
 import ctypes
 import os
@@ -46,6 +49,50 @@ def _train_fused(module, x0, convs, bns):
     if not (_FUSED_TRAINING and module.training) or pointnet2_utils._deterministic():
         return False
     return train_mlp.fusable_training(x0, convs, bns)
+
+
+def _train_blocks(module, convs, bns, xyzs, feats, nsample=None):
+    """Training-mode block Functions (train_mlp.sa_scale_train / fp_block_train): wherever the fused training chain runs,
+    for fp32 CUDA inputs, coordinates that need no gradient and at most 256 samples per ball (the pooled arg-max is uint8)."""
+    if not _train_fused(module, xyzs[0], convs, bns):
+        return False
+    if any(t.requires_grad for t in xyzs):
+        return False
+    if not all(t is None or (t.is_cuda and t.dtype == torch.float32) for t in list(xyzs) + list(feats)):
+        return False
+    return nsample is None or nsample <= 256
+
+
+def _cl_view(x):
+    """(B, C, N) -> (B, N, C) under autograd: the permuted view itself when x is a permuted channel-last tensor (what every
+    block after the first receives), else a contiguous copy."""
+    t = x.permute(0, 2, 1)
+    return t if t.is_contiguous() else t.contiguous()
+
+
+def _cl_xyz(xyz):
+    """Coordinates (B, 3, N) that need no gradient -> contiguous (B, N, 3), without a copy when they already lie so."""
+    t = xyz.permute(0, 2, 1)
+    return t if t.is_contiguous() else to_channel_last(xyz)
+
+
+def _sampled(xyz_cl, xyz, npoint, fps_idx):
+    """new_xyz (B, npoint, 3) of the furthest point sampling, or of the caller's `fps_idx`."""
+    if fps_idx is None:
+        return fps_gather_cl(xyz_cl, npoint)[1]
+    return pointnet2_utils.gather_operation(xyz.contiguous(), fps_idx).permute(0, 2, 1).contiguous()
+
+
+def _three_nn_weights_torch(xyz1_t, xyz2_t):
+    """three_nn + the reference's weight formula (model/pointnet_util.py:205-208) as torch operators: xyz1 (B, n, 3),
+    xyz2 (B, m, 3) -> idx, weight (B, n, 3).  pn2_three_nn_weights computes the same formula in one kernel but differs
+    from it in the last bit of some weights, so training keeps these."""
+    B, N, _ = xyz1_t.shape
+    dist, idx = pointnet2_utils.three_nn(xyz1_t, xyz2_t)
+    dist = torch.where(dist < 1e-10, torch.full_like(dist, 1e-10), dist)
+    weight = 1.0 / dist
+    weight = weight / torch.sum(weight, dim=-1).view(B, N, 1)
+    return idx, weight
 
 
 def timeit(tag, t):
@@ -495,6 +542,13 @@ class PointNetSetAbstraction(nn.Module):
         if self._fused_ok(xyz, points):
             new_xyz, out = self.forward_cl(to_channel_last(xyz), to_channel_last(points))
             return new_xyz.permute(0, 2, 1), to_channel_first(out)
+        if not self.group_all and _train_blocks(self, self.mlp_convs, self.mlp_bns, [xyz], [points], self.nsample):
+            xyz_cl = _cl_xyz(xyz)
+            new_xyz = _sampled(xyz_cl, xyz, self.npoint, fps_idx)
+            idx = pointnet2_utils.ball_query(self.radius, self.nsample, xyz_cl, new_xyz)
+            out = train_mlp.sa_scale_train(xyz_cl, new_xyz, idx, _cl_view(points) if points is not None else None,
+                                           _lib.ORDER_XYZ_FIRST, self.mlp_convs, self.mlp_bns)
+            return new_xyz.permute(0, 2, 1), out.permute(0, 2, 1)
         xyz_t = xyz.permute(0, 2, 1)
         pts_t = points.permute(0, 2, 1) if points is not None else None
         if self.group_all:
@@ -583,17 +637,27 @@ class PointNetSetAbstractionMsg(nn.Module):
             new_xyz, out = self.forward_cl(to_channel_last(xyz), to_channel_last(points))
             return new_xyz.permute(0, 2, 1), to_channel_first(out)
         xyz_t = xyz.permute(0, 2, 1)
-        pts_cf = points.contiguous() if points is not None else None
         B, N, C = xyz_t.shape
         S = self.npoint
-        xyz_c, xyz_cf = xyz_t.contiguous(), xyz.contiguous()
-        if fps_idx is None:
-            fps_idx = pointnet2_utils.furthest_point_sample(xyz_c, S)
-        new_xyz = pointnet2_utils.gather_operation(xyz_cf, fps_idx).permute(0, 2, 1).contiguous()
+        blocks = all(_train_blocks(self, self.conv_blocks[i], self.bn_blocks[i], [xyz], [points], k)
+                     for i, k in enumerate(self.nsample_list))
+        if blocks:
+            xyz_c = _cl_xyz(xyz)
+            feat_cl = _cl_view(points) if points is not None else None
+            new_xyz = _sampled(xyz_c, xyz, S, fps_idx)
+        else:
+            pts_cf = points.contiguous() if points is not None else None
+            xyz_c, xyz_cf = xyz_t.contiguous(), xyz.contiguous()
+            if fps_idx is None:
+                fps_idx = pointnet2_utils.furthest_point_sample(xyz_c, S)
+            new_xyz = pointnet2_utils.gather_operation(xyz_cf, fps_idx).permute(0, 2, 1).contiguous()
 
         def scale(i):
             radius, K = self.radius_list[i], self.nsample_list[i]
             idx = pointnet2_utils.ball_query(radius, K, xyz_c, new_xyz)
+            if blocks:  # (B, S, C_i) channel-last; features first, centred xyz last (:157)
+                return train_mlp.sa_scale_train(xyz_c, new_xyz, idx, feat_cl, _lib.ORDER_FEAT_FIRST, self.conv_blocks[i],
+                                                self.bn_blocks[i])
             grouped_xyz = pointnet2_utils.grouping_operation(xyz_cf, idx).permute(0, 2, 3, 1).contiguous()
             grouped_xyz = grouped_xyz - new_xyz.view(B, S, 1, C)
             if pts_cf is not None:
@@ -634,6 +698,8 @@ class PointNetSetAbstractionMsg(nn.Module):
                 cur.wait_stream(st)
                 if not torch.cuda.is_current_stream_capturing():
                     outs[i].record_stream(cur)  # allocated on the side stream, consumed on the caller's
+        if blocks:
+            return new_xyz.permute(0, 2, 1), torch.cat(outs, dim=2).permute(0, 2, 1)
         return new_xyz.permute(0, 2, 1), torch.cat(outs, dim=1)
 
 
@@ -683,6 +749,11 @@ class PointNetFeaturePropagation(nn.Module):
             out = self.forward_cl(to_channel_last(xyz1), to_channel_last(xyz2), to_channel_last(points1),
                                   to_channel_last(points2))
             return to_channel_first(out)
+        if _train_blocks(self, self.mlp_convs, self.mlp_bns, [xyz1, xyz2], [points1, points2]):
+            idx, w = (None, None) if xyz2.shape[2] == 1 else _three_nn_weights_torch(_cl_xyz(xyz1), _cl_xyz(xyz2))
+            out = train_mlp.fp_block_train(_cl_view(points1) if points1 is not None else None, _cl_view(points2), idx, w,
+                                           self.mlp_convs, self.mlp_bns, xyz1.shape[2])
+            return out.permute(0, 2, 1)
         xyz1_t = xyz1.permute(0, 2, 1).contiguous()
         xyz2_t = xyz2.permute(0, 2, 1).contiguous()
         B, N, _ = xyz1_t.shape
@@ -690,10 +761,7 @@ class PointNetFeaturePropagation(nn.Module):
         if S == 1:
             interpolated = points2.permute(0, 2, 1).repeat(1, N, 1)
         else:
-            dist, idx = pointnet2_utils.three_nn(xyz1_t, xyz2_t)
-            dist = torch.where(dist < 1e-10, torch.full_like(dist, 1e-10), dist)
-            weight = 1.0 / dist
-            weight = weight / torch.sum(weight, dim=-1).view(B, N, 1)
+            idx, weight = _three_nn_weights_torch(xyz1_t, xyz2_t)
             interpolated = pointnet2_utils.three_interpolate(points2.contiguous(), idx, weight).permute(0, 2, 1)
         if points1 is not None:
             new_points = torch.cat([points1.permute(0, 2, 1), interpolated], dim=-1)  # skip features FIRST (:213)

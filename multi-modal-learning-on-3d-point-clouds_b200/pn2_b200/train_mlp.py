@@ -19,6 +19,80 @@ def _stream(t):
     return _lib.stream_ptr(t.device)
 
 
+def _forward_layers(R, meta, tensors, dev, st, first):
+    """The per-layer forward of a stack of L = len(tensors) // 6 layers over R rows; `first(cin, cout, W, b, z, stats)`
+    issues layer 0's forward (its operand is the caller's), layers 1.. read the previous z through act_in.
+    -> (zs, scales, shifts, mrs), per layer."""
+    L = len(tensors) // 6
+    zs, scales, shifts, mrs = [], [], [], []
+    for l in range(L):
+        W, b, gamma, beta, rmean, rvar = tensors[6 * l:6 * l + 6]
+        eps, momentum = meta[l]
+        cout, cin = W.shape
+        Wc, bc = W.detach().contiguous(), b.detach().contiguous()
+        gc, bec = gamma.detach().contiguous(), beta.detach().contiguous()
+        z = torch.empty((R, cout), dtype=torch.float32, device=dev)
+        stats = torch.zeros((2, cout), dtype=torch.float64, device=dev)
+        if l == 0:
+            first(cin, cout, Wc, bc, z, stats)
+        else:
+            _lib.call("pn2_train_linear_fwd", R, cin, cout, ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(Wc), ptr(bc), ptr(z),
+                      ptr(stats), st)
+        scale = torch.empty(cout, dtype=torch.float32, device=dev)
+        shift = torch.empty(cout, dtype=torch.float32, device=dev)
+        mr = torch.empty((2, cout), dtype=torch.float64, device=dev)
+        _lib.call("pn2_train_bn_finalize", R, cout, ptr(stats), ptr(gc), ptr(bec), float(eps), float(momentum), ptr(scale), ptr(shift),
+                  ptr(mr), ptr(rmean), ptr(rvar), st)
+        zs.append(z); scales.append(scale); shifts.append(shift); mrs.append(mr)
+    return zs, scales, shifts, mrs
+
+
+def _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first):
+    """The per-layer backward from g = dL/da_L (R, C_L) down to layer 0; `first(cin, cout, Wt, g, z, scale, shift, coef, dW)`
+    issues layer 0's backward and returns its input gradient(s).  -> (that return value, parameter gradients)."""
+    L = len(zs)
+    grads = [None] * (6 * L)
+    out = None
+    for l in range(L - 1, -1, -1):
+        W, b, gamma, beta = params[4 * l:4 * l + 4]
+        cout, cin = W.shape
+        z, scale, shift, mr = zs[l], scales[l], shifts[l], mrs[l]
+        sums = torch.zeros((2, cout), dtype=torch.float64, device=dev)
+        _lib.call("pn2_train_bn_bwd_reduce", R, cout, ptr(g), ptr(z), ptr(scale), ptr(shift), ptr(sums), st)
+        coef = torch.empty((3, cout), dtype=torch.float32, device=dev)
+        dgamma = torch.empty(cout, dtype=torch.float32, device=dev)
+        dbeta = torch.empty(cout, dtype=torch.float32, device=dev)
+        gc = gamma.detach().contiguous()
+        _lib.call("pn2_train_bn_bwd_coeffs", R, cout, ptr(sums), ptr(mr), ptr(gc), ptr(coef), ptr(dgamma), ptr(dbeta), st)
+        dW = torch.zeros((cout, cin), dtype=torch.float32, device=dev)
+        Wt = torch.empty((cin, cout), dtype=torch.float32, device=dev)
+        _lib.call("pn2_transpose", 1, cout, cin, ptr(W.detach().contiguous()), ptr(Wt), st)  # W^T: an exact copy, one launch
+        if l == 0:
+            out = first(cin, cout, Wt, g, z, scale, shift, coef, dW)
+        else:
+            g_in = torch.empty((R, cin), dtype=torch.float32, device=dev)
+            _lib.call("pn2_train_linear_bwd", R, cin, cout, ptr(zs[l - 1]), ptr(scales[l - 1]), ptr(shifts[l - 1]), ptr(Wt), ptr(g),
+                      ptr(z), ptr(scale), ptr(shift), ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), ptr(dW), st)
+            g = g_in
+        grads[6 * l] = dW.view_as(W)
+        grads[6 * l + 1] = torch.zeros_like(b)   # a bias in front of a batch-statistics BatchNorm has zero gradient
+        grads[6 * l + 2] = dgamma
+        grads[6 * l + 3] = dbeta
+    return out, grads
+
+
+def _saved_layers(saved, L):
+    zs, scales, shifts, mrs = saved[:L], saved[L:2 * L], saved[2 * L:3 * L], saved[3 * L:4 * L]
+    return zs, scales, shifts, mrs, saved[4 * L:]
+
+
+def _params(tensors, L):
+    params = []
+    for l in range(L):
+        params += list(tensors[6 * l:6 * l + 4])
+    return params
+
+
 class _FusedMlpTrain(Function):
     @staticmethod
     def forward(ctx, x0, meta, *tensors):
@@ -29,80 +103,200 @@ class _FusedMlpTrain(Function):
         R = x0.shape[0]
         dev = x0.device
         x0 = _lib.check_f32(x0, "x0")
-        zs, scales, shifts, mrs = [], [], [], []
-        in_scale = in_shift = None
-        x = x0
         st = _stream(x0)
         with torch.cuda.device(dev):
-            for l in range(L):
-                W, b, gamma, beta, rmean, rvar = tensors[6 * l:6 * l + 6]
-                eps, momentum = meta[l]
-                cout, cin = W.shape
-                Wc, bc = W.detach().contiguous(), b.detach().contiguous()
-                gc, bec = gamma.detach().contiguous(), beta.detach().contiguous()
-                z = torch.empty((R, cout), dtype=torch.float32, device=dev)
-                stats = torch.zeros((2, cout), dtype=torch.float64, device=dev)
-                _lib.call("pn2_train_linear_fwd", R, cin, cout, ptr(x), ptr(in_scale), ptr(in_shift), ptr(Wc), ptr(bc), ptr(z), ptr(stats), st)
-                scale = torch.empty(cout, dtype=torch.float32, device=dev)
-                shift = torch.empty(cout, dtype=torch.float32, device=dev)
-                mr = torch.empty((2, cout), dtype=torch.float64, device=dev)
-                _lib.call("pn2_train_bn_finalize", R, cout, ptr(stats), ptr(gc), ptr(bec), float(eps), float(momentum), ptr(scale), ptr(shift),
-                          ptr(mr), ptr(rmean), ptr(rvar), st)
-                zs.append(z); scales.append(scale); shifts.append(shift); mrs.append(mr)
-                x, in_scale, in_shift = z, scale, shift
+            def first(cin, cout, W, b, z, stats):
+                _lib.call("pn2_train_linear_fwd", R, cin, cout, ptr(x0), None, None, ptr(W), ptr(b), ptr(z), ptr(stats), st)
+
+            zs, scales, shifts, mrs = _forward_layers(R, meta, tensors, dev, st, first)
             a = torch.empty_like(zs[-1])
             _lib.call("pn2_train_bn_relu", R, a.shape[1], ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(a), st)
         ctx.L = L
-        params = []
-        for l in range(L):
-            params += list(tensors[6 * l:6 * l + 4])
-        ctx.save_for_backward(x0, *zs, *scales, *shifts, *mrs, *params)
+        ctx.save_for_backward(x0, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
         return a
 
     @staticmethod
     def backward(ctx, g_a):
-        L = ctx.L
         saved = ctx.saved_tensors
         x0 = saved[0]
-        zs, scales, shifts, mrs = saved[1:1 + L], saved[1 + L:1 + 2 * L], saved[1 + 2 * L:1 + 3 * L], saved[1 + 3 * L:1 + 4 * L]
-        params = saved[1 + 4 * L:]
+        zs, scales, shifts, mrs, params = _saved_layers(saved[1:], ctx.L)
         R = x0.shape[0]
         dev = x0.device
-        g = g_a.contiguous()
-        grads = [None] * (6 * L)
         st = _stream(x0)
+        need_x0 = ctx.needs_input_grad[0]
         with torch.cuda.device(dev):
-            for l in range(L - 1, -1, -1):
-                W, b, gamma, beta = params[4 * l:4 * l + 4]
-                cout, cin = W.shape
-                z, scale, shift, mr = zs[l], scales[l], shifts[l], mrs[l]
-                sums = torch.zeros((2, cout), dtype=torch.float64, device=dev)
-                _lib.call("pn2_train_bn_bwd_reduce", R, cout, ptr(g), ptr(z), ptr(scale), ptr(shift), ptr(sums), st)
-                coef = torch.empty((3, cout), dtype=torch.float32, device=dev)
-                dgamma = torch.empty(cout, dtype=torch.float32, device=dev)
-                dbeta = torch.empty(cout, dtype=torch.float32, device=dev)
-                gc = gamma.detach().contiguous()
-                _lib.call("pn2_train_bn_bwd_coeffs", R, cout, ptr(sums), ptr(mr), ptr(gc), ptr(coef), ptr(dgamma), ptr(dbeta), st)
-                need_in = l > 0 or ctx.needs_input_grad[0]
-                g_in = torch.empty((R, cin), dtype=torch.float32, device=dev) if need_in else None
-                dW = torch.zeros((cout, cin), dtype=torch.float32, device=dev)
-                x_in = x0 if l == 0 else zs[l - 1]
-                in_scale = None if l == 0 else scales[l - 1]
-                in_shift = None if l == 0 else shifts[l - 1]
-                Wt = W.detach().t().contiguous()
-                _lib.call("pn2_train_linear_bwd", R, cin, cout, ptr(x_in), ptr(in_scale), ptr(in_shift), ptr(Wt), ptr(g), ptr(z),
-                          ptr(scale), ptr(shift), ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), ptr(dW), st)
-                grads[6 * l] = dW.view_as(W)
-                grads[6 * l + 1] = torch.zeros_like(b)   # a bias in front of a batch-statistics BatchNorm has zero gradient
-                grads[6 * l + 2] = dgamma
-                grads[6 * l + 3] = dbeta
-                g = g_in
-        return (g, None, *grads)
+            def first(cin, cout, Wt, g, z, scale, shift, coef, dW):
+                g_in = torch.empty((R, cin), dtype=torch.float32, device=dev) if need_x0 else None
+                _lib.call("pn2_train_linear_bwd", R, cin, cout, ptr(x0), None, None, ptr(Wt), ptr(g), ptr(z), ptr(scale), ptr(shift),
+                          ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), ptr(dW), st)
+                return g_in
+
+            g_x0, grads = _backward_layers(R, g_a.contiguous(), zs, scales, shifts, mrs, params, dev, st, first)
+        return (g_x0, None, *grads)
 
 
-def fused_mlp_train(x0, convs, bns):
-    """x0 (R, C0) rows -> (R, C_L) = the conv -> BatchNorm(train) -> ReLU chain; updates the BatchNorm running statistics
-    (momentum, unbiased variance, num_batches_tracked) exactly like torch.nn.BatchNorm in training mode."""
+def _rows_desc(kind, **fields):
+    d = _lib.Pn2Rows()
+    d.kind = kind
+    for k, v in fields.items():
+        setattr(d, k, v)
+    return d
+
+
+def _pooled_grad_view(g):
+    """(tensor, row stride) of a (B, S, C) gradient: itself when its (b, s) rows are C contiguous floats at a fixed
+    stride (e.g. a slice of the gradient of a channel concatenation), else a contiguous copy (a broadcast gradient such
+    as that of a sum has stride 0)."""
+    B, S, C = g.shape
+    if not (g.stride(2) == 1 and g.stride(1) >= C and g.stride(0) == S * g.stride(1)):
+        g = g.contiguous()
+    return g, g.stride(1)
+
+
+class _SaScaleTrain(Function):
+    """One SA scale in training mode: grouping + centring + concat read by the first layer's load, the conv -> BatchNorm
+    (batch statistics) -> ReLU chain, and the max over nsample fused into the last layer.  Channel-last throughout."""
+
+    @staticmethod
+    def forward(ctx, xyz, new_xyz, idx, feat, order, meta, *tensors):
+        """xyz (B, N, 3), new_xyz (B, S, 3), idx (B, S, K) int32, feat (B, N, D) or None, order PN2_ORDER_* ->
+        (B, S, C_L).  The max's winning sample (first maximum) is kept as uint8 per (b, s, c)."""
+        L = len(tensors) // 6
+        B, N, _ = xyz.shape
+        S, K = idx.shape[1], idx.shape[2]
+        D = 0 if feat is None else feat.shape[2]
+        R = B * S * K
+        dev = xyz.device
+        st = _stream(xyz)
+        desc = _rows_desc(_lib.ROWS_GROUPED, order=order, b=B, n=N, m=S, k=K, d=D, xyz=ptr(xyz), new_xyz=ptr(new_xyz),
+                          feat=ptr(feat), idx=ptr(idx))
+        with torch.cuda.device(dev):
+            def first(cin, cout, W, b, z, stats):
+                _lib.call("pn2_train_linear_fwd_rows", R, cin, cout, desc, ptr(W), ptr(b), ptr(z), ptr(stats), st)
+
+            zs, scales, shifts, mrs = _forward_layers(R, meta, tensors, dev, st, first)
+            C = zs[-1].shape[1]
+            out = torch.empty((B, S, C), dtype=torch.float32, device=dev)
+            arg = torch.empty((B, S, C), dtype=torch.uint8, device=dev)
+            _lib.call("pn2_train_bn_relu_max", B * S, K, C, ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(out), C, 0, ptr(arg), st)
+        ctx.L, ctx.order, ctx.has_feat = L, order, feat is not None
+        ctx.save_for_backward(xyz, new_xyz, idx, feat, arg, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
+        return out
+
+    @staticmethod
+    def backward(ctx, g_out):
+        saved = ctx.saved_tensors
+        xyz, new_xyz, idx, feat, arg = saved[:5]
+        zs, scales, shifts, mrs, params = _saved_layers(saved[5:], ctx.L)
+        B, N, _ = xyz.shape
+        S, K = idx.shape[1], idx.shape[2]
+        D = 0 if feat is None else feat.shape[2]
+        R = B * S * K
+        C = zs[-1].shape[1]
+        dev = xyz.device
+        st = _stream(xyz)
+        need_feat = D > 0 and ctx.needs_input_grad[3]
+        desc = _rows_desc(_lib.ROWS_GROUPED, order=ctx.order, b=B, n=N, m=S, k=K, d=D, xyz=ptr(xyz), new_xyz=ptr(new_xyz),
+                          feat=ptr(feat), idx=ptr(idx))
+        with torch.cuda.device(dev):
+            gp, gp_stride = _pooled_grad_view(g_out)
+            g = torch.empty((R, C), dtype=torch.float32, device=dev)
+            _lib.call("pn2_train_max_bwd", B * S, K, C, ptr(gp), gp_stride, 0, ptr(arg), ptr(g), st)
+
+            def first(cin, cout, Wt, g, z, scale, shift, coef, dW):
+                g_in = torch.empty((R, cin), dtype=torch.float32, device=dev) if need_feat else None
+                _lib.call("pn2_train_linear_bwd_rows", R, cin, cout, desc, ptr(Wt), ptr(g), ptr(z), ptr(scale), ptr(shift),
+                          ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), None, ptr(dW), st)
+                return g_in
+
+            g_in, grads = _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first)
+            g_feat = None
+            if need_feat:
+                # grouping backward without atomics: every point sums the feature columns of its rows in row order
+                seg_start = torch.empty(B * N + 1, dtype=torch.int32, device=dev)
+                pos = torch.empty(R, dtype=torch.int32, device=dev)
+                _lib.call("pn2_inverse_index", B, N, S * K, ptr(idx), ptr(seg_start), ptr(pos), st)
+                g_feat = torch.empty((B, N, D), dtype=torch.float32, device=dev)
+                col = 3 if ctx.order == _lib.ORDER_XYZ_FIRST else 0
+                _lib.call("pn2_scatter_rows_det_cl", B, D, N, S * K, 1, ptr(g_in), 3 + D, col, ptr(seg_start), ptr(pos), None,
+                          ptr(g_feat), st)
+        return (None, None, None, g_feat, None, None, *grads)
+
+
+class _FpBlockTrain(Function):
+    """One FP block in training mode: 3-NN interpolation and the skip concat read by the first layer's load, then the
+    conv -> BatchNorm (batch statistics) -> ReLU chain.  Channel-last throughout."""
+
+    @staticmethod
+    def forward(ctx, feat1, feat2, idx, weight, n, meta, *tensors):
+        """feat1 (B, n, D1) or None, feat2 (B, m, D2), idx / weight (B, n, 3) (None when m == 1: the coarse row is repeated)
+        -> (B, n, C_L)."""
+        L = len(tensors) // 6
+        B, m, D2 = feat2.shape
+        D1 = 0 if feat1 is None else feat1.shape[2]
+        R = B * n
+        dev = feat2.device
+        st = _stream(feat2)
+        desc = _rows_desc(_lib.ROWS_INTERP, b=B, n=n, m=m, d=D2, d_skip=D1, feat=ptr(feat2), skip=ptr(feat1), idx=ptr(idx),
+                          weight=ptr(weight))
+        with torch.cuda.device(dev):
+            def first(cin, cout, W, b, z, stats):
+                _lib.call("pn2_train_linear_fwd_rows", R, cin, cout, desc, ptr(W), ptr(b), ptr(z), ptr(stats), st)
+
+            zs, scales, shifts, mrs = _forward_layers(R, meta, tensors, dev, st, first)
+            C = zs[-1].shape[1]
+            a = torch.empty((B, n, C), dtype=torch.float32, device=dev)
+            _lib.call("pn2_train_bn_relu", R, C, ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(a), st)
+        ctx.L, ctx.n = L, n
+        ctx.save_for_backward(feat1, feat2, idx, weight, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
+        return a
+
+    @staticmethod
+    def backward(ctx, g_a):
+        saved = ctx.saved_tensors
+        feat1, feat2, idx, weight = saved[:4]
+        zs, scales, shifts, mrs, params = _saved_layers(saved[4:], ctx.L)
+        B, m, D2 = feat2.shape
+        n = ctx.n
+        D1 = 0 if feat1 is None else feat1.shape[2]
+        R = B * n
+        dev = feat2.device
+        st = _stream(feat2)
+        need1, need2 = D1 > 0 and ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        desc = _rows_desc(_lib.ROWS_INTERP, b=B, n=n, m=m, d=D2, d_skip=D1, feat=ptr(feat2), skip=ptr(feat1), idx=ptr(idx),
+                          weight=ptr(weight))
+        with torch.cuda.device(dev):
+            def first(cin, cout, Wt, g, z, scale, shift, coef, dW):
+                g1 = torch.empty((B, n, D1), dtype=torch.float32, device=dev) if need1 else None  # row i is point i: no scatter
+                g_in = torch.empty((R, D2), dtype=torch.float32, device=dev) if need2 else None
+                _lib.call("pn2_train_linear_bwd_rows", R, cin, cout, desc, ptr(Wt), ptr(g), ptr(z), ptr(scale), ptr(shift),
+                          ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), ptr(g1), ptr(dW), st)
+                return g1, g_in
+
+            (g1, g_in), grads = _backward_layers(R, g_a.contiguous(), zs, scales, shifts, mrs, params, dev, st, first)
+            g2 = None
+            if need2:
+                g2 = torch.empty((B, m, D2), dtype=torch.float32, device=dev)
+                if idx is None:
+                    # m == 1: the one coarse row was repeated n times; every row refers to point 0
+                    idx_rep = torch.zeros((B, n), dtype=torch.int32, device=dev)
+                    seg_start = torch.empty(B + 1, dtype=torch.int32, device=dev)
+                    pos = torch.empty(B * n, dtype=torch.int32, device=dev)
+                    _lib.call("pn2_inverse_index", B, 1, n, ptr(idx_rep), ptr(seg_start), ptr(pos), st)
+                    _lib.call("pn2_scatter_rows_det_cl", B, D2, 1, n, 1, ptr(g_in), D2, 0, ptr(seg_start), ptr(pos), None, ptr(g2), st)
+                else:
+                    # three_interpolate backward without atomics: every coarse point sums w * g over its rows in order
+                    seg_start = torch.empty(B * m + 1, dtype=torch.int32, device=dev)
+                    pos = torch.empty(B * n * 3, dtype=torch.int32, device=dev)
+                    _lib.call("pn2_inverse_index", B, m, 3 * n, ptr(idx), ptr(seg_start), ptr(pos), st)
+                    _lib.call("pn2_scatter_rows_det_cl", B, D2, m, 3 * n, 3, ptr(g_in), D2, 0, ptr(seg_start), ptr(pos), ptr(weight),
+                              ptr(g2), st)
+        return (g1, g2, None, None, None, None, *grads)
+
+
+def _layer_tensors(convs, bns):
+    """(tensors, meta) of a conv / BatchNorm stack for the Functions above; counts the batch for the running statistics
+    (num_batches_tracked) like torch.nn.BatchNorm in training mode."""
     tensors, meta = [], []
     for conv, bn in zip(convs, bns):
         track = bn.track_running_stats and bn.running_mean is not None
@@ -112,7 +306,34 @@ def fused_mlp_train(x0, convs, bns):
         tensors += [conv.weight.reshape(conv.out_channels, conv.in_channels), conv.bias, bn.weight, bn.bias,
                     bn.running_mean if track else None, bn.running_var if track else None]
         meta.append((float(bn.eps), float(momentum)))
+    return tensors, meta
+
+
+def fused_mlp_train(x0, convs, bns):
+    """x0 (R, C0) rows -> (R, C_L) = the conv -> BatchNorm(train) -> ReLU chain; updates the BatchNorm running statistics
+    (momentum, unbiased variance, num_batches_tracked) exactly like torch.nn.BatchNorm in training mode."""
+    tensors, meta = _layer_tensors(convs, bns)
     return _FusedMlpTrain.apply(x0, meta, *tensors)
+
+
+def sa_scale_train(xyz, new_xyz, idx, feat, order, convs, bns):
+    """One SA scale in training mode, channel-last: xyz (B, N, 3), new_xyz (B, S, 3), idx (B, S, K) int32 (K <= 256),
+    feat (B, N, D) or None, order _lib.ORDER_XYZ_FIRST (SSG) / ORDER_FEAT_FIRST (MSG) -> (B, S, C_L) = the max over the K
+    grouped rows of the conv -> BatchNorm(train) -> ReLU chain.  Same values, gradients and running statistics as
+    sample_and_group + fused_mlp_train + max(dim=2); xyz and new_xyz get no gradient."""
+    xyz, new_xyz, idx = _lib.check_f32(xyz, "xyz"), _lib.check_f32(new_xyz, "new_xyz"), _lib.check_i32(idx, "idx")
+    feat = _lib.check_f32(feat, "feat")
+    tensors, meta = _layer_tensors(convs, bns)
+    return _SaScaleTrain.apply(xyz, new_xyz, idx, feat, int(order), meta, *tensors)
+
+
+def fp_block_train(feat1, feat2, idx, weight, convs, bns, n):
+    """One FP block in training mode, channel-last: feat1 (B, n, D1) or None (skip features, first), feat2 (B, m, D2),
+    idx / weight (B, n, 3) of the 3-NN (None when m == 1) -> (B, n, C_L)."""
+    feat1, feat2 = _lib.check_f32(feat1, "feat1"), _lib.check_f32(feat2, "feat2")
+    idx, weight = _lib.check_i32(idx, "idx"), _lib.check_f32(weight, "weight")
+    tensors, meta = _layer_tensors(convs, bns)
+    return _FpBlockTrain.apply(feat1, feat2, idx, weight, int(n), meta, *tensors)
 
 
 def fusable_training(x0, convs, bns):
