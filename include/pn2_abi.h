@@ -169,8 +169,19 @@ int pn2_sa_mlp_max(int b, int n, int m, int k, int d, const float *xyz, const fl
 int pn2_fp_mlp(int b, int n, int m, int d1, int d2, const float *feat1, const float *feat2, const int32_t *idx,
                const float *weight, const pn2_mlp *mlp, float *out, void *stream);
 
-/* 1 if pn2_sa_mlp_max (nsample >= 1) / pn2_fp_mlp (nsample == 0) supports this stack fed with c0 input channels
- * (layer count, nsample a power of two <= 128, widths within shared memory); 0 otherwise.  No CUDA call. */
+/* The group_all SA layer (model/pointnet_util.py:50-67, 101-109): concat + shared MLP + max over ALL n points of each
+ * cloud, channel-last:
+ *   xyz (B,n,3), feat (B,n,D) or NULL (D=0); row bb*n + i = [xyz[bb,i] | feat[bb,i]] (xyz first, not centred);
+ *   out: element (bb, ch) at out[bb*out_stride + out_offset + ch], ch < cout[last]; nothing else of `out` is written.
+ * n is any value >= 1.  The tiles of one cloud are combined with an integer atomicMax on the bits of the non-negative
+ * pooled values, so the last layer must have a ReLU (else PN2_ERR_UNSUPPORTED); the result is bit-identical from run
+ * to run.  The pooled columns are zeroed by a kernel on `stream` first: no host synchronisation, graph capturable.
+ * Supported stacks: those pn2_mlp_fp32_supported(mlp, 3 + D, 0) accepts (the same row tiles and shared memory layout). */
+int pn2_sa_all_mlp_max(int b, int n, int d, const float *xyz, const float *feat, const pn2_mlp *mlp, float *out,
+                       int out_stride, int out_offset, void *stream);
+
+/* 1 if pn2_sa_mlp_max (nsample >= 1) / pn2_fp_mlp and pn2_sa_all_mlp_max (nsample == 0) supports this stack fed with c0
+ * input channels (layer count, nsample a power of two <= 128, widths within shared memory); 0 otherwise.  No CUDA call. */
 int pn2_mlp_fp32_supported(const pn2_mlp *mlp, int c0, int nsample);
 
 /* ---- the shared-MLP layer in TRAINING mode (batch-statistics BatchNorm; model/pointnet_util.py:105-107,162-165,218-220
@@ -208,9 +219,12 @@ int pn2_train_linear_bwd(long long rows, int cin, int cout, const float *x, cons
  *     (PN2_ORDER_FEAT_FIRST), p = idx[bb,s,j]; the centring is one fp32 subtraction.  rows = b*m*k, cin = 3 + d.
  *   PN2_ROWS_INTERP (FP): skip (b,n,d_skip) or NULL (d_skip == 0), feat (b,m,d), idx / weight (b,n,3);
  *     row bb*n + i = [skip[i] | fma(w2,f[i2],fma(w0,f[i0],w1*f[i1]))] (three_interpolate's order); with m == 1 idx and
- *     weight are NULL and the one coarse row is repeated.  rows = b*n, cin = d_skip + d. */
+ *     weight are NULL and the one coarse row is repeated.  rows = b*n, cin = d_skip + d.
+ *   PN2_ROWS_ALL (group_all SA): xyz (b,n,3), feat (b,n,d) or NULL (d == 0); row bb*n + i = [xyz[bb,i] | feat[bb,i]]
+ *     (not centred).  rows = b*n, cin = 3 + d. */
 #define PN2_ROWS_GROUPED 1
 #define PN2_ROWS_INTERP 2
+#define PN2_ROWS_ALL 3
 typedef struct pn2_rows {
     int kind;
     int order; /* PN2_ROWS_GROUPED: PN2_ORDER_XYZ_FIRST or PN2_ORDER_FEAT_FIRST */
@@ -224,7 +238,8 @@ int pn2_train_linear_fwd_rows(long long rows, int cin, int cout, const pn2_rows 
                               float *z, double *stats, void *stream);
 /* pn2_train_linear_bwd of the first layer with x read from `src`.  g_in (rows, cin) (NULL = not needed); for
  * PN2_ROWS_INTERP the first d_skip columns go to g_skip (rows, d_skip) and g_in holds the d interpolated columns
- * (rows, d); either may be NULL. */
+ * (rows, d); either may be NULL.  For PN2_ROWS_ALL a row is a point: g_in is the feature gradient (b, n, d) itself
+ * (NULL when d == 0) and the xyz columns get no gradient. */
 int pn2_train_linear_bwd_rows(long long rows, int cin, int cout, const pn2_rows *src, const float *wt, const float *g,
                               const float *z, const float *scale, const float *shift, const float *ca, const float *cb,
                               const float *cc, float *g_in, float *g_skip, float *dw, void *stream);
@@ -235,6 +250,15 @@ int pn2_train_bn_relu_max(long long groups, int k, int c, const float *z, const 
 /* Backward of the pooling: g (groups*k, c) written in full, g = gp[gr*gp_stride + gp_offset + ch] on row j == arg, 0 elsewhere. */
 int pn2_train_max_bwd(long long groups, int k, int c, const float *gp, int gp_stride, int gp_offset, const uint8_t *arg,
                       float *g, void *stream);
+/* The same pooling over all k >= 1 rows of each group (group_all: a group is a cloud, k its points): out as above, arg
+ * (groups, c) int32 = the first row holding the maximum (torch.max(dim)'s index).  Row ranges of one group are combined
+ * by a 64-bit atomicMax on (value bits, ~row), exact and independent of the order of the CTAs; out and arg are written
+ * in full.  Temporary storage comes from the stream-ordered allocator; no host synchronisation. */
+int pn2_train_bn_relu_max_all(long long groups, long long k, int c, const float *z, const float *scale, const float *shift,
+                              float *out, int out_stride, int out_offset, int32_t *arg, void *stream);
+/* Its backward: g (groups*k, c) written in full, g = gp[gr*gp_stride + gp_offset + ch] on row arg[gr, ch], 0 elsewhere. */
+int pn2_train_max_bwd_all(long long groups, long long k, int c, const float *gp, int gp_stride, int gp_offset,
+                          const int32_t *arg, float *g, void *stream);
 
 /* ---- the same two blocks on the tcgen05 tensor cores: bf16 operands, fp32 accumulation in TMEM ----
  * Outputs agree with the fp32 entry points within bf16 rounding (2e-2 relative).  Weights are packed once

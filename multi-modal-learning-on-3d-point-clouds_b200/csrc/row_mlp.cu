@@ -6,6 +6,8 @@
 // and per feature-propagation block (model/pointnet_util.py:209-220, model/pointnet2.py:158-159):
 //     three_interpolate + concat + permutes + L x (Conv1d 1x1 -> BatchNorm1d(eval) -> ReLU)
 //     (+ the head's conv1/bn1/relu/conv2 appended as two more layers)
+// and per group_all SA layer (model/pointnet_util.py:50-67, 101-109):
+//     concat [xyz | feat] + L x (Conv2d 1x1 -> BatchNorm2d(eval) -> ReLU) + max over all N points of a cloud
 // which the reference runs as ~5 custom launches + ~8 layout copies + 3 x (cuDNN conv, BN, ReLU) +
 // max, writing every intermediate activation to HBM (~100 MB per scene in sa1, SURVEY.md 8a A9).
 //
@@ -24,7 +26,7 @@
 namespace pn2 {
 namespace {
 
-enum { MODE_SA = 0, MODE_FP = 1 };
+enum { MODE_SA = 0, MODE_FP = 1, MODE_ALL = 2 };
 
 struct RowMlpParams {
     int mode;
@@ -40,7 +42,7 @@ struct RowMlpParams {
     const int32_t *idx;
     float *out;
     int out_stride, out_offset;
-    // FP
+    // FP, ALL
     long long rows;  // B*n
     int d1, d2, fp_m;
     const float *feat1, *feat2, *weight;
@@ -162,6 +164,39 @@ __device__ __forceinline__ void gather_fp(const RowMlpParams &p, float *x0, long
     }
 }
 
+// group_all: row bb*n + i = [xyz[bb, i] | feat[bb, i]], read as it lies (no index list, no centring)
+template <int TR>
+__device__ __forceinline__ void gather_all(const RowMlpParams &p, float *x0, long long tile) {
+    constexpr int TRP = TR + 4;
+    const int D = p.d, C0 = 3 + D;
+    const int cpad = round_up(C0, KC);
+    if (C0 <= 16) {
+        // few channels: consecutive threads take consecutive rows (conflict-free stores)
+        for (int e = threadIdx.x; e < cpad * TR; e += RM_THREADS) {
+            const int r = e % TR, c = e / TR;
+            const long long row = tile * TR + r;
+            float v = 0.f;
+            if (row < p.rows && c < C0) v = c < 3 ? __ldg(p.xyz + row * 3 + c) : __ldg(p.feat + row * D + (c - 3));
+            x0[(size_t)c * TRP + r] = v;
+        }
+    } else {
+        // wide rows: one warp per row, lanes along the (contiguous, channel-last) feature row
+        constexpr int NW = RM_THREADS / 32, RPW = TR / NW;
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll 2
+        for (int i = 0; i < RPW; ++i) {
+            const int r = warp + NW * i;
+            const long long row = tile * TR + r;
+            const bool ok = row < p.rows;
+            if (lane < 3) x0[(size_t)lane * TRP + r] = ok ? __ldg(p.xyz + row * 3 + lane) : 0.f;
+            const float *f = p.feat + (ok ? row : 0) * D;
+#pragma unroll 4
+            for (int c = lane; c < D; c += 32) x0[(size_t)(3 + c) * TRP + r] = ok ? __ldg(f + c) : 0.f;
+            for (int c = C0 + lane; c < cpad; c += 32) x0[(size_t)c * TRP + r] = 0.f;
+        }
+    }
+}
+
 template <int TR>
 #ifndef PN2_RM_MINB
 #define PN2_RM_MINB 2
@@ -178,8 +213,10 @@ __global__ void __launch_bounds__(RM_THREADS, PN2_RM_MINB) row_mlp_kernel(const 
 
     if (p.mode == MODE_SA)
         gather_sa<TR>(p, smem, tile);
-    else
+    else if (p.mode == MODE_FP)
         gather_fp<TR>(p, smem, tile);
+    else
+        gather_all<TR>(p, smem, tile);
     __syncthreads();
 
     int cur = 0;  // which buffer holds the current layer's input
@@ -217,6 +254,24 @@ __global__ void __launch_bounds__(RM_THREADS, PN2_RM_MINB) row_mlp_kernel(const 
                     for (int s = 1; s < K; ++s) mx = fmaxf(mx, src[s]);
                     p.out[(size_t)g * p.out_stride + p.out_offset + n0 + col] = mx;
                 }
+            } else if (p.mode == MODE_ALL) {
+                // max over the rows of each cloud in this tile (a tile may end one cloud and start the next, or hold
+                // many clouds when n < TR), combined across tiles by an integer atomicMax on the bits: the last layer
+                // has a ReLU, so every value is a non-negative float whose bit pattern orders like the value (out was
+                // zeroed first; -0 has the sign bit and loses to +0).  Max is exact: the result does not depend on the
+                // order in which the CTAs finish.
+                const long long r0 = tile * TR, r1 = min(r0 + TR, p.rows);
+                const long long cl0 = r0 / p.n;
+                const int ncl = (int)((r1 - 1) / p.n - cl0) + 1;
+                for (int e = threadIdx.x; e < ncl * nv; e += RM_THREADS) {
+                    const int col = e % nv;
+                    const long long cl = cl0 + e / nv;
+                    const int lo = (int)(max(cl * p.n, r0) - r0), hi = (int)(min((cl + 1) * p.n, r1) - r0);
+                    const float *src = xout + (size_t)col * TRP;
+                    float mx = src[lo];
+                    for (int s = lo + 1; s < hi; ++s) mx = fmaxf(mx, src[s]);
+                    atomicMax(reinterpret_cast<int *>(p.out) + (size_t)cl * p.out_stride + p.out_offset + n0 + col, __float_as_int(mx));
+                }
             } else {
                 for (int e = threadIdx.x; e < TR * nv; e += RM_THREADS) {
                     const int col = e % nv, r = e / nv;
@@ -230,6 +285,14 @@ __global__ void __launch_bounds__(RM_THREADS, PN2_RM_MINB) row_mlp_kernel(const 
         // layer_tile ends with a barrier after its last chunk, but its epilogue stores come after
         // that barrier: make them visible before the next layer reads them.
         __syncthreads();
+    }
+}
+
+// out[r*stride + offset + ch] = 0 for r < rows, ch < c: the start value of the group_all pooling's atomicMax
+__global__ void __launch_bounds__(256) zero_cols_kernel(long long rows, int c, float *out, int stride, int offset) {
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < rows * c; e += (long long)gridDim.x * 256) {
+        const long long r = e / c;
+        out[r * stride + offset + (e - r * c)] = 0.f;
     }
 }
 
@@ -325,7 +388,8 @@ void copy_mlp(RowMlpParams &p, const pn2_mlp *mlp) {
 }  // namespace
 }  // namespace pn2
 
-// 1 when pn2_sa_mlp_max (nsample > 0) / pn2_fp_mlp (nsample == 0) can run this stack with `c0` input channels: the
+// 1 when pn2_sa_mlp_max (nsample > 0) / pn2_fp_mlp and pn2_sa_all_mlp_max (nsample == 0: the same row tiles and shared
+// memory layout; pn2_sa_all_mlp_max also needs a ReLU on the last layer) can run this stack with `c0` input channels: the
 // callers (pn2_b200/pointnet_util.py::_fusable) use the reference's operator composition otherwise, so a module that
 // trains on the composed path never fails at eval time for its shape alone.
 extern "C" int pn2_mlp_fp32_supported(const pn2_mlp *mlp, int c0, int nsample) {
@@ -378,4 +442,30 @@ extern "C" int pn2_fp_mlp(int b, int n, int m, int d1, int d2, const float *feat
     p.feat1 = feat1; p.feat2 = feat2; p.idx = idx; p.weight = weight;
     p.out = out;
     return dispatch(p, mlp, d1 + d2, p.rows, 16, (cudaStream_t)stream);
+}
+
+extern "C" int pn2_sa_all_mlp_max(int b, int n, int d, const float *xyz, const float *feat, const pn2_mlp *mlp, float *out,
+                                  int out_stride, int out_offset, void *stream) {
+    using namespace pn2;
+    PN2_REQUIRE(b >= 0 && n >= 1 && d >= 0, "sa_all_mlp_max: bad dims b=%d n=%d d=%d", b, n, d);
+    if (int st = check_mlp("sa_all_mlp_max", mlp, 3 + d)) return st;
+    const int cl = mlp->cout[mlp->num_layers - 1];
+    PN2_REQUIRE(out_offset >= 0 && out_stride >= out_offset + cl, "sa_all_mlp_max: out_stride/out_offset do not hold %d channels", cl);
+    if (!mlp->relu[mlp->num_layers - 1])
+        return set_error(PN2_ERR_UNSUPPORTED, "sa_all_mlp_max: the last layer needs a ReLU (the pooling combines non-negative values)");
+    if (b == 0) return PN2_OK;
+    PN2_REQUIRE(xyz && out && (feat || d == 0), "sa_all_mlp_max: null pointer");
+    cudaStream_t s = (cudaStream_t)stream;
+    const long long total = (long long)b * cl;
+    const unsigned zgrid = (unsigned)((total + 255) / 256 < 8ll * sm_count() ? (total + 255) / 256 : 8ll * sm_count());
+    zero_cols_kernel<<<zgrid, 256, 0, s>>>(b, cl, out, out_stride, out_offset);
+    PN2_LAUNCH_OK("zero_cols_kernel");
+    RowMlpParams p = {};
+    p.mode = MODE_ALL;
+    copy_mlp(p, mlp);
+    p.n = n; p.d = d;
+    p.rows = (long long)b * n;
+    p.xyz = xyz; p.feat = feat;
+    p.out = out; p.out_stride = out_stride; p.out_offset = out_offset;
+    return dispatch(p, mlp, 3 + d, p.rows, 16, s);
 }

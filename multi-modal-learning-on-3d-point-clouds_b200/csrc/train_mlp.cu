@@ -258,6 +258,29 @@ struct InterpIn {  // row bb*n + i: columns [0, ds) = skip[i], [ds, ds + d) = th
     }
 };
 
+struct AllIn {  // row r = bb*n + i of a group_all SA layer: columns [0, 3) = xyz[r], [3, 3 + d) = feat[r] (not centred)
+    const float *xyz, *feat;
+    long long rows;
+    int c, d;
+    // the feature columns start at 3, so no 4-aligned k-chunk lies on 4-aligned feature columns: scalar loads, as for
+    // the materialised (rows, 3 + d) operand of the composition
+    struct Raw {
+        float4 v;
+    };
+    __device__ __forceinline__ Raw raw(long long r, int kc) const {
+        float v[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const int col = kc + e;
+            v[e] = r >= rows || col >= c ? 0.f : (col < 3 ? __ldg(xyz + r * 3 + col) : __ldg(feat + r * d + (col - 3)));
+        }
+        Raw q;
+        q.v = make_float4(v[0], v[1], v[2], v[3]);
+        return q;
+    }
+    __device__ __forceinline__ float4 finish(const Raw &q, long long, int) const { return q.v; }
+};
+
 struct WeightIn {  // w (n_total, k_total) row-major: 4 consecutive k of output column n
     const float *w;
     int n_total, k_total;
@@ -609,17 +632,64 @@ train_bn_relu_max_kernel(long long groups, int k, int c, const float *__restrict
     }
 }
 
-// ---- its backward: the pooled gradient on the winning row, 0 on the others; every element of g is written --------------------
+// ---- the same pooling over ALL k rows of a group (group_all), k unbounded: warp <-> (group, 32 channels, row range) --------
+// Lanes along channels (coalesced z rows); a warp keeps the largest activation and its first row over its range, then the
+// ranges of a group are combined by a 64-bit atomicMax on key = (value bits << 32) | ~row: the values are non-negative
+// (ReLU; -0 is stored as +0), so the bits order like the values, and on equal values the smaller row has the larger ~row.
+// Exact and independent of the order of the CTAs.  keys (groups, c) start at 0, below every real key.
 __global__ void __launch_bounds__(256)
-train_max_bwd_kernel(long long groups, int k, int c, const float *__restrict__ gp, int gp_stride, int gp_offset,
-                     const uint8_t *__restrict__ arg, float *__restrict__ g) {
+train_bn_relu_max_all_kernel(long long groups, long long k, int c, const float *__restrict__ z, const float *__restrict__ scale,
+                             const float *__restrict__ shift, long long rows_per_range, unsigned long long *__restrict__ keys) {
+    const int lane = threadIdx.x & 31;
+    const int nchunks = (c + 31) / 32;
+    const long long nranges = (k + rows_per_range - 1) / rows_per_range;
+    const long long items = groups * nchunks * nranges;
+    for (long long it = ((long long)blockIdx.x * 256 + threadIdx.x) / 32; it < items; it += (long long)gridDim.x * 8) {
+        const long long gr = it / (nchunks * nranges);
+        const long long rest = it - gr * nchunks * nranges;
+        const int ch = (int)(rest / nranges) * 32 + lane;
+        const long long j0 = (rest % nranges) * rows_per_range, j1 = min(k, j0 + rows_per_range);
+        if (ch >= c) continue;
+        const float sc = __ldg(scale + ch), sh = __ldg(shift + ch);
+        const float *zr = z + gr * k * c + ch;
+        float best = -1.f;
+        long long bj = j0;
+#pragma unroll 4
+        for (long long j = j0; j < j1; ++j) {
+            const float a = fmaxf(fmaf(__ldg(zr + j * c), sc, sh), 0.f);
+            if (a > best) {  // strict: the first maximum wins, as torch.max(dim) reports it
+                best = a;
+                bj = j;
+            }
+        }
+        const unsigned long long key = ((unsigned long long)(best > 0.f ? __float_as_uint(best) : 0u) << 32) | (unsigned)~(unsigned)bj;
+        atomicMax(keys + gr * c + ch, key);
+    }
+}
+
+__global__ void __launch_bounds__(256)
+train_max_all_finalize_kernel(long long groups, int c, const unsigned long long *__restrict__ keys, float *__restrict__ out,
+                              int out_stride, int out_offset, int32_t *__restrict__ arg) {
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < groups * c; e += (long long)gridDim.x * 256) {
+        const long long gr = e / c;
+        const unsigned long long key = keys[e];
+        out[gr * out_stride + out_offset + (e - gr * c)] = __uint_as_float((unsigned)(key >> 32));
+        arg[e] = (int32_t)~(unsigned)key;
+    }
+}
+
+// ---- backward of either pooling: the pooled gradient on the winning row, 0 on the others; every element of g is written -------
+template <class Arg>
+__global__ void __launch_bounds__(256)
+train_max_bwd_kernel(long long groups, long long k, int c, const float *__restrict__ gp, int gp_stride, int gp_offset,
+                     const Arg *__restrict__ arg, float *__restrict__ g) {
     const long long total = groups * k * c;
     for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < total; e += (long long)gridDim.x * 256) {
         const long long row = e / c;
         const int ch = (int)(e - row * c);
         const long long gr = row / k;
-        const int j = (int)(row - gr * k);
-        g[e] = __ldg(arg + gr * c + ch) == j ? __ldg(gp + gr * gp_stride + gp_offset + ch) : 0.f;
+        const long long j = row - gr * k;
+        g[e] = (long long)__ldg(arg + gr * c + ch) == j ? __ldg(gp + gr * gp_stride + gp_offset + ch) : 0.f;
     }
 }
 
@@ -743,9 +813,10 @@ int launch_bwd(const DzIn &dz, const LX &a, const float *wt, float *g_in, float 
 bool aligned16(const void *p) { return ((uintptr_t)p & 15) == 0; }
 
 // Validates a pn2_rows against (rows, cin) and builds its loader.  Returns PN2_OK or the error status.
-int rows_loader(const char *who, long long rows, int cin, const pn2_rows *src, GroupIn &gi, InterpIn &ii) {
+int rows_loader(const char *who, long long rows, int cin, const pn2_rows *src, GroupIn &gi, InterpIn &ii, AllIn &ai) {
     PN2_REQUIRE(src, "%s: null row source", who);
-    PN2_REQUIRE(src->kind == PN2_ROWS_GROUPED || src->kind == PN2_ROWS_INTERP, "%s: unknown row source kind %d", who, src->kind);
+    PN2_REQUIRE(src->kind == PN2_ROWS_GROUPED || src->kind == PN2_ROWS_INTERP || src->kind == PN2_ROWS_ALL,
+                "%s: unknown row source kind %d", who, src->kind);
     PN2_REQUIRE(rows < (1ll << 31), "%s: more than 2^31 rows", who);
     const pn2_rows &r = *src;
     if (r.kind == PN2_ROWS_GROUPED) {
@@ -756,6 +827,11 @@ int rows_loader(const char *who, long long rows, int cin, const pn2_rows *src, G
         const bool xyz_first = r.order == PN2_ORDER_XYZ_FIRST;
         gi = {r.xyz, r.new_xyz, r.feat, r.idx, rows, cin, r.n, r.m, r.k, r.d, xyz_first ? 0 : r.d, xyz_first ? 3 : 0,
               r.d > 0 && (r.d & 3) == 0 && aligned16(r.feat)};
+    } else if (r.kind == PN2_ROWS_ALL) {
+        PN2_REQUIRE(r.b >= 1 && r.n >= 1 && r.d >= 0, "%s: bad group_all source b=%d n=%d d=%d", who, r.b, r.n, r.d);
+        PN2_REQUIRE(rows == (long long)r.b * r.n && cin == 3 + r.d, "%s: rows=%lld cin=%d do not match the group_all source", who, rows, cin);
+        PN2_REQUIRE(r.xyz && ((r.feat == nullptr) == (r.d == 0)), "%s: null pointer", who);
+        ai = {r.xyz, r.feat, rows, cin, r.d};
     } else {
         PN2_REQUIRE(r.b >= 1 && r.n >= 1 && r.m >= 1 && r.d >= 1 && r.d_skip >= 0, "%s: bad interpolated source b=%d n=%d m=%d d=%d d_skip=%d",
                     who, r.b, r.n, r.m, r.d, r.d_skip);
@@ -789,11 +865,13 @@ extern "C" int pn2_train_linear_fwd_rows(long long rows, int cin, int cout, cons
     if (rows == 0) return PN2_OK;
     GroupIn gi;
     InterpIn ii;
-    if (int st = rows_loader("train_linear_fwd_rows", rows, cin, src, gi, ii)) return st;
+    AllIn ai;
+    if (int st = rows_loader("train_linear_fwd_rows", rows, cin, src, gi, ii, ai)) return st;
     PN2_REQUIRE(w && bias && z && stats, "train_linear_fwd_rows: null pointer");
     PN2_REQUIRE((((uintptr_t)w | (uintptr_t)z) & 15) == 0, "train_linear_fwd_rows: 16-byte alignment");
     const WeightIn b = {w, cout, cin};
     cudaStream_t s = (cudaStream_t)stream;
+    if (src->kind == PN2_ROWS_ALL) return launch_fwd(ai, b, bias, z, stats, s);
     return src->kind == PN2_ROWS_GROUPED ? launch_fwd(gi, b, bias, z, stats, s) : launch_fwd(ii, b, bias, z, stats, s);
 }
 
@@ -833,16 +911,21 @@ extern "C" int pn2_train_linear_bwd_rows(long long rows, int cin, int cout, cons
     if (rows == 0) return PN2_OK;
     GroupIn gi;
     InterpIn ii;
-    if (int st = rows_loader("train_linear_bwd_rows", rows, cin, src, gi, ii)) return st;
+    AllIn ai;
+    if (int st = rows_loader("train_linear_bwd_rows", rows, cin, src, gi, ii, ai)) return st;
     PN2_REQUIRE(wt && g && z && scale && shift && ca && cb && cc && dw, "train_linear_bwd_rows: null pointer");
     PN2_REQUIRE(g_skip == nullptr || (src->kind == PN2_ROWS_INTERP && src->d_skip > 0),
                 "train_linear_bwd_rows: g_skip needs an interpolated source with skip columns (d_skip > 0)");
+    PN2_REQUIRE(g_in == nullptr || src->kind != PN2_ROWS_ALL || src->d > 0,
+                "train_linear_bwd_rows: a group_all source without features (d == 0) has no input gradient");
     PN2_REQUIRE((((uintptr_t)wt | (uintptr_t)g | (uintptr_t)z | (uintptr_t)g_in) & 15) == 0, "train_linear_bwd_rows: 16-byte alignment");
     PN2_REQUIRE((cout & 3) != 0 || (((uintptr_t)scale | (uintptr_t)shift | (uintptr_t)ca | (uintptr_t)cb | (uintptr_t)cc) & 15) == 0,
                 "train_linear_bwd_rows: 16-byte alignment of the per-channel vectors");
     DzIn dz = {g, z, scale, shift, ca, cb, cc, rows, cout};
     cudaStream_t s = (cudaStream_t)stream;
     if (src->kind == PN2_ROWS_GROUPED) return launch_bwd(dz, gi, wt, g_in, nullptr, 0, dw, s);
+    // group_all: a row is a point, so the feature columns go straight to g_in = (b, n, d); the 3 xyz columns are dropped
+    if (src->kind == PN2_ROWS_ALL) return launch_bwd(dz, ai, wt, g_in, nullptr, 3, dw, s);
     // an FP block's skip columns come first: split them off into g_skip (without skip columns g_in is (rows, cin))
     return launch_bwd(dz, ii, wt, g_in, g_skip, src->d_skip, dw, s);
 }
@@ -905,6 +988,49 @@ extern "C" int pn2_train_max_bwd(long long groups, int k, int c, const float *gp
     PN2_REQUIRE(gp_offset >= 0 && gp_stride >= gp_offset + c, "train_max_bwd: gp_stride=%d gp_offset=%d c=%d", gp_stride, gp_offset, c);
     if (groups == 0) return PN2_OK;
     PN2_REQUIRE(gp && arg && g, "train_max_bwd: null pointer");
+    const long long total = groups * k * c;
+    const unsigned grid = (unsigned)((total + 255) / 256 < 8ll * sm_count() ? (total + 255) / 256 : 8ll * sm_count());
+    train_max_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(groups, k, c, gp, gp_stride, gp_offset, arg, g);
+    PN2_LAUNCH_OK("train_max_bwd_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_train_bn_relu_max_all(long long groups, long long k, int c, const float *z, const float *scale, const float *shift,
+                                         float *out, int out_stride, int out_offset, int32_t *arg, void *stream) {
+    PN2_REQUIRE(groups >= 0 && k >= 1 && k < (1ll << 31) && c >= 1, "train_bn_relu_max_all: bad dims groups=%lld k=%lld c=%d (1 <= k < 2^31)",
+                groups, k, c);
+    PN2_REQUIRE(out_offset >= 0 && out_stride >= out_offset + c, "train_bn_relu_max_all: out_stride=%d out_offset=%d c=%d", out_stride,
+                out_offset, c);
+    if (groups == 0) return PN2_OK;
+    PN2_REQUIRE(z && scale && shift && out && arg, "train_bn_relu_max_all: null pointer");
+    cudaStream_t s = (cudaStream_t)stream;
+    Scratch keys(s);
+    PN2_CUDA(keys.alloc((size_t)groups * c * sizeof(unsigned long long)));
+    PN2_CUDA(cudaMemsetAsync(keys.ptr, 0, (size_t)groups * c * sizeof(unsigned long long), s));
+    // row ranges: about 64 warps per SM in total, at least 128 rows each (one atomic per lane and range)
+    const long long nchunks = (c + 31) / 32;
+    const long long warps = 64ll * sm_count();
+    long long per = (groups * nchunks * k + warps - 1) / warps;
+    if (per < 128) per = 128;
+    const long long items = groups * nchunks * ((k + per - 1) / per);
+    const long long want = (items + 7) / 8;
+    const unsigned grid = (unsigned)(want < 8ll * sm_count() ? want : 8ll * sm_count());
+    train_bn_relu_max_all_kernel<<<grid, 256, 0, s>>>(groups, k, c, z, scale, shift, per, (unsigned long long *)keys.ptr);
+    PN2_LAUNCH_OK("train_bn_relu_max_all_kernel");
+    const long long total = groups * c;
+    const unsigned fgrid = (unsigned)((total + 255) / 256 < 8ll * sm_count() ? (total + 255) / 256 : 8ll * sm_count());
+    train_max_all_finalize_kernel<<<fgrid, 256, 0, s>>>(groups, c, (const unsigned long long *)keys.ptr, out, out_stride, out_offset, arg);
+    PN2_LAUNCH_OK("train_max_all_finalize_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_train_max_bwd_all(long long groups, long long k, int c, const float *gp, int gp_stride, int gp_offset,
+                                     const int32_t *arg, float *g, void *stream) {
+    PN2_REQUIRE(groups >= 0 && k >= 1 && k < (1ll << 31) && c >= 1, "train_max_bwd_all: bad dims groups=%lld k=%lld c=%d (1 <= k < 2^31)",
+                groups, k, c);
+    PN2_REQUIRE(gp_offset >= 0 && gp_stride >= gp_offset + c, "train_max_bwd_all: gp_stride=%d gp_offset=%d c=%d", gp_stride, gp_offset, c);
+    if (groups == 0) return PN2_OK;
+    PN2_REQUIRE(gp && arg && g, "train_max_bwd_all: null pointer");
     const long long total = groups * k * c;
     const unsigned grid = (unsigned)((total + 255) / 256 < 8ll * sm_count() ? (total + 255) / 256 : 8ll * sm_count());
     train_max_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(groups, k, c, gp, gp_stride, gp_offset, arg, g);

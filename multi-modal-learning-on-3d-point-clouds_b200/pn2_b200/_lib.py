@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(CSRC, "libpn2_b200.so")
 PN2_MAX_LAYERS = 6
 REDUCE_MAX, REDUCE_FIRST = 0, 1
 ORDER_XYZ_FIRST, ORDER_FEAT_FIRST = 0, 1
-ROWS_GROUPED, ROWS_INTERP = 1, 2
+ROWS_GROUPED, ROWS_INTERP, ROWS_ALL = 1, 2, 3
 FLAG_IN_BF16, FLAG_SKIP_BF16, FLAG_OUT_BF16, FLAG_OUT_ARGMAX = 1, 2, 4, 8
 
 _c_int, _c_float, _vp = ctypes.c_int, ctypes.c_float, ctypes.c_void_p
@@ -66,6 +66,7 @@ _SIGNATURES = {
     "pn2_frustum_count": [_c_int, _c_int, _vp, _vp, _vp, _vp, _vp, _vp],
     "pn2_sa_mlp_max": [_c_int] * 5 + [_vp] * 4 + [_c_int, ctypes.POINTER(Pn2Mlp), _vp, _c_int, _c_int, _vp],
     "pn2_fp_mlp": [_c_int] * 5 + [_vp] * 4 + [ctypes.POINTER(Pn2Mlp), _vp, _vp],
+    "pn2_sa_all_mlp_max": [_c_int] * 3 + [_vp] * 2 + [ctypes.POINTER(Pn2Mlp), _vp, _c_int, _c_int, _vp],
     "pn2_mlp_pack_bf16": [ctypes.POINTER(Pn2Mlp), _c_int, _vp, _vp],
     "pn2_sa_mlp_max_bf16": [_c_int] * 5 + [_vp] * 4 + [ctypes.POINTER(Pn2Mlp), _vp, _vp, _c_int, _c_int, _c_int, _vp],
     "pn2_fp_mlp_bf16": [_c_int] * 5 + [_vp] * 4 + [ctypes.POINTER(Pn2Mlp), _vp, _vp, _vp, _c_int, _vp],
@@ -84,6 +85,8 @@ _SIGNATURES = {
     "pn2_train_linear_bwd_rows": [ctypes.c_longlong, _c_int, _c_int, _ROWS] + [_vp] * 12,
     "pn2_train_bn_relu_max": [ctypes.c_longlong, _c_int, _c_int] + [_vp] * 4 + [_c_int, _c_int, _vp, _vp],
     "pn2_train_max_bwd": [ctypes.c_longlong, _c_int, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
+    "pn2_train_bn_relu_max_all": [ctypes.c_longlong, ctypes.c_longlong, _c_int] + [_vp] * 4 + [_c_int, _c_int, _vp, _vp],
+    "pn2_train_max_bwd_all": [ctypes.c_longlong, ctypes.c_longlong, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
 }
 _OTHER = {
     "pn2_last_error": ([], ctypes.c_char_p),

@@ -18,6 +18,8 @@ Two execution paths per module:
     input gradients without atomics; with deterministic algorithms, set_fused_training(False) or coordinates that need a
     gradient, the reference's own composition of operators -- our kernels for the geometry, torch.nn for conv/BN.  Both
     with identical semantics.
+The group_all SA layer (one group of all N points per cloud, xyz not centred) takes the same two paths: in eval one
+fp32 kernel that pools whole clouds (under both set_mlp_precision settings), in training one autograd Function.
 """
 import ctypes
 import os
@@ -418,6 +420,21 @@ def sa_mlp_max_cl(xyz_cl, feat_cl, new_xyz_cl, idx, order, mlp, out=None, out_of
     return out
 
 
+def sa_all_mlp_max_cl(xyz_cl, feat_cl, mlp, out=None, out_offset=0):
+    """Fused group_all SA layer: rows [xyz | feat] of every point, MLP, max over all N points of each cloud.
+    xyz (B, N, 3), feat (B, N, D) or None -> (B, 1, cout) (or writes a channel slice of `out`).  Always the fp32 kernel:
+    the last layer must have a ReLU (every folded SA stack has one)."""
+    xyz_cl, feat_cl = _lib.check_f32(xyz_cl, "xyz"), _lib.check_f32(feat_cl, "features")
+    B, N, _ = xyz_cl.shape
+    D = 0 if feat_cl is None else feat_cl.shape[2]
+    if out is None:
+        out = torch.empty((B, 1, mlp.cout), dtype=torch.float32, device=xyz_cl.device)
+    with torch.cuda.device(xyz_cl.device):
+        _lib.call("pn2_sa_all_mlp_max", B, N, D, ptr(xyz_cl), ptr(feat_cl), mlp.desc, ptr(out), out.shape[-1], out_offset,
+                  _lib.stream_ptr(xyz_cl.device))
+    return out
+
+
 def three_nn_weights_cl(xyz1_cl, xyz2_cl):
     """-> idx (B, n, 3) int32, weight (B, n, 3): three_nn + sqrt + clamp + inverse-distance weights
     (model/pointnet_util.py:205-208) in one kernel."""
@@ -520,14 +537,19 @@ class PointNetSetAbstraction(nn.Module):
 
     def _fused_ok(self, xyz, points):
         """Eval / no-autograd / fp32 (see _fusable) and a shape the fused kernel supports: up to PN2_MAX_LAYERS layers,
-        nsample a power of two <= 128, widths within shared memory -- otherwise the reference's composition runs."""
-        if self.group_all or len(self.mlp_convs) > _lib.PN2_MAX_LAYERS or not _fusable(self, xyz, points):
+        nsample a power of two <= 128 (any N with group_all), widths within shared memory -- otherwise the reference's
+        composition runs."""
+        if len(self.mlp_convs) > _lib.PN2_MAX_LAYERS or not _fusable(self, xyz, points):
             return False
-        return _fp32_supported(self.folded(), 3 + (0 if points is None else points.shape[1]), self.nsample)
+        return _fp32_supported(self.folded(), 3 + (0 if points is None else points.shape[1]), 0 if self.group_all else self.nsample)
 
     def forward_cl(self, xyz_cl, feat_cl, geometry=None, out_dtype=torch.float32):
         """Channel-last fused path: xyz (B, N, 3), feat (B, N, D) or None -> new_xyz (B, S, 3), (B, S, D').
-        `geometry` = (new_xyz, ball_idx) lets several modules share one sampling / ball query."""
+        `geometry` = (new_xyz, ball_idx) lets several modules share one sampling / ball query.  With group_all: new_xyz
+        is zeros (B, 1, 3) and the fp32 kernel pools whole clouds (geometry and out_dtype do not apply)."""
+        if self.group_all:
+            new_xyz = torch.zeros((xyz_cl.shape[0], 1, 3), dtype=torch.float32, device=xyz_cl.device)
+            return new_xyz, sa_all_mlp_max_cl(xyz_cl, feat_cl, self.folded())
         if geometry is None:
             _, new_xyz = fps_gather_cl(xyz_cl, self.npoint)
             idx = pointnet2_utils.ball_query(self.radius, self.nsample, xyz_cl, new_xyz)
@@ -542,6 +564,10 @@ class PointNetSetAbstraction(nn.Module):
         if self._fused_ok(xyz, points):
             new_xyz, out = self.forward_cl(to_channel_last(xyz), to_channel_last(points))
             return new_xyz.permute(0, 2, 1), to_channel_first(out)
+        if self.group_all and _train_blocks(self, self.mlp_convs, self.mlp_bns, [xyz], [points]):
+            out = train_mlp.sa_all_train(_cl_xyz(xyz), _cl_view(points) if points is not None else None, self.mlp_convs,
+                                         self.mlp_bns)
+            return torch.zeros((xyz.shape[0], 3, 1), dtype=torch.float32, device=xyz.device), out.permute(0, 2, 1)
         if not self.group_all and _train_blocks(self, self.mlp_convs, self.mlp_bns, [xyz], [points], self.nsample):
             xyz_cl = _cl_xyz(xyz)
             new_xyz = _sampled(xyz_cl, xyz, self.npoint, fps_idx)

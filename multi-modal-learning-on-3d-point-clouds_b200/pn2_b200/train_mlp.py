@@ -294,6 +294,64 @@ class _FpBlockTrain(Function):
         return (g1, g2, None, None, None, None, *grads)
 
 
+class _SaAllTrain(Function):
+    """The group_all SA layer in training mode: the [xyz | feat] rows read by the first layer's load, the conv ->
+    BatchNorm (batch statistics) -> ReLU chain, and the max over all N points of each cloud fused into the last layer."""
+
+    @staticmethod
+    def forward(ctx, xyz, feat, meta, *tensors):
+        """xyz (B, N, 3), feat (B, N, D) or None -> (B, 1, C_L).  The max's winning point (first maximum) is kept as int32
+        per (b, c)."""
+        L = len(tensors) // 6
+        B, N, _ = xyz.shape
+        D = 0 if feat is None else feat.shape[2]
+        R = B * N
+        dev = xyz.device
+        st = _stream(xyz)
+        desc = _rows_desc(_lib.ROWS_ALL, b=B, n=N, d=D, xyz=ptr(xyz), feat=ptr(feat))
+        with torch.cuda.device(dev):
+            def first(cin, cout, W, b, z, stats):
+                _lib.call("pn2_train_linear_fwd_rows", R, cin, cout, desc, ptr(W), ptr(b), ptr(z), ptr(stats), st)
+
+            zs, scales, shifts, mrs = _forward_layers(R, meta, tensors, dev, st, first)
+            C = zs[-1].shape[1]
+            out = torch.empty((B, 1, C), dtype=torch.float32, device=dev)
+            arg = torch.empty((B, C), dtype=torch.int32, device=dev)
+            _lib.call("pn2_train_bn_relu_max_all", B, N, C, ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(out), C, 0, ptr(arg), st)
+        ctx.L = L
+        ctx.save_for_backward(xyz, feat, arg, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
+        return out
+
+    @staticmethod
+    def backward(ctx, g_out):
+        saved = ctx.saved_tensors
+        xyz, feat, arg = saved[:3]
+        zs, scales, shifts, mrs, params = _saved_layers(saved[3:], ctx.L)
+        B, N, _ = xyz.shape
+        D = 0 if feat is None else feat.shape[2]
+        R = B * N
+        C = zs[-1].shape[1]
+        dev = xyz.device
+        st = _stream(xyz)
+        need_feat = D > 0 and ctx.needs_input_grad[1]
+        desc = _rows_desc(_lib.ROWS_ALL, b=B, n=N, d=D, xyz=ptr(xyz), feat=ptr(feat))
+        with torch.cuda.device(dev):
+            gp = g_out[:, 0]  # (B, C): read in place when its rows are C contiguous floats (not for a broadcast gradient)
+            if not (gp.stride(1) == 1 and gp.stride(0) >= C):
+                gp = gp.contiguous()
+            g = torch.empty((R, C), dtype=torch.float32, device=dev)
+            _lib.call("pn2_train_max_bwd_all", B, N, C, ptr(gp), gp.stride(0), 0, ptr(arg), ptr(g), st)
+
+            def first(cin, cout, Wt, g, z, scale, shift, coef, dW):
+                g_feat = torch.empty((B, N, D), dtype=torch.float32, device=dev) if need_feat else None  # row = point: no scatter
+                _lib.call("pn2_train_linear_bwd_rows", R, cin, cout, desc, ptr(Wt), ptr(g), ptr(z), ptr(scale), ptr(shift),
+                          ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_feat), None, ptr(dW), st)
+                return g_feat
+
+            g_feat, grads = _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first)
+        return (None, g_feat, None, *grads)
+
+
 def _layer_tensors(convs, bns):
     """(tensors, meta) of a conv / BatchNorm stack for the Functions above; counts the batch for the running statistics
     (num_batches_tracked) like torch.nn.BatchNorm in training mode."""
@@ -325,6 +383,15 @@ def sa_scale_train(xyz, new_xyz, idx, feat, order, convs, bns):
     feat = _lib.check_f32(feat, "feat")
     tensors, meta = _layer_tensors(convs, bns)
     return _SaScaleTrain.apply(xyz, new_xyz, idx, feat, int(order), meta, *tensors)
+
+
+def sa_all_train(xyz, feat, convs, bns):
+    """The group_all SA layer in training mode, channel-last: xyz (B, N, 3), feat (B, N, D) or None -> (B, 1, C_L) = the
+    max over all N rows [xyz | feat] of each cloud of the conv -> BatchNorm(train) -> ReLU chain.  Same values, gradients
+    and running statistics as sample_and_group_all + fused_mlp_train + max(dim=2); xyz gets no gradient."""
+    xyz, feat = _lib.check_f32(xyz, "xyz"), _lib.check_f32(feat, "feat")
+    tensors, meta = _layer_tensors(convs, bns)
+    return _SaAllTrain.apply(xyz, feat, meta, *tensors)
 
 
 def fp_block_train(feat1, feat2, idx, weight, convs, bns, n):
