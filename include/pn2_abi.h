@@ -184,10 +184,11 @@ int pn2_sa_all_mlp_max(int b, int n, int d, const float *xyz, const float *feat,
  * input channels (layer count, nsample a power of two <= 128, widths within shared memory); 0 otherwise.  No CUDA call. */
 int pn2_mlp_fp32_supported(const pn2_mlp *mlp, int c0, int nsample);
 
-/* ---- the shared-MLP layer in TRAINING mode (batch-statistics BatchNorm; model/pointnet_util.py:105-107,162-165,218-220
- * under autograd), fp32, channel-last row matrices (rows x channels).  See csrc/train_mlp.cu for the algebra. ----
+/* ---- the shared-MLP layer in TRAINING mode (BatchNorm with batch or running statistics; model/pointnet_util.py:105-107,
+ * 162-165,218-220 under autograd), fp32, channel-last row matrices (rows x channels).  See csrc/train_mlp.cu for the algebra. ----
  * forward: z (rows,cout) = act_in(x) W^T + bias, act_in(v) = relu(in_scale v + in_shift) per input channel (the previous
- *   layer's BatchNorm + ReLU; NULL/NULL = identity), w (cout,cin); stats (2,cout) float64, PRE-ZEROED: += sum_r z, sum_r z^2. */
+ *   layer's BatchNorm + ReLU; NULL/NULL = identity), w (cout,cin); stats (2,cout) float64, PRE-ZEROED: += sum_r z, sum_r z^2.
+ *   stats NULL: no statistics are reduced (a layer whose BatchNorm uses its running statistics), z only. */
 int pn2_train_linear_fwd(long long rows, int cin, int cout, const float *x, const float *in_scale, const float *in_shift,
                          const float *w, const float *bias, float *z, double *stats, void *stream);
 /* Per-channel BatchNorm quantities from the forward sums (one tiny launch): scale = gamma rstd, shift = beta - mean scale
@@ -199,6 +200,16 @@ int pn2_train_bn_finalize(long long rows, int c, const double *stats, const floa
 /* Coefficients of dz = ca dy + cb + cc z from the backward sums: coef (3,c) = ca | cb | cc; dgamma (c), dbeta (c). */
 int pn2_train_bn_bwd_coeffs(long long rows, int c, const double *sums, const double *mean_rstd, const float *gamma, float *coef,
                             float *dgamma, float *dbeta, void *stream);
+/* A BatchNorm that normalises with its RUNNING statistics (eval mode; torch uses batch statistics iff bn.training or no
+ * running statistics): scale = gamma rstd, shift = beta - running_mean scale with rstd = 1 / sqrt(running_var + eps) (fp32,
+ * the same roles as pn2_train_bn_finalize's), mean_rstd (2,c) float64 = (running_mean, rstd) for the backward.  Writes
+ * nothing else: the running statistics are read only. */
+int pn2_train_bn_running(int c, const float *running_mean, const float *running_var, const float *gamma, const float *beta,
+                         double eps, float *scale, float *shift, double *mean_rstd, void *stream);
+/* Its backward from the sums of pn2_train_bn_bwd_reduce (S1 = sum dy, S2 = sum dy z): coef (3,c) = scale | 0 | 0 (dz = scale dy),
+ * dgamma = rstd (S2 - running_mean S1), dbeta = S1, dbias = scale S1 (the conv bias gradient, sum_r dz). */
+int pn2_train_bn_running_bwd_coeffs(int c, const double *sums, const double *mean_rstd, const float *scale, float *coef,
+                                    float *dgamma, float *dbeta, float *dbias, void *stream);
 /* a (rows,c) = relu(scale z + shift): the materialised output of the last layer of a stack. */
 int pn2_train_bn_relu(long long rows, int c, const float *z, const float *scale, const float *shift, float *a, void *stream);
 /* BatchNorm backward reductions: dy = g [scale z + shift > 0]; sums (2,c) float64, PRE-ZEROED: += sum_r dy, sum_r dy z. */

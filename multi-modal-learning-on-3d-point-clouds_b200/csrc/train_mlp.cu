@@ -1,4 +1,5 @@
-// train_mlp.cu -- the shared-MLP layer of the SA / FP blocks in TRAINING mode (batch-statistics BatchNorm), fp32.
+// train_mlp.cu -- the shared-MLP layer of the SA / FP blocks in TRAINING mode (BatchNorm with batch statistics, or with
+// its running statistics when torch's rule says so: see train_bn_running_kernel), fp32.
 //
 // Replaces, per layer of model/pointnet_util.py:105-107 / 162-165 / 218-220 run under autograd,
 //     Conv2d/Conv1d 1x1 (cuDNN fprop, dgrad, wgrad) + BatchNorm (forward statistics, normalise, backward reductions,
@@ -353,7 +354,9 @@ __device__ __forceinline__ void gemm_rows(const LA &la, const WeightIn &lb, long
 }
 
 // ---- forward: z = act_in(x) W^T + b, per-channel sum / sum of squares of z ---------------------------------------------------
-template <int NT, class LX>
+// STATS = false (stats == NULL: every layer whose BatchNorm normalises with its running statistics) stores z only: no
+// column-sum shuffles, no shared-memory partials, no float64 atomics
+template <int NT, class LX, bool STATS>
 __global__ void __launch_bounds__(TG_THREADS, 2)
 train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, float *__restrict__ z, double *__restrict__ stats,
                         long long tiles) {
@@ -382,7 +385,7 @@ train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, floa
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 v[j] = acc[i][j] + bv[j];
-                if (col + j < cout) {
+                if (STATS && col + j < cout) {
                     s1[j] += v[j];
                     s2[j] = fmaf(v[j], v[j], s2[j]);
                 }
@@ -395,6 +398,7 @@ train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, floa
                     if (col + j < cout) z[r * cout + col + j] = v[j];
             }
         }
+        if constexpr (!STATS) continue;
         // column sums: lanes of a warp that share tx (32 / TX rows of threads) by shuffles, the 8 warps through shared
         // memory (shared-memory float atomics compile to compare-and-swap loops: 8-way contended, they were 7 % of the
         // kernel's instructions and a quarter of its stall samples)
@@ -736,6 +740,40 @@ __global__ void train_bn_bwd_coeffs_kernel(int c, double rows, const double *__r
     dbeta[k] = (float)S1;
 }
 
+// ---- the same two coefficient kernels for a BatchNorm that normalises with its RUNNING statistics (eval mode: torch's
+// rule is batch statistics iff bn.training or running_mean is None).  zhat = (z - rm) rstd with constant rm, rstd, so
+// dL/dz = gamma rstd dy: ca = scale, cb = cc = 0.  Nothing but the outputs is written (the running statistics stay as they are).
+__global__ void train_bn_running_kernel(int c, const float *__restrict__ running_mean, const float *__restrict__ running_var,
+                                        const float *__restrict__ gamma, const float *__restrict__ beta, double eps,
+                                        float *__restrict__ scale, float *__restrict__ shift, double *__restrict__ mean_rstd) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= c) return;
+    const double rm = (double)running_mean[k];
+    const double rstd = rsqrt((double)running_var[k] + eps);
+    const double g = (double)gamma[k];
+    scale[k] = (float)(g * rstd);
+    shift[k] = (float)((double)beta[k] - rm * g * rstd);
+    mean_rstd[k] = rm;
+    mean_rstd[c + k] = rstd;
+}
+
+// (S1 = sum dy, S2 = sum dy z) -> coef = (scale, 0, 0); dgamma = rstd (S2 - rm S1), dbeta = S1, and the conv bias gradient
+// dbias = sum dz = scale S1 (not zero here: nothing subtracts the batch mean)
+__global__ void train_bn_running_bwd_coeffs_kernel(int c, const double *__restrict__ sums, const double *__restrict__ mean_rstd,
+                                                   const float *__restrict__ scale, float *__restrict__ coef,
+                                                   float *__restrict__ dgamma, float *__restrict__ dbeta, float *__restrict__ dbias) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= c) return;
+    const double S1 = sums[k], S2 = sums[c + k], rm = mean_rstd[k], rstd = mean_rstd[c + k];
+    const float sc = scale[k];
+    coef[k] = sc;
+    coef[c + k] = 0.f;
+    coef[2 * c + k] = 0.f;
+    dgamma[k] = (float)(rstd * (S2 - rm * S1));
+    dbeta[k] = (float)S1;
+    dbias[k] = (float)((double)sc * S1);
+}
+
 int pick_nt(int n) { return n <= 32 ? 32 : (n <= 64 ? 64 : 128); }
 
 template <int NT>
@@ -750,13 +788,13 @@ int launch_fwd(const LX &a, const WeightIn &b, const float *bias, float *z, doub
     const int nt = pick_nt(cout);
     const long long work = tiles * ((cout + nt - 1) / nt);
     const unsigned grid = (unsigned)(work < 2ll * sm_count() ? work : 2ll * sm_count());
-    if (nt == 32) {
-        train_linear_fwd_kernel<32><<<grid, TG_THREADS, tile_smem<32>(), s>>>(a, b, bias, z, stats, tiles);
-    } else if (nt == 64) {
-        train_linear_fwd_kernel<64><<<grid, TG_THREADS, tile_smem<64>(), s>>>(a, b, bias, z, stats, tiles);
+#define PN2_FW(NTV, ST) train_linear_fwd_kernel<NTV, LX, ST><<<grid, TG_THREADS, tile_smem<NTV>(), s>>>(a, b, bias, z, stats, tiles)
+    if (stats) {
+        if (nt == 32) PN2_FW(32, true); else if (nt == 64) PN2_FW(64, true); else PN2_FW(128, true);
     } else {
-        train_linear_fwd_kernel<128><<<grid, TG_THREADS, tile_smem<128>(), s>>>(a, b, bias, z, stats, tiles);
+        if (nt == 32) PN2_FW(32, false); else if (nt == 64) PN2_FW(64, false); else PN2_FW(128, false);
     }
+#undef PN2_FW
     PN2_LAUNCH_OK("train_linear_fwd_kernel");
     return PN2_OK;
 }
@@ -853,7 +891,7 @@ extern "C" int pn2_train_linear_fwd(long long rows, int cin, int cout, const flo
                                     const float *w, const float *bias, float *z, double *stats, void *stream) {
     PN2_REQUIRE(rows >= 0 && cin >= 1 && cout >= 1, "train_linear_fwd: bad dims rows=%lld cin=%d cout=%d", rows, cin, cout);
     if (rows == 0) return PN2_OK;
-    PN2_REQUIRE(x && w && bias && z && stats && ((in_scale == nullptr) == (in_shift == nullptr)), "train_linear_fwd: null pointer");
+    PN2_REQUIRE(x && w && bias && z && ((in_scale == nullptr) == (in_shift == nullptr)), "train_linear_fwd: null pointer");
     PN2_REQUIRE((((uintptr_t)x | (uintptr_t)w | (uintptr_t)z | (uintptr_t)in_scale | (uintptr_t)in_shift) & 15) == 0, "train_linear_fwd: 16-byte alignment");
     ActIn a = {x, in_scale, in_shift, rows, cin};
     return launch_fwd(a, WeightIn{w, cout, cin}, bias, z, stats, (cudaStream_t)stream);
@@ -867,7 +905,7 @@ extern "C" int pn2_train_linear_fwd_rows(long long rows, int cin, int cout, cons
     InterpIn ii;
     AllIn ai;
     if (int st = rows_loader("train_linear_fwd_rows", rows, cin, src, gi, ii, ai)) return st;
-    PN2_REQUIRE(w && bias && z && stats, "train_linear_fwd_rows: null pointer");
+    PN2_REQUIRE(w && bias && z, "train_linear_fwd_rows: null pointer");
     PN2_REQUIRE((((uintptr_t)w | (uintptr_t)z) & 15) == 0, "train_linear_fwd_rows: 16-byte alignment");
     const WeightIn b = {w, cout, cin};
     cudaStream_t s = (cudaStream_t)stream;
@@ -966,6 +1004,26 @@ extern "C" int pn2_train_bn_bwd_coeffs(long long rows, int c, const double *sums
     PN2_REQUIRE(sums && mean_rstd && gamma && coef && dgamma && dbeta, "train_bn_bwd_coeffs: null pointer");
     train_bn_bwd_coeffs_kernel<<<(c + 127) / 128, 128, 0, (cudaStream_t)stream>>>(c, (double)rows, sums, mean_rstd, gamma, coef, dgamma, dbeta);
     PN2_LAUNCH_OK("train_bn_bwd_coeffs_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_train_bn_running(int c, const float *running_mean, const float *running_var, const float *gamma, const float *beta,
+                                    double eps, float *scale, float *shift, double *mean_rstd, void *stream) {
+    PN2_REQUIRE(c >= 1 && eps >= 0.0, "train_bn_running: bad dims c=%d eps=%g", c, eps);
+    PN2_REQUIRE(running_mean && running_var && gamma && beta && scale && shift && mean_rstd, "train_bn_running: null pointer");
+    train_bn_running_kernel<<<(c + 127) / 128, 128, 0, (cudaStream_t)stream>>>(c, running_mean, running_var, gamma, beta, eps, scale,
+                                                                               shift, mean_rstd);
+    PN2_LAUNCH_OK("train_bn_running_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_train_bn_running_bwd_coeffs(int c, const double *sums, const double *mean_rstd, const float *scale, float *coef,
+                                               float *dgamma, float *dbeta, float *dbias, void *stream) {
+    PN2_REQUIRE(c >= 1, "train_bn_running_bwd_coeffs: bad dims c=%d", c);
+    PN2_REQUIRE(sums && mean_rstd && scale && coef && dgamma && dbeta && dbias, "train_bn_running_bwd_coeffs: null pointer");
+    train_bn_running_bwd_coeffs_kernel<<<(c + 127) / 128, 128, 0, (cudaStream_t)stream>>>(c, sums, mean_rstd, scale, coef, dgamma,
+                                                                                          dbeta, dbias);
+    PN2_LAUNCH_OK("train_bn_running_bwd_coeffs_kernel");
     return PN2_OK;
 }
 

@@ -78,6 +78,8 @@ _SIGNATURES = {
     "pn2_train_linear_fwd": [ctypes.c_longlong, _c_int, _c_int] + [_vp] * 8,
     "pn2_train_bn_finalize": [ctypes.c_longlong, _c_int, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double] + [_vp] * 6,
     "pn2_train_bn_bwd_coeffs": [ctypes.c_longlong, _c_int] + [_vp] * 7,
+    "pn2_train_bn_running": [_c_int] + [_vp] * 4 + [ctypes.c_double] + [_vp] * 4,
+    "pn2_train_bn_running_bwd_coeffs": [_c_int] + [_vp] * 8,
     "pn2_train_bn_relu": [ctypes.c_longlong, _c_int] + [_vp] * 5,
     "pn2_train_bn_bwd_reduce": [ctypes.c_longlong, _c_int] + [_vp] * 6,
     "pn2_train_linear_bwd": [ctypes.c_longlong, _c_int, _c_int] + [_vp] * 14,

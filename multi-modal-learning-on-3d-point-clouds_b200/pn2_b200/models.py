@@ -8,7 +8,8 @@ PointNet2Multiview2Msg  model/pointnet2multiview.py:179-233     (the MSG semseg 
 Attribute names match the reference so its state_dicts load unchanged.  In eval mode under
 torch.no_grad() the forward is 17 kernel launches (2 layout transposes, 4 x (FPS+gather, ball
 query, fused SA), 4 x (three_nn+weights, fused FP; the head is folded into the last FP block) -- the reference issues ~170
-(SURVEY.md 3.2).  Otherwise the reference's own composition runs (training / autograd).
+(SURVEY.md 3.2).  Otherwise (training, or eval under autograd) the modules' training paths run: block Functions on
+the fused training kernels, each BatchNorm in its own mode (batch or running statistics) as in torch.
 """
 import threading
 
@@ -23,8 +24,9 @@ from .pointnet_util import (PointNetFeaturePropagation, PointNetSetAbstraction, 
 
 
 def _semseg_head(model, l0_points):
-    """conv1 -> bn1 -> ReLU -> dropout -> conv2 -> (B, N, classes) (model/pointnet2.py:158-161).  In training mode on the
-    fused training kernels: conv1 + BatchNorm + ReLU as one row chain, conv2 as a row GEMM (no 1x1 cuDNN convolutions)."""
+    """conv1 -> bn1 -> ReLU -> dropout -> conv2 -> (B, N, classes) (model/pointnet2.py:158-161).  In training mode, and in
+    eval mode under autograd, on the fused training kernels: conv1 + BatchNorm (batch or running statistics, as bn1's mode
+    says) + ReLU as one row chain, conv2 as a row GEMM (no 1x1 cuDNN convolutions)."""
     from . import pointnet_util, train_mlp
     if pointnet_util._train_fused(model, l0_points, [model.conv1], [model.bn1]):
         B, C, N = l0_points.shape

@@ -13,11 +13,14 @@ Two execution paths per module:
     grouping, centring, concat, every 1x1 conv with its eval BatchNorm folded in, ReLU and the max
     over nsample never leave shared memory (csrc/row_mlp.cu).  Activations are channel-last inside;
     `forward_cl` exposes that layout so a whole network can stay in it (pn2_b200/models.py).
-  * training (batch statistics / autograd): one autograd Function per SA scale / FP block (pn2_b200/train_mlp.py):
+  * training, and eval() under autograd: one autograd Function per SA scale / FP block (pn2_b200/train_mlp.py):
     the first layer reads the grouped / interpolated rows where they lie, the last one pools, the backward scatters the
-    input gradients without atomics; with deterministic algorithms, set_fused_training(False) or coordinates that need a
-    gradient, the reference's own composition of operators -- our kernels for the geometry, torch.nn for conv/BN.  Both
-    with identical semantics.
+    input gradients without atomics.  Every BatchNorm follows its own mode as in torch -- batch statistics iff
+    bn.training or it has no running statistics, else its running statistics, left untouched -- so frozen-BatchNorm
+    fine-tuning (`net.train()`, then `m.eval()` on every BatchNorm) and eval-mode gradients run here too.  With
+    deterministic algorithms, set_fused_training(False) or coordinates that need a gradient, the reference's own
+    composition of operators -- our kernels for the geometry, torch.nn for conv/BN (coordinates that need a gradient
+    still take the fused training chain over the materialised rows).  Both with identical semantics.
 The group_all SA layer (one group of all N points per cloud, xyz not centred) takes the same two paths: in eval one
 fp32 kernel that pools whole clouds (under both set_mlp_precision settings), in training one autograd Function.
 """
@@ -45,10 +48,15 @@ def set_fused_training(enabled):
     return prev
 
 
-def _train_fused(module, x0, convs, bns):
+def _train_fused(module, x0, convs, bns, *inputs):
+    """The fused training chain serves training mode and eval mode under autograd (the calls _fusable declines because
+    of autograd; each BatchNorm then normalises as torch would, see train_mlp._layer_tensors).  `inputs`: further
+    tensors of the call besides x0 that may require grad."""
     # the weight gradients are accumulated with fp32 atomics (order unspecified, like the reference's backward kernels):
     # bit-reproducible training (pointnet2_utils.set_deterministic / torch.use_deterministic_algorithms) keeps torch's modules
-    if not (_FUSED_TRAINING and module.training) or pointnet2_utils._deterministic():
+    if not _FUSED_TRAINING or pointnet2_utils._deterministic():
+        return False
+    if not (module.training or _autograd(module, x0, *inputs)):
         return False
     return train_mlp.fusable_training(x0, convs, bns)
 
@@ -56,7 +64,7 @@ def _train_fused(module, x0, convs, bns):
 def _train_blocks(module, convs, bns, xyzs, feats, nsample=None):
     """Training-mode block Functions (train_mlp.sa_scale_train / fp_block_train): wherever the fused training chain runs,
     for fp32 CUDA inputs, coordinates that need no gradient and at most 256 samples per ball (the pooled arg-max is uint8)."""
-    if not _train_fused(module, xyzs[0], convs, bns):
+    if not _train_fused(module, xyzs[0], convs, bns, *feats):
         return False
     if any(t.requires_grad for t in xyzs):
         return False
@@ -249,14 +257,17 @@ def _all_f32(*tensors):
     return all(t is None or t.dtype == torch.float32 for t in tensors)
 
 
+def _autograd(module, *tensors):
+    """Grad mode is on and one of `tensors` or a parameter of `module` requires grad: the call builds an autograd graph."""
+    return torch.is_grad_enabled() and (any(t is not None and t.requires_grad for t in tensors)
+                                        or any(p.requires_grad for p in module.parameters()))
+
+
 def _fusable(module, *tensors):
     """The fused kernels serve eval-mode, no-autograd calls on CUDA fp32 tensors with fp32 parameters; everything else
-    (training, autograd, half / double models or inputs) takes the reference's operator composition, where torch raises
-    the same dtype errors the reference would."""
-    if module.training:
-        return False
-    if torch.is_grad_enabled() and (any(t is not None and t.requires_grad for t in tensors)
-                                    or any(p.requires_grad for p in module.parameters())):
+    (training, autograd, half / double models or inputs) takes the training path (_train_fused) or the reference's
+    operator composition, where torch raises the same dtype errors the reference would."""
+    if module.training or _autograd(module, *tensors):
         return False
     if not all(t is None or t.is_cuda for t in tensors) or not _all_f32(*tensors):
         return False

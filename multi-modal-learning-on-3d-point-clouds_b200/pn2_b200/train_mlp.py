@@ -1,12 +1,17 @@
-"""Training-mode shared MLP: n x (1x1 conv -> BatchNorm (batch statistics) -> ReLU) as ONE autograd Function over
-channel-last row matrices, on the kernels of csrc/train_mlp.cu.
+"""Training-mode shared MLP: n x (1x1 conv -> BatchNorm -> ReLU) as ONE autograd Function over channel-last row matrices,
+on the kernels of csrc/train_mlp.cu.
 
 The reference runs this chain as torch.nn.Conv2d / Conv1d + BatchNorm + F.relu per layer (model/pointnet_util.py:105-107,
 162-165, 218-220): cuDNN fprop / dgrad / wgrad plus separate BatchNorm and ReLU passes in both directions.  Here every
 layer is one forward launch (the previous layer's normalisation and ReLU are applied while the operand is loaded, the
 batch statistics are reduced in the same pass) and three backward launches (BatchNorm reductions, input gradient, weight
-gradient); only the pre-BatchNorm activations are kept for the backward.  Semantics are torch's: biased variance for the
-normalisation, unbiased for the running estimate, eps / momentum of the module, running statistics updated in place.
+gradient); only the pre-BatchNorm activations are kept for the backward.  Semantics are torch's, per layer: a BatchNorm
+normalises with the batch statistics iff bn.training or it has no running statistics (biased variance for the
+normalisation, unbiased for the running estimate, eps / momentum of the module, running statistics and
+num_batches_tracked updated in place when bn.training and bn.track_running_stats); otherwise with its running statistics,
+which it leaves untouched -- a frozen BatchNorm (`m.eval()` inside a training network) and an eval() network under
+autograd.  Such a layer's forward reduces no statistics, its backward is dz = gamma rstd dy, and its conv bias gets the
+gradient sum dz.  One stack may mix the two modes.
 """
 import torch
 from torch.autograd import Function
@@ -21,18 +26,18 @@ def _stream(t):
 
 def _forward_layers(R, meta, tensors, dev, st, first):
     """The per-layer forward of a stack of L = len(tensors) // 6 layers over R rows; `first(cin, cout, W, b, z, stats)`
-    issues layer 0's forward (its operand is the caller's), layers 1.. read the previous z through act_in.
-    -> (zs, scales, shifts, mrs), per layer."""
+    issues layer 0's forward (its operand is the caller's; stats None: no statistics), layers 1.. read the previous z
+    through act_in.  -> (zs, scales, shifts, mrs), per layer."""
     L = len(tensors) // 6
     zs, scales, shifts, mrs = [], [], [], []
     for l in range(L):
         W, b, gamma, beta, rmean, rvar = tensors[6 * l:6 * l + 6]
-        eps, momentum = meta[l]
+        eps, momentum, batch = meta[l]
         cout, cin = W.shape
         Wc, bc = W.detach().contiguous(), b.detach().contiguous()
         gc, bec = gamma.detach().contiguous(), beta.detach().contiguous()
         z = torch.empty((R, cout), dtype=torch.float32, device=dev)
-        stats = torch.zeros((2, cout), dtype=torch.float64, device=dev)
+        stats = torch.zeros((2, cout), dtype=torch.float64, device=dev) if batch else None
         if l == 0:
             first(cin, cout, Wc, bc, z, stats)
         else:
@@ -41,15 +46,20 @@ def _forward_layers(R, meta, tensors, dev, st, first):
         scale = torch.empty(cout, dtype=torch.float32, device=dev)
         shift = torch.empty(cout, dtype=torch.float32, device=dev)
         mr = torch.empty((2, cout), dtype=torch.float64, device=dev)
-        _lib.call("pn2_train_bn_finalize", R, cout, ptr(stats), ptr(gc), ptr(bec), float(eps), float(momentum), ptr(scale), ptr(shift),
-                  ptr(mr), ptr(rmean), ptr(rvar), st)
+        if batch:
+            _lib.call("pn2_train_bn_finalize", R, cout, ptr(stats), ptr(gc), ptr(bec), float(eps), float(momentum), ptr(scale),
+                      ptr(shift), ptr(mr), ptr(rmean), ptr(rvar), st)
+        else:
+            _lib.call("pn2_train_bn_running", cout, ptr(rmean), ptr(rvar), ptr(gc), ptr(bec), float(eps), ptr(scale), ptr(shift),
+                      ptr(mr), st)
         zs.append(z); scales.append(scale); shifts.append(shift); mrs.append(mr)
     return zs, scales, shifts, mrs
 
 
-def _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first):
+def _backward_layers(R, g, zs, scales, shifts, mrs, params, batch, dev, st, first):
     """The per-layer backward from g = dL/da_L (R, C_L) down to layer 0; `first(cin, cout, Wt, g, z, scale, shift, coef, dW)`
-    issues layer 0's backward and returns its input gradient(s).  -> (that return value, parameter gradients)."""
+    issues layer 0's backward and returns its input gradient(s); batch[l]: layer l used batch statistics.
+    -> (that return value, parameter gradients)."""
     L = len(zs)
     grads = [None] * (6 * L)
     out = None
@@ -62,8 +72,14 @@ def _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first):
         coef = torch.empty((3, cout), dtype=torch.float32, device=dev)
         dgamma = torch.empty(cout, dtype=torch.float32, device=dev)
         dbeta = torch.empty(cout, dtype=torch.float32, device=dev)
-        gc = gamma.detach().contiguous()
-        _lib.call("pn2_train_bn_bwd_coeffs", R, cout, ptr(sums), ptr(mr), ptr(gc), ptr(coef), ptr(dgamma), ptr(dbeta), st)
+        if batch[l]:
+            _lib.call("pn2_train_bn_bwd_coeffs", R, cout, ptr(sums), ptr(mr), ptr(gamma.detach().contiguous()), ptr(coef), ptr(dgamma),
+                      ptr(dbeta), st)
+            dbias = torch.zeros_like(b)  # a bias in front of a batch-statistics BatchNorm has zero gradient
+        else:
+            dbias = torch.empty(cout, dtype=torch.float32, device=dev)
+            _lib.call("pn2_train_bn_running_bwd_coeffs", cout, ptr(sums), ptr(mr), ptr(scale), ptr(coef), ptr(dgamma), ptr(dbeta),
+                      ptr(dbias), st)
         dW = torch.zeros((cout, cin), dtype=torch.float32, device=dev)
         Wt = torch.empty((cin, cout), dtype=torch.float32, device=dev)
         _lib.call("pn2_transpose", 1, cout, cin, ptr(W.detach().contiguous()), ptr(Wt), st)  # W^T: an exact copy, one launch
@@ -75,7 +91,7 @@ def _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first):
                       ptr(z), ptr(scale), ptr(shift), ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), ptr(dW), st)
             g = g_in
         grads[6 * l] = dW.view_as(W)
-        grads[6 * l + 1] = torch.zeros_like(b)   # a bias in front of a batch-statistics BatchNorm has zero gradient
+        grads[6 * l + 1] = dbias.view_as(b)
         grads[6 * l + 2] = dgamma
         grads[6 * l + 3] = dbeta
     return out, grads
@@ -96,9 +112,10 @@ def _params(tensors, L):
 class _FusedMlpTrain(Function):
     @staticmethod
     def forward(ctx, x0, meta, *tensors):
-        """x0 (R, C0) fp32 rows; meta = [(eps, momentum or None, track), ...] per layer; tensors = (W (cout, cin), b, gamma,
-        beta, running_mean or None, running_var or None) per layer -> a_L (R, C_L).  The running statistics are updated in
-        place by the per-channel kernel (momentum, unbiased variance), like torch.nn.BatchNorm in training mode."""
+        """x0 (R, C0) fp32 rows; meta = [(eps, momentum, batch statistics?), ...] per layer; tensors = (W (cout, cin), b,
+        gamma, beta, running_mean or None, running_var or None) per layer -> a_L (R, C_L).  A batch-statistics layer updates
+        the running statistics it is given in place (momentum, unbiased variance), like torch.nn.BatchNorm in training
+        mode; a running-statistics layer only reads them."""
         L = len(tensors) // 6
         R = x0.shape[0]
         dev = x0.device
@@ -111,7 +128,7 @@ class _FusedMlpTrain(Function):
             zs, scales, shifts, mrs = _forward_layers(R, meta, tensors, dev, st, first)
             a = torch.empty_like(zs[-1])
             _lib.call("pn2_train_bn_relu", R, a.shape[1], ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(a), st)
-        ctx.L = L
+        ctx.L, ctx.batch = L, [m[2] for m in meta]
         ctx.save_for_backward(x0, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
         return a
 
@@ -131,7 +148,7 @@ class _FusedMlpTrain(Function):
                           ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), ptr(dW), st)
                 return g_in
 
-            g_x0, grads = _backward_layers(R, g_a.contiguous(), zs, scales, shifts, mrs, params, dev, st, first)
+            g_x0, grads = _backward_layers(R, g_a.contiguous(), zs, scales, shifts, mrs, params, ctx.batch, dev, st, first)
         return (g_x0, None, *grads)
 
 
@@ -155,7 +172,7 @@ def _pooled_grad_view(g):
 
 class _SaScaleTrain(Function):
     """One SA scale in training mode: grouping + centring + concat read by the first layer's load, the conv -> BatchNorm
-    (batch statistics) -> ReLU chain, and the max over nsample fused into the last layer.  Channel-last throughout."""
+    -> ReLU chain, and the max over nsample fused into the last layer.  Channel-last throughout."""
 
     @staticmethod
     def forward(ctx, xyz, new_xyz, idx, feat, order, meta, *tensors):
@@ -179,7 +196,7 @@ class _SaScaleTrain(Function):
             out = torch.empty((B, S, C), dtype=torch.float32, device=dev)
             arg = torch.empty((B, S, C), dtype=torch.uint8, device=dev)
             _lib.call("pn2_train_bn_relu_max", B * S, K, C, ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(out), C, 0, ptr(arg), st)
-        ctx.L, ctx.order, ctx.has_feat = L, order, feat is not None
+        ctx.L, ctx.order, ctx.has_feat, ctx.batch = L, order, feat is not None, [m[2] for m in meta]
         ctx.save_for_backward(xyz, new_xyz, idx, feat, arg, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
         return out
 
@@ -209,7 +226,7 @@ class _SaScaleTrain(Function):
                           ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), None, ptr(dW), st)
                 return g_in
 
-            g_in, grads = _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first)
+            g_in, grads = _backward_layers(R, g, zs, scales, shifts, mrs, params, ctx.batch, dev, st, first)
             g_feat = None
             if need_feat:
                 # grouping backward without atomics: every point sums the feature columns of its rows in row order
@@ -225,7 +242,7 @@ class _SaScaleTrain(Function):
 
 class _FpBlockTrain(Function):
     """One FP block in training mode: 3-NN interpolation and the skip concat read by the first layer's load, then the
-    conv -> BatchNorm (batch statistics) -> ReLU chain.  Channel-last throughout."""
+    conv -> BatchNorm -> ReLU chain.  Channel-last throughout."""
 
     @staticmethod
     def forward(ctx, feat1, feat2, idx, weight, n, meta, *tensors):
@@ -247,7 +264,7 @@ class _FpBlockTrain(Function):
             C = zs[-1].shape[1]
             a = torch.empty((B, n, C), dtype=torch.float32, device=dev)
             _lib.call("pn2_train_bn_relu", R, C, ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(a), st)
-        ctx.L, ctx.n = L, n
+        ctx.L, ctx.n, ctx.batch = L, n, [m[2] for m in meta]
         ctx.save_for_backward(feat1, feat2, idx, weight, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
         return a
 
@@ -273,7 +290,7 @@ class _FpBlockTrain(Function):
                           ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_in), ptr(g1), ptr(dW), st)
                 return g1, g_in
 
-            (g1, g_in), grads = _backward_layers(R, g_a.contiguous(), zs, scales, shifts, mrs, params, dev, st, first)
+            (g1, g_in), grads = _backward_layers(R, g_a.contiguous(), zs, scales, shifts, mrs, params, ctx.batch, dev, st, first)
             g2 = None
             if need2:
                 g2 = torch.empty((B, m, D2), dtype=torch.float32, device=dev)
@@ -296,7 +313,7 @@ class _FpBlockTrain(Function):
 
 class _SaAllTrain(Function):
     """The group_all SA layer in training mode: the [xyz | feat] rows read by the first layer's load, the conv ->
-    BatchNorm (batch statistics) -> ReLU chain, and the max over all N points of each cloud fused into the last layer."""
+    BatchNorm -> ReLU chain, and the max over all N points of each cloud fused into the last layer."""
 
     @staticmethod
     def forward(ctx, xyz, feat, meta, *tensors):
@@ -318,7 +335,7 @@ class _SaAllTrain(Function):
             out = torch.empty((B, 1, C), dtype=torch.float32, device=dev)
             arg = torch.empty((B, C), dtype=torch.int32, device=dev)
             _lib.call("pn2_train_bn_relu_max_all", B, N, C, ptr(zs[-1]), ptr(scales[-1]), ptr(shifts[-1]), ptr(out), C, 0, ptr(arg), st)
-        ctx.L = L
+        ctx.L, ctx.batch = L, [m[2] for m in meta]
         ctx.save_for_backward(xyz, feat, arg, *zs, *scales, *shifts, *mrs, *_params(tensors, L))
         return out
 
@@ -348,28 +365,31 @@ class _SaAllTrain(Function):
                           ptr(coef[0]), ptr(coef[1]), ptr(coef[2]), ptr(g_feat), None, ptr(dW), st)
                 return g_feat
 
-            g_feat, grads = _backward_layers(R, g, zs, scales, shifts, mrs, params, dev, st, first)
+            g_feat, grads = _backward_layers(R, g, zs, scales, shifts, mrs, params, ctx.batch, dev, st, first)
         return (None, g_feat, None, *grads)
 
 
 def _layer_tensors(convs, bns):
-    """(tensors, meta) of a conv / BatchNorm stack for the Functions above; counts the batch for the running statistics
-    (num_batches_tracked) like torch.nn.BatchNorm in training mode."""
+    """(tensors, meta) of a conv / BatchNorm stack for the Functions above, each BatchNorm in its own mode by torch's rule:
+    batch statistics iff bn.training or it has no running statistics; the running statistics (and num_batches_tracked)
+    are updated iff bn.training and bn.track_running_stats, and are read instead of the batch's otherwise."""
     tensors, meta = [], []
     for conv, bn in zip(convs, bns):
-        track = bn.track_running_stats and bn.running_mean is not None
-        if track:
+        batch = bn.training or bn.running_mean is None
+        update = bn.training and bn.track_running_stats and bn.running_mean is not None
+        if update:
             bn.num_batches_tracked += 1
-        momentum = bn.momentum if bn.momentum is not None else (1.0 / float(bn.num_batches_tracked) if track else 0.0)
+        momentum = bn.momentum if bn.momentum is not None else (1.0 / float(bn.num_batches_tracked) if update else 0.0)
+        running = update or not batch
         tensors += [conv.weight.reshape(conv.out_channels, conv.in_channels), conv.bias, bn.weight, bn.bias,
-                    bn.running_mean if track else None, bn.running_var if track else None]
-        meta.append((float(bn.eps), float(momentum)))
+                    bn.running_mean if running else None, bn.running_var if running else None]
+        meta.append((float(bn.eps), float(momentum), batch))
     return tensors, meta
 
 
 def fused_mlp_train(x0, convs, bns):
-    """x0 (R, C0) rows -> (R, C_L) = the conv -> BatchNorm(train) -> ReLU chain; updates the BatchNorm running statistics
-    (momentum, unbiased variance, num_batches_tracked) exactly like torch.nn.BatchNorm in training mode."""
+    """x0 (R, C0) rows -> (R, C_L) = the conv -> BatchNorm -> ReLU chain under autograd, every BatchNorm in its own mode
+    (batch or running statistics, running statistics and num_batches_tracked updated) exactly like torch.nn.BatchNorm."""
     tensors, meta = _layer_tensors(convs, bns)
     return _FusedMlpTrain.apply(x0, meta, *tensors)
 
@@ -377,7 +397,7 @@ def fused_mlp_train(x0, convs, bns):
 def sa_scale_train(xyz, new_xyz, idx, feat, order, convs, bns):
     """One SA scale in training mode, channel-last: xyz (B, N, 3), new_xyz (B, S, 3), idx (B, S, K) int32 (K <= 256),
     feat (B, N, D) or None, order _lib.ORDER_XYZ_FIRST (SSG) / ORDER_FEAT_FIRST (MSG) -> (B, S, C_L) = the max over the K
-    grouped rows of the conv -> BatchNorm(train) -> ReLU chain.  Same values, gradients and running statistics as
+    grouped rows of the conv -> BatchNorm -> ReLU chain.  Same values, gradients and running statistics as
     sample_and_group + fused_mlp_train + max(dim=2); xyz and new_xyz get no gradient."""
     xyz, new_xyz, idx = _lib.check_f32(xyz, "xyz"), _lib.check_f32(new_xyz, "new_xyz"), _lib.check_i32(idx, "idx")
     feat = _lib.check_f32(feat, "feat")
@@ -387,7 +407,7 @@ def sa_scale_train(xyz, new_xyz, idx, feat, order, convs, bns):
 
 def sa_all_train(xyz, feat, convs, bns):
     """The group_all SA layer in training mode, channel-last: xyz (B, N, 3), feat (B, N, D) or None -> (B, 1, C_L) = the
-    max over all N rows [xyz | feat] of each cloud of the conv -> BatchNorm(train) -> ReLU chain.  Same values, gradients
+    max over all N rows [xyz | feat] of each cloud of the conv -> BatchNorm -> ReLU chain.  Same values, gradients
     and running statistics as sample_and_group_all + fused_mlp_train + max(dim=2); xyz gets no gradient."""
     xyz, feat = _lib.check_f32(xyz, "xyz"), _lib.check_f32(feat, "feat")
     tensors, meta = _layer_tensors(convs, bns)
