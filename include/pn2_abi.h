@@ -361,6 +361,50 @@ int pn2_voxel_first_index(int b, int n, const float *xyz, const unsigned char *m
 int pn2_label_counts(int b, int n, int num_classes, const int32_t *select, const int32_t *count, const unsigned char *mask,
                      const long long *target, const unsigned char *pred, long long *out, void *stream);
 
+/* ---- whole-scene segmentation (csrc/scene_blocks.cu; the protocol is stated in oracle/whole_scene_ref.py) ----
+ * A scene is xyz (n,3) fp32.  Its grid has 1.5 m blocks in x and y from the scene minimum, block id = i * ny + j; a
+ * block's segment is the points inside it padded by 0.2 m, in ascending scene index.  Every call only enqueues work;
+ * the block counts and chunk counts the caller needs for its allocations are in the device record below, so one
+ * evaluation or labelling pass reads back one record.  Not graph-capturable by the caller: output sizes depend on data. */
+#define PN2_SCENE_MAX_BLOCKS 65536
+typedef struct pn2_scene_grid {
+    float cmin[3], cmax[3]; /* per-axis minimum / maximum of the scene */
+    int32_t nx, ny;         /* ceil(fp64(fl32(cmax - cmin)) / 1.5) along x / y (0 for a zero extent) */
+    int32_t count;          /* kept blocks after pn2_scene_keep, chunks after pn2_scene_chunks */
+    int32_t reserved;
+} pn2_scene_grid;
+/* Grid, bounds and segments: grid (device, written), seg_start (PN2_SCENE_MAX_BLOCKS + 2) int32, pos (4n) int32: the
+ * segment of block b is pos[seg_start[b] .. seg_start[b+1]).  n >= 1, 4n < 2^31.  A grid of zero extent or of more than
+ * PN2_SCENE_MAX_BLOCKS blocks gets empty segments. */
+int pn2_scene_index(int n, const float *xyz, pn2_scene_grid *grid, int32_t *seg_start, int32_t *pos, void *stream);
+/* Evaluation blocks: slot s of block b reads segment position ((h >> 32) * count) >> 32, h = splitmix64(seed *
+ * 0x9E3779B97F4A7C15 + (b << 32 | s)); a block is kept if it is non-empty and (core slots) / npoints >= 0.01 (fp64), core
+ * = inside the block padded by 0.001 m.  kept (PN2_SCENE_MAX_BLOCKS) int32 = kept ids ascending, grid->count = their number. */
+int pn2_scene_keep(int npoints, unsigned long long seed, const float *xyz, pn2_scene_grid *grid, const int32_t *seg_start,
+                   const int32_t *pos, int32_t *kept, void *stream);
+/* The nb kept blocks' samples (nx, ny, nb as read from the grid record; more than PN2_SCENE_MAX_BLOCKS blocks is refused):
+ * point_index (nb,npoints) int32 scene indices, points (nb,npoints,3+c) = [xyz | feats] rows, weights (nb,npoints) =
+ * labelweights[label] * core (core alone without labelweights; 0 for a label outside [0, num_classes)), target
+ * (nb,npoints) int64 = labels (labels, labelweights, target may be NULL). */
+int pn2_scene_sample(int nx, int ny, int nb, int npoints, unsigned long long seed, int c, const float *xyz, const float *feats,
+                     const long long *labels, const float *labelweights, int num_classes, const pn2_scene_grid *grid,
+                     const int32_t *seg_start, const int32_t *pos, const int32_t *kept, int32_t *point_index, float *points,
+                     long long *target, float *weights, void *stream);
+/* Labelling cover: every non-empty block b splits into k = ceil(count / npoints) chunks, chunk c holding segment positions
+ * c, c+k, c+2k, ...  first (PN2_SCENE_MAX_BLOCKS + 1) int32 = first chunk of each block (exclusive scan, ends with the
+ * total), grid->count = number of chunks. */
+int pn2_scene_chunks(int npoints, pn2_scene_grid *grid, const int32_t *seg_start, int32_t *first, void *stream);
+/* The chunks in (block, c) order: sizes (n_chunks) int32 = ceil((count - c) / k), point_index (n_chunks,npoints) int32 with
+ * slot s reading position c + k * (s mod size), points (n_chunks,npoints,3+c) rows. */
+int pn2_scene_chunk_rows(int nx, int ny, int n_chunks, int npoints, int c, const float *xyz, const float *feats,
+                         const pn2_scene_grid *grid, const int32_t *seg_start, const int32_t *pos, const int32_t *first,
+                         int32_t *point_index, int32_t *sizes, float *points, void *stream);
+/* votes (n,num_classes) int32, written in full: one vote votes[point_index, pred] per slot s < sizes[chunk] (integer
+ * atomics: exact, independent of order; predictions >= num_classes are ignored).  labels (n) uint8 or NULL = first
+ * maximum of each row, as numpy.argmax.  num_classes <= 256. */
+int pn2_scene_votes(int n_chunks, int npoints, const int32_t *point_index, const int32_t *sizes, const uint8_t *pred, int n,
+                    int num_classes, int32_t *votes, uint8_t *labels, void *stream);
+
 /* ---- proposal layer of the nuScenes detector (SURVEY 8f N4) ----
  * model/pointmaskrcnn.py:233-288 iou_spheres: spheres (x, y, z, r), 16-byte aligned rows -> iou (m,n) fp32, every
  * operation rounded to fp32 in the reference's order. */

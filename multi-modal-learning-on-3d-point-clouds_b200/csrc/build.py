@@ -14,6 +14,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 SOURCES = ["abi.cu", "fps.cu", "gather_group.cu", "ball_query.cu", "interpolate.cu", "lift.cu", "row_mlp.cu", "row_mlp_tc.cu", "train_mlp.cu", "grid.cu", "scatter_det.cu", "voxel.cu", "sphere.cu"]
+SOURCES.append("scene_blocks.cu")  # whole-scene block tiling, sampling and votes
 HEADERS = ["common.cuh", "row_mlp_tile.cuh", os.path.join(ROOT, "include", "pn2_abi.h")]
 OUT = os.path.join(HERE, "libpn2_b200.so")
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

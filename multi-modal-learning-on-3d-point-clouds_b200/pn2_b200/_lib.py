@@ -89,6 +89,12 @@ _SIGNATURES = {
     "pn2_train_max_bwd": [ctypes.c_longlong, _c_int, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
     "pn2_train_bn_relu_max_all": [ctypes.c_longlong, ctypes.c_longlong, _c_int] + [_vp] * 4 + [_c_int, _c_int, _vp, _vp],
     "pn2_train_max_bwd_all": [ctypes.c_longlong, ctypes.c_longlong, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
+    "pn2_scene_index": [_c_int] + [_vp] * 5,
+    "pn2_scene_keep": [_c_int, ctypes.c_ulonglong] + [_vp] * 6,
+    "pn2_scene_sample": [_c_int] * 4 + [ctypes.c_ulonglong, _c_int] + [_vp] * 4 + [_c_int] + [_vp] * 9,
+    "pn2_scene_chunks": [_c_int] + [_vp] * 4,
+    "pn2_scene_chunk_rows": [_c_int] * 5 + [_vp] * 10,
+    "pn2_scene_votes": [_c_int, _c_int, _vp, _vp, _vp, _c_int, _c_int, _vp, _vp, _vp],
 }
 _OTHER = {
     "pn2_last_error": ([], ctypes.c_char_p),

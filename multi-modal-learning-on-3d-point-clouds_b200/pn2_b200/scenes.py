@@ -64,6 +64,49 @@ def scannet_batch(first_scene_id, batch, npoints=8192):
     return out
 
 
+def scannet_room(scene_id, n_points, extent):
+    """A whole synthetic room, the input of pn2_b200.whole_scene: a floor, four walls and furniture boxes in a room of
+    extent x (0.6 .. 1) * extent metres (extent > 0.5), 2.7 m high, with 5 mm sensor noise.
+    -> (xyz (n_points, 3) float32 absolute coordinates, rgb (n_points, 3) float32 in [-0.5, 0.5], labels (n_points,)
+    int64: floor 1, walls 2, each box one class in 3..20, and about 5 % unannotated points (label 0) on every surface)."""
+    rng = np.random.default_rng(5000 + int(scene_id))
+    sx, sy, sz = float(extent), float(extent) * rng.uniform(0.6, 1.0), 2.7
+    n_floor, n_wall = int(n_points * 0.3), int(n_points * 0.1)
+    n_box_total = n_points - n_floor - 4 * n_wall
+    parts, labels = [], []
+    parts.append(np.stack([rng.uniform(0, sx, n_floor), rng.uniform(0, sy, n_floor), np.zeros(n_floor)], 1))
+    labels.append(np.full(n_floor, 1))
+    for ax, val in ((0, 0.0), (0, sx), (1, 0.0), (1, sy)):
+        w = np.empty((n_wall, 3))
+        w[:, ax] = val
+        w[:, 1 - ax] = rng.uniform(0, sy if ax == 0 else sx, n_wall)
+        w[:, 2] = rng.uniform(0, sz, n_wall)
+        parts.append(w)
+        labels.append(np.full(n_wall, 2))
+    n_boxes = max(int(sx * sy / 4), 3)
+    counts = np.full(n_boxes, n_box_total // n_boxes)
+    counts[: n_box_total - counts.sum()] += 1
+    for cnt in counts:
+        size = rng.uniform(0.2, 1.0, 3) * np.array([min(1.5, sx / 2), min(1.5, sy / 2), 1.5])
+        org = np.array([rng.uniform(0.05, sx - size[0] - 0.05), rng.uniform(0.05, sy - size[1] - 0.05), 0.0])
+        u, v, face = rng.uniform(0, 1, cnt), rng.uniform(0, 1, cnt), rng.integers(0, 5, cnt)
+        p = np.stack([u * size[0], v * size[1], np.full(cnt, size[2])], 1)  # top face
+        for f, (ax, val) in zip((1, 2, 3, 4), ((0, 0.0), (0, size[0]), (1, 0.0), (1, size[1]))):
+            m = face == f
+            p[m, ax] = val
+            p[m, 1 - ax] = u[m] * size[1 - ax]
+            p[m, 2] = v[m] * size[2]
+        parts.append(p + org)
+        labels.append(np.full(cnt, rng.integers(3, 21)))
+    xyz = np.concatenate(parts, 0) + rng.normal(0.0, 0.005, (n_points, 3))
+    xyz += np.array([rng.uniform(-5, 5), rng.uniform(-5, 5), 0.0])
+    labels = np.concatenate(labels).astype(np.int64)
+    labels[rng.random(n_points) < 0.05] = 0
+    perm = rng.permutation(n_points)  # scan order is not surface order
+    rgb = (rng.uniform(-0.5, 0.5, (n_points, 3)) * 0.2 + (labels[:, None] * np.array([0.37, 0.61, 0.83])) % 1.0 - 0.5).clip(-0.5, 0.5)
+    return xyz[perm].astype(np.float32), rgb[perm].astype(np.float32), labels[perm]
+
+
 def lidar_sweep(scene_id, npoints=None):
     """nuScenes-shaped synthetic 32-beam sweep (data_utils/NuScenesDataLoader.py:462-473): rays at
     elevations -30.67..+10.67 deg x 1085 azimuths onto a ground plane at z=-1.84 m plus boxes, range
