@@ -405,6 +405,32 @@ int pn2_scene_chunk_rows(int nx, int ny, int n_chunks, int npoints, int c, const
 int pn2_scene_votes(int n_chunks, int npoints, const int32_t *point_index, const int32_t *sizes, const uint8_t *pred, int n,
                     int num_classes, int32_t *votes, uint8_t *labels, void *stream);
 
+/* ---- training crops from a resident scene bank (csrc/scene_blocks.cu; the protocol is stated in
+ * oracle/scene_crops_ref.py) ----
+ * A bank packs s scenes: xyz (n,3) fp32, feats (n,c) fp32, labels (n) int64, offsets (s+1) int64, scene k = rows
+ * offsets[k] .. offsets[k+1]).  The library trusts offsets (0 = offsets[0] < offsets[1] < ... < offsets[s] = n): the
+ * caller validates them once.  bounds (s,6) fp32 = per-scene [min xyz | max xyz].  n >= 1, n < 2^31. */
+int pn2_scene_bank_bounds(int s, long long n, const float *xyz, const long long *offsets, float *bounds, void *stream);
+/* One training batch of b crops of npoints, crop i from scene scene_ids[i] (device int32).  The call reads the device
+ * counter *step, draws with h = splitmix64(seed * 0x9E3779B97F4A7C15 + step) and increments *step on the stream, so it
+ * makes no host read and a captured graph draws the next batch on every replay.  Per crop, try t = 0..9 centres a
+ * 1.5 m column (full z range) on the scene point at sample_pos(h, i, 2^31 + t, count); the first try whose 0.2 m padded
+ * column is >= 70 % labelled (label > 0) and whose 0.01 m core occupies >= 2 % of its 31 x 31 x 62 voxel keys is
+ * taken, else the tenth.  Slot j reads position sample_pos(h, i, j, padded count) of the padded points in ascending
+ * scene index.  sample_pos(h, i, j, m) = ((splitmix64(h * 0x9E3779B97F4A7C15 + (i << 32 | j)) >> 32) * m) >> 32.
+ * Outputs: point_index (b,npoints) int32 bank rows, points (b,npoints,3+c) [xyz | feats], target (b,npoints) int64
+ * labels, weights (b,npoints) fp32 = labelweights[label] * core (core alone when labelweights is NULL; 0 for a label
+ * outside [0, num_classes)), center (b) int32 scene-local index of the taken centre, tries (b) int32 in 1..10, valid (b)
+ * uint8.  A scene id outside [0, s) cannot be refused without a host read: its crop gets tries = 0, valid = 0, center
+ * = -1, point_index = -1 and zero rows, targets and weights.  max_count = the largest scene's point count (scratch of
+ * b * max_count int32).  Refused: b < 1, npoints < 1, b * npoints >= 2^31, c < 0, n < 1 or n >= 2^31, s < 1,
+ * max_count outside [1, n], null pointers. */
+int pn2_scene_crops(int s, long long n, int c, int max_count, const float *xyz, const float *feats, const long long *labels,
+                    const long long *offsets, const float *bounds, int b, const int32_t *scene_ids, int npoints,
+                    unsigned long long seed, long long *step, const float *labelweights, int num_classes, int32_t *point_index,
+                    float *points, long long *target, float *weights, int32_t *center, int32_t *tries, uint8_t *valid,
+                    void *stream);
+
 /* ---- proposal layer of the nuScenes detector (SURVEY 8f N4) ----
  * model/pointmaskrcnn.py:233-288 iou_spheres: spheres (x, y, z, r), 16-byte aligned rows -> iou (m,n) fp32, every
  * operation rounded to fp32 in the reference's order. */

@@ -12,6 +12,12 @@
 //   pn2_scene_chunk_rows  chunk sizes, index map and rows
 //   pn2_scene_votes   integer-atomic votes (exact, order independent), optional first-maximum labels
 //
+// The training loader's crops (oracle/scene_crops_ref.py) draw up to ten random 1.5 m columns per crop from a bank of
+// scenes resident on the device, with no host read, so a batch can be graph-captured:
+//   pn2_scene_bank_bounds  per-scene min / max, once per bank
+//   pn2_scene_crops   try 0 of every crop, then tries 1-9 where it failed (counts and a voxel bitmap per try, integer
+//                     atomics), the taken column compacted by a stable block scan, slots, rows
+//
 // Membership tests run in fp64 on the widened fp32 values, in the loader's operation order.
 #include <cub/cub.cuh>
 
@@ -264,7 +270,8 @@ __global__ void __launch_bounds__(THREADS) chunk_index_kernel(long long total, i
     point_index[e] = pos[seg_start[b] + c + k * (s % sizes[ch])];
 }
 
-// out (rows, 3 + C) = [xyz | feats] of point_index, exact copies
+// out (rows, 3 + C) = [xyz | feats] of point_index, exact copies; NEG_ZERO: a row of index -1 is zeros
+template <bool NEG_ZERO>
 __global__ void __launch_bounds__(THREADS) rows_kernel(long long total, int c, const int32_t *__restrict__ point_index,
                                                         const float *__restrict__ xyz, const float *__restrict__ feats,
                                                         float *__restrict__ out) {
@@ -272,7 +279,12 @@ __global__ void __launch_bounds__(THREADS) rows_kernel(long long total, int c, c
     for (long long e = (long long)blockIdx.x * THREADS + threadIdx.x; e < total; e += (long long)gridDim.x * THREADS) {
         const long long r = e / w;
         const int col = (int)(e - r * w);
-        const size_t p = (size_t)__ldg(point_index + r);
+        const int32_t i = __ldg(point_index + r);
+        if (NEG_ZERO && i < 0) {
+            out[e] = 0.f;
+            continue;
+        }
+        const size_t p = (size_t)i;
         out[e] = col < 3 ? __ldg(xyz + 3 * p + col) : __ldg(feats + p * c + (col - 3));
     }
 }
@@ -298,6 +310,278 @@ __global__ void __launch_bounds__(THREADS) vote_labels_kernel(int n, int num_cla
     for (int c = 1; c < num_classes; ++c)
         if (v[c] > bv) best = c, bv = v[c];
     labels[p] = (uint8_t)best;
+}
+
+// ---- training crops: the loader's random 1.5 m columns (pn2_scene_bank_bounds, pn2_scene_crops) ----
+constexpr double HALF_XY = 0.75;   // half the column edge (m); z spans the scene
+constexpr double CROP_PAD = 0.2;   // margin of the points taken into the crop
+constexpr double CROP_CORE = 0.01; // margin of the scored points, the ones whose voxels count
+constexpr int CROP_TRIES = 10;
+constexpr unsigned CENTRE_SLOT = 0x80000000u;          // try t draws its centre with counter 2^31 + t
+constexpr int VOX_KEYS = 32 * 31 * 62 + 32 * 62 + 62 + 1; // keys vx*31*62 + vy*62 + vz, vx, vy in 0..32, vz in 0..62
+constexpr int VOX_WORDS = (VOX_KEYS + 31) / 32;
+constexpr int TRY_HEAD = 8;       // try record: [labelled, NaN key seen, padded, valid, ...] then the occupancy bitmap
+constexpr int TRY_STRIDE = 2048;  // words per (crop, try) record
+constexpr int CROP_CHUNK = 8192;  // scene points per work item of a try or of the compaction
+constexpr int CROP_ITEMS = CROP_CHUNK / THREADS;
+constexpr int R_LAB = 0, R_NAN = 1, R_PAD = 2, R_VALID = 3;
+
+static_assert(VOX_KEYS == 63551 && TRY_HEAD + VOX_WORDS <= TRY_STRIDE, "occupancy bitmap layout");
+static_assert(CROP_ITEMS == 32, "the compaction keeps a thread's membership flags in one 32-bit mask");
+
+__device__ __forceinline__ int centre_pos(uint64_t h, int b, int t, int count) {
+    return sample_pos(h, b, (int)(CENTRE_SLOT + (unsigned)t), count);
+}
+
+// The loader's curmin / curmax in x and y (fp64: the fp32 centre widened, -/+ 0.75) and its z range [zmin, zmax] of the
+// scene.  Every point lies within the scene's z range, so z sets no membership condition.
+struct Column {
+    double lo[2], hi[2], zmin, zext;
+};
+
+__device__ __forceinline__ Column column_at(const float *__restrict__ xyz, long long p, const float *__restrict__ bnd) {
+    Column col;
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+        const double v = (double)xyz[3 * (size_t)p + a];
+        col.lo[a] = __dsub_rn(v, HALF_XY);
+        col.hi[a] = __dadd_rn(v, HALF_XY);
+    }
+    col.zmin = (double)bnd[2];
+    col.zext = __dsub_rn((double)bnd[5], col.zmin);
+    return col;
+}
+
+// p >= curmin - margin and p <= curmax + margin in x and y, fp64
+__device__ __forceinline__ bool in_column(const Column &col, float x, float y, double margin) {
+    const double vx = x, vy = y;
+    return vx >= __dsub_rn(col.lo[0], margin) && vx <= __dadd_rn(col.hi[0], margin) && vy >= __dsub_rn(col.lo[1], margin) &&
+           vy <= __dadd_rn(col.hi[1], margin);
+}
+
+// ceil((p - curmin) / (curmax - curmin) * cells), the loader's fp64 order; -0.0 and 0.0 give the same key
+__device__ __forceinline__ double vox(double p, double lo, double ext, double cells) {
+    return ceil(__dmul_rn(__ddiv_rn(__dsub_rn(p, lo), ext), cells));
+}
+
+// Voxel key of a core point, or -1 for the one key value numpy gives every NaN (zero z extent makes all of them NaN).
+// For finite points in the core vx, vy lie in -0..32 and vz in 0..62, so the range test fails for NaN only.
+__device__ __forceinline__ int vox_key(const Column &col, float x, float y, float z) {
+    const double vx = vox(x, col.lo[0], __dsub_rn(col.hi[0], col.lo[0]), 31.0);
+    const double vy = vox(y, col.lo[1], __dsub_rn(col.hi[1], col.lo[1]), 31.0);
+    const double vz = vox(z, col.zmin, col.zext, 62.0);
+    if (!(vx >= 0.0 && vx <= 32.0 && vy >= 0.0 && vy <= 32.0 && vz >= 0.0 && vz <= 62.0)) return -1;
+    return (int)vx * (31 * 62) + (int)vy * 62 + (int)vz;
+}
+
+__device__ __forceinline__ bool bad_scene(int sid, int s) { return sid < 0 || sid >= s; }
+
+// one CTA per scene (strided): per-axis fp32 minimum and maximum, exact in any order
+__global__ void __launch_bounds__(THREADS) bank_bounds_kernel(int s, const float *__restrict__ xyz, const long long *__restrict__ offsets,
+                                                               float *__restrict__ bounds) {
+    using Reduce = cub::BlockReduce<float, THREADS>;
+    __shared__ typename Reduce::TempStorage tmp;
+    for (int k = blockIdx.x; k < s; k += gridDim.x) {
+        float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+        for (long long p = offsets[k] + threadIdx.x; p < offsets[k + 1]; p += THREADS)
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                const float v = xyz[3 * (size_t)p + a];
+                lo[a] = fminf(lo[a], v);
+                hi[a] = fmaxf(hi[a], v);
+            }
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            const float l = Reduce(tmp).Reduce(lo[a], cub::Min());
+            __syncthreads();
+            const float h = Reduce(tmp).Reduce(hi[a], cub::Max());
+            __syncthreads();
+            if (threadIdx.x == 0) bounds[6 * (size_t)k + a] = l, bounds[6 * (size_t)k + 3 + a] = h;
+        }
+    }
+}
+
+// h of this call, then step + 1.  Every later kernel of the call reads h, so the counter may move on here.
+__global__ void crop_draw_kernel(uint64_t seed, long long *__restrict__ step, uint64_t *__restrict__ h) {
+    const uint64_t st = (uint64_t)*step;
+    *h = mix64(seed * 0x9E3779B97F4A7C15ull + st);
+    *step = (long long)(st + 1);
+}
+
+// Work item (crop b, try t, chunk k of the scene): padded and labelled counts and the occupancy bits of the core points
+// of CROP_CHUNK scene points.  Bits are gathered in shared memory and OR-ed into the try's record; counts combine by
+// integer atomics (labelled) and per-chunk slots (padded, which the compaction also needs), so the result is exact and
+// independent of CTA order.  Tries t >= 1 of a crop whose try 0 is valid are skipped.
+__global__ void __launch_bounds__(THREADS) crop_try_kernel(int nb, int s, int t0, int ntries, int chunks, const float *__restrict__ xyz,
+                                                            const long long *__restrict__ labels, const long long *__restrict__ offsets,
+                                                            const float *__restrict__ bounds, const int32_t *__restrict__ scene_ids,
+                                                            const uint64_t *__restrict__ hp, int32_t *__restrict__ rec,
+                                                            int32_t *__restrict__ chunk_pad) {
+    using Reduce = cub::BlockReduce<int, THREADS>;
+    __shared__ typename Reduce::TempStorage tmp;
+    __shared__ uint32_t bits[VOX_WORDS];
+    __shared__ int nan_key;
+    const uint64_t h = *hp;
+    const long long items = (long long)nb * ntries * chunks;
+    for (long long it = blockIdx.x; it < items; it += gridDim.x) {
+        const int k = (int)(it % chunks);
+        const long long bt = it / chunks;
+        const int t = t0 + (int)(bt % ntries), b = (int)(bt / ntries);
+        const int sid = scene_ids[b];
+        if (bad_scene(sid, s)) continue;
+        if (t > 0 && rec[(size_t)b * CROP_TRIES * TRY_STRIDE + R_VALID]) continue;
+        const long long off = offsets[sid];
+        const int count = (int)(offsets[sid + 1] - off), p0 = k * CROP_CHUNK;
+        if (p0 >= count) continue;
+        int32_t *r = rec + ((size_t)b * CROP_TRIES + t) * TRY_STRIDE;
+        const Column col = column_at(xyz, off + centre_pos(h, b, t, count), bounds + 6 * (size_t)sid);
+        for (int w = threadIdx.x; w < VOX_WORDS; w += THREADS) bits[w] = 0;
+        if (threadIdx.x == 0) nan_key = 0;
+        __syncthreads();
+        int pad = 0, lab = 0;
+        const int p1 = min(count, p0 + CROP_CHUNK);
+        for (int p = p0 + threadIdx.x; p < p1; p += THREADS) {
+            const float *q = xyz + 3 * (size_t)(off + p);
+            const float x = q[0], y = q[1];
+            if (!in_column(col, x, y, CROP_PAD)) continue;
+            ++pad;
+            lab += labels[off + p] > 0;
+            if (!in_column(col, x, y, CROP_CORE)) continue;
+            const int key = vox_key(col, x, y, q[2]);
+            if (key >= 0) atomicOr(&bits[key >> 5], 1u << (key & 31));
+            else nan_key = 1;
+        }
+        pad = Reduce(tmp).Sum(pad);
+        __syncthreads();
+        lab = Reduce(tmp).Sum(lab);
+        __syncthreads();  // bits and nan_key complete
+        if (threadIdx.x == 0) {
+            chunk_pad[((size_t)b * CROP_TRIES + t) * chunks + k] = pad;
+            if (lab) atomicAdd(r + R_LAB, lab);
+            if (nan_key) atomicOr(r + R_NAN, 1);
+        }
+        for (int w = threadIdx.x; w < VOX_WORDS; w += THREADS)
+            if (bits[w]) atomicOr((uint32_t *)r + TRY_HEAD + w, bits[w]);
+        __syncthreads();  // before the next item clears bits
+    }
+}
+
+// Work item (crop b, try t): padded count, occupied keys (+1 for NaN) and the loader's test, fp64 in its order:
+// labelled / padded >= 0.7 and keys / 31 / 31 / 62 >= 0.02.
+__global__ void __launch_bounds__(THREADS) crop_judge_kernel(int nb, int s, int t0, int ntries, int chunks, const long long *__restrict__ offsets,
+                                                              const int32_t *__restrict__ scene_ids, int32_t *__restrict__ rec,
+                                                              const int32_t *__restrict__ chunk_pad) {
+    using Reduce = cub::BlockReduce<int, THREADS>;
+    __shared__ typename Reduce::TempStorage tmp;
+    for (int it = blockIdx.x; it < nb * ntries; it += gridDim.x) {
+        const int t = t0 + it % ntries, b = it / ntries;
+        const int sid = scene_ids[b];
+        if (bad_scene(sid, s)) continue;
+        if (t > 0 && rec[(size_t)b * CROP_TRIES * TRY_STRIDE + R_VALID]) continue;
+        int32_t *r = rec + ((size_t)b * CROP_TRIES + t) * TRY_STRIDE;
+        const int nch = ceil_div((int)(offsets[sid + 1] - offsets[sid]), CROP_CHUNK);
+        const int32_t *cp = chunk_pad + ((size_t)b * CROP_TRIES + t) * chunks;
+        int pad = 0, keys = 0;
+        for (int k = threadIdx.x; k < nch; k += THREADS) pad += cp[k];
+        for (int w = threadIdx.x; w < VOX_WORDS; w += THREADS) keys += __popc((uint32_t)r[TRY_HEAD + w]);
+        pad = Reduce(tmp).Sum(pad);
+        __syncthreads();
+        keys = Reduce(tmp).Sum(keys);
+        if (threadIdx.x == 0) {
+            keys += r[R_NAN];
+            r[R_PAD] = pad;
+            r[R_VALID] = pad > 0 && __ddiv_rn((double)r[R_LAB], (double)pad) >= 0.7 &&
+                         __ddiv_rn(__ddiv_rn(__ddiv_rn((double)keys, 31.0), 31.0), 62.0) >= 0.02;
+        }
+        __syncthreads();
+    }
+}
+
+// Work item (crop b, chunk k): the taken try (the first valid one, else the tenth), then the scene-local indices of its
+// padded points in chunk k, in ascending order, at local[b * max_count + (padded points of the chunks before k) ...]
+// (a stable block scan).  Chunk 0 also writes the crop's center, tries, valid and padded count.
+__global__ void __launch_bounds__(THREADS) crop_compact_kernel(int nb, int s, int chunks, int max_count, const float *__restrict__ xyz,
+                                                                const long long *__restrict__ offsets, const float *__restrict__ bounds,
+                                                                const int32_t *__restrict__ scene_ids, const uint64_t *__restrict__ hp,
+                                                                const int32_t *__restrict__ rec, const int32_t *__restrict__ chunk_pad,
+                                                                int32_t *__restrict__ local, int32_t *__restrict__ crop_count,
+                                                                int32_t *__restrict__ center, int32_t *__restrict__ tries,
+                                                                uint8_t *__restrict__ valid) {
+    using Reduce = cub::BlockReduce<int, THREADS>;
+    using Scan = cub::BlockScan<int, THREADS>;
+    __shared__ typename Reduce::TempStorage rtmp;
+    __shared__ typename Scan::TempStorage stmp;
+    const uint64_t h = *hp;
+    for (long long it = blockIdx.x; it < (long long)nb * chunks; it += gridDim.x) {
+        const int k = (int)(it % chunks), b = (int)(it / chunks);
+        const int sid = scene_ids[b];
+        if (bad_scene(sid, s)) {
+            if (k == 0 && threadIdx.x == 0) center[b] = -1, tries[b] = 0, valid[b] = 0, crop_count[b] = 0;
+            continue;
+        }
+        const long long off = offsets[sid];
+        const int count = (int)(offsets[sid + 1] - off), p0 = k * CROP_CHUNK;
+        if (p0 >= count) continue;
+        const int32_t *r0 = rec + (size_t)b * CROP_TRIES * TRY_STRIDE;
+        int t = 0;
+        while (t < CROP_TRIES - 1 && !r0[(size_t)t * TRY_STRIDE + R_VALID]) ++t;
+        const int32_t *r = r0 + (size_t)t * TRY_STRIDE;
+        const int c = centre_pos(h, b, t, count);
+        if (k == 0 && threadIdx.x == 0) center[b] = c, tries[b] = t + 1, valid[b] = (uint8_t)r[R_VALID], crop_count[b] = r[R_PAD];
+        const int32_t *cp = chunk_pad + ((size_t)b * CROP_TRIES + t) * chunks;
+        int base = 0;
+        for (int j = threadIdx.x; j < k; j += THREADS) base += cp[j];
+        base = Reduce(rtmp).Sum(base);  // valid in thread 0
+        const Column col = column_at(xyz, off + c, bounds + 6 * (size_t)sid);
+        const int q0 = p0 + threadIdx.x * CROP_ITEMS;
+        uint32_t in = 0;
+#pragma unroll 4
+        for (int i = 0; i < CROP_ITEMS; ++i) {
+            const int p = q0 + i;
+            if (p < count) {
+                const float *q = xyz + 3 * (size_t)(off + p);
+                if (in_column(col, q[0], q[1], CROP_PAD)) in |= 1u << i;
+            }
+        }
+        // thread 0 feeds base into the scan, so every other thread's exclusive sum already includes it
+        int rank;
+        Scan(stmp).ExclusiveSum(threadIdx.x == 0 ? base + __popc(in) : __popc(in), rank);
+        int32_t *out = local + (size_t)b * max_count + (threadIdx.x == 0 ? base : rank);
+        for (; in; in &= in - 1) *out++ = q0 + __ffs(in) - 1;
+        __syncthreads();
+    }
+}
+
+// slot (b, j): bank row of position sample_pos(h, b, j, padded count) of the taken column, its target and weight
+__global__ void __launch_bounds__(THREADS) crop_slot_kernel(long long total, int npoints, int s, int max_count, int num_classes,
+                                                             const float *__restrict__ xyz, const long long *__restrict__ labels,
+                                                             const long long *__restrict__ offsets, const float *__restrict__ bounds,
+                                                             const int32_t *__restrict__ scene_ids, const uint64_t *__restrict__ hp,
+                                                             const int32_t *__restrict__ local, const int32_t *__restrict__ crop_count,
+                                                             const int32_t *__restrict__ center, const float *__restrict__ labelweights,
+                                                             int32_t *__restrict__ point_index, long long *__restrict__ target,
+                                                             float *__restrict__ weights) {
+    const long long e = (long long)blockIdx.x * THREADS + threadIdx.x;
+    if (e >= total) return;
+    const int b = (int)(e / npoints), j = (int)(e - (long long)b * npoints);
+    const int sid = scene_ids[b];
+    // an empty column needs a non-finite centre (a finite one lies in its own column): nothing to draw from
+    if (bad_scene(sid, s) || crop_count[b] == 0) {
+        point_index[e] = -1;
+        target[e] = 0;
+        weights[e] = 0.f;
+        return;
+    }
+    const long long off = offsets[sid];
+    const long long p = off + local[(size_t)b * max_count + sample_pos(*hp, b, j, crop_count[b])];
+    point_index[e] = (int32_t)p;
+    const Column col = column_at(xyz, off + center[b], bounds + 6 * (size_t)sid);
+    const bool core = in_column(col, xyz[3 * (size_t)p], xyz[3 * (size_t)p + 1], CROP_CORE);
+    const long long l = labels[p];
+    target[e] = l;
+    float w = core ? 1.f : 0.f;
+    if (labelweights) w = (l >= 0 && l < num_classes) ? __fmul_rn(labelweights[l], w) : 0.f;
+    weights[e] = w;
 }
 
 inline unsigned blocks_for(long long total) { return (unsigned)((total + THREADS - 1) / THREADS); }
@@ -372,7 +656,7 @@ extern "C" int pn2_scene_sample(int nx, int ny, int nb, int npoints, unsigned lo
     sample_kernel<<<blocks_for(slots), THREADS, 0, s>>>(slots, npoints, (uint64_t)seed, xyz, labels, labelweights, num_classes, grid,
                                                         seg_start, pos, kept, point_index, target, weights);
     PN2_LAUNCH_OK("sample_kernel");
-    rows_kernel<<<strided_blocks(elems), THREADS, 0, s>>>(elems, c, point_index, xyz, feats, points);
+    rows_kernel<false><<<strided_blocks(elems), THREADS, 0, s>>>(elems, c, point_index, xyz, feats, points);
     PN2_LAUNCH_OK("rows_kernel");
     return PN2_OK;
 }
@@ -405,7 +689,7 @@ extern "C" int pn2_scene_chunk_rows(int nx, int ny, int n_chunks, int npoints, i
     chunk_index_kernel<<<blocks_for(slots), THREADS, 0, s>>>(slots, npoints, seg_start, pos, first, (const int32_t *)block_of.ptr, sizes,
                                                              point_index);
     PN2_LAUNCH_OK("chunk_index_kernel");
-    rows_kernel<<<strided_blocks(elems), THREADS, 0, s>>>(elems, c, point_index, xyz, feats, points);
+    rows_kernel<false><<<strided_blocks(elems), THREADS, 0, s>>>(elems, c, point_index, xyz, feats, points);
     PN2_LAUNCH_OK("rows_kernel");
     return PN2_OK;
 }
@@ -428,5 +712,72 @@ extern "C" int pn2_scene_votes(int n_chunks, int npoints, const int32_t *point_i
         vote_labels_kernel<<<blocks_for(n), THREADS, 0, s>>>(n, num_classes, votes, labels);
         PN2_LAUNCH_OK("vote_labels_kernel");
     }
+    return PN2_OK;
+}
+
+extern "C" int pn2_scene_bank_bounds(int s, long long n, const float *xyz, const long long *offsets, float *bounds, void *stream) {
+    using namespace pn2;
+    PN2_REQUIRE(s >= 1, "scene_bank_bounds: need s >= 1 scenes (s=%d)", s);
+    PN2_REQUIRE(n >= 1 && n < (1ll << 31), "scene_bank_bounds: need 1 <= n < 2^31 points (n=%lld)", n);
+    PN2_REQUIRE(xyz && offsets && bounds, "scene_bank_bounds: null pointer");
+    bank_bounds_kernel<<<min(s, 4 * sm_count()), THREADS, 0, (cudaStream_t)stream>>>(s, xyz, offsets, bounds);
+    PN2_LAUNCH_OK("bank_bounds_kernel");
+    return PN2_OK;
+}
+
+extern "C" int pn2_scene_crops(int s, long long n, int c, int max_count, const float *xyz, const float *feats, const long long *labels,
+                               const long long *offsets, const float *bounds, int b, const int32_t *scene_ids, int npoints,
+                               unsigned long long seed, long long *step, const float *labelweights, int num_classes, int32_t *point_index,
+                               float *points, long long *target, float *weights, int32_t *center, int32_t *tries, uint8_t *valid,
+                               void *stream) {
+    using namespace pn2;
+    PN2_REQUIRE(b >= 1 && npoints >= 1 && c >= 0, "scene_crops: bad dims b=%d npoints=%d c=%d", b, npoints, c);
+    PN2_REQUIRE((long long)b * npoints < (1ll << 31), "scene_crops: b * npoints must be < 2^31");
+    PN2_REQUIRE(s >= 1 && n >= 1 && n < (1ll << 31), "scene_crops: need s >= 1 scenes and 1 <= n < 2^31 points (s=%d n=%lld)", s, n);
+    PN2_REQUIRE(max_count >= 1 && max_count <= n, "scene_crops: max_count must be in [1, n] (max_count=%d)", max_count);
+    PN2_REQUIRE(!labelweights || num_classes >= 1, "scene_crops: labelweights need num_classes >= 1");
+    PN2_REQUIRE(xyz && (c == 0 || feats) && labels && offsets && bounds && scene_ids && step && point_index && points && target &&
+                    weights && center && tries && valid,
+                "scene_crops: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int chunks = ceil_div(max_count, CROP_CHUNK);
+    auto round = [](size_t v) { return (v + 255) / 256 * 256; };
+    const size_t h_bytes = 256, rec_bytes = round((size_t)b * CROP_TRIES * TRY_STRIDE * sizeof(int32_t)),
+                 cp_bytes = round((size_t)b * CROP_TRIES * chunks * sizeof(int32_t)), cc_bytes = round((size_t)b * sizeof(int32_t)),
+                 local_bytes = (size_t)b * max_count * sizeof(int32_t);
+    Scratch scratch_mem(st);  // [h | try records | per-chunk padded counts | padded count per crop | compacted columns]
+    PN2_CUDA(scratch_mem.alloc(h_bytes + rec_bytes + cp_bytes + cc_bytes + local_bytes));
+    unsigned char *scratch = (unsigned char *)scratch_mem.ptr;
+    uint64_t *h = (uint64_t *)scratch;
+    int32_t *rec = (int32_t *)(scratch + h_bytes), *chunk_pad = (int32_t *)(scratch + h_bytes + rec_bytes);
+    int32_t *crop_count = (int32_t *)(scratch + h_bytes + rec_bytes + cp_bytes);
+    int32_t *local = (int32_t *)(scratch + h_bytes + rec_bytes + cp_bytes + cc_bytes);
+    PN2_CUDA(cudaMemsetAsync(rec, 0, rec_bytes, st));
+    crop_draw_kernel<<<1, 1, 0, st>>>((uint64_t)seed, step, h);
+    PN2_LAUNCH_OK("crop_draw_kernel");
+    const long long cap = 32ll * sm_count();
+    auto ctas = [cap](long long items) { return (unsigned)(items < cap ? items : cap); };
+    // try 0 of every crop first; tries 1-9 only where it failed (the other CTAs skip at once)
+    crop_try_kernel<<<ctas((long long)b * chunks), THREADS, 0, st>>>(b, s, 0, 1, chunks, xyz, labels, offsets, bounds, scene_ids, h, rec,
+                                                                      chunk_pad);
+    PN2_LAUNCH_OK("crop_try_kernel");
+    crop_judge_kernel<<<ctas(b), THREADS, 0, st>>>(b, s, 0, 1, chunks, offsets, scene_ids, rec, chunk_pad);
+    PN2_LAUNCH_OK("crop_judge_kernel");
+    crop_try_kernel<<<ctas((long long)b * (CROP_TRIES - 1) * chunks), THREADS, 0, st>>>(b, s, 1, CROP_TRIES - 1, chunks, xyz, labels, offsets,
+                                                                                         bounds, scene_ids, h, rec, chunk_pad);
+    PN2_LAUNCH_OK("crop_try_kernel");
+    crop_judge_kernel<<<ctas((long long)b * (CROP_TRIES - 1)), THREADS, 0, st>>>(b, s, 1, CROP_TRIES - 1, chunks, offsets, scene_ids, rec,
+                                                                                  chunk_pad);
+    PN2_LAUNCH_OK("crop_judge_kernel");
+    crop_compact_kernel<<<ctas((long long)b * chunks), THREADS, 0, st>>>(b, s, chunks, max_count, xyz, offsets, bounds, scene_ids, h, rec,
+                                                                          chunk_pad, local, crop_count, center, tries, valid);
+    PN2_LAUNCH_OK("crop_compact_kernel");
+    const long long slots = (long long)b * npoints, elems = slots * (3 + c);
+    crop_slot_kernel<<<blocks_for(slots), THREADS, 0, st>>>(slots, npoints, s, max_count, labelweights ? num_classes : 0, xyz, labels, offsets,
+                                                            bounds, scene_ids, h, local, crop_count, center, labelweights, point_index,
+                                                            target, weights);
+    PN2_LAUNCH_OK("crop_slot_kernel");
+    rows_kernel<true><<<strided_blocks(elems), THREADS, 0, st>>>(elems, c, point_index, xyz, feats, points);
+    PN2_LAUNCH_OK("rows_kernel");
     return PN2_OK;
 }

@@ -95,6 +95,9 @@ _SIGNATURES = {
     "pn2_scene_chunks": [_c_int] + [_vp] * 4,
     "pn2_scene_chunk_rows": [_c_int] * 5 + [_vp] * 10,
     "pn2_scene_votes": [_c_int, _c_int, _vp, _vp, _vp, _c_int, _c_int, _vp, _vp, _vp],
+    "pn2_scene_bank_bounds": [_c_int, ctypes.c_longlong, _vp, _vp, _vp, _vp],
+    "pn2_scene_crops": [_c_int, ctypes.c_longlong, _c_int, _c_int] + [_vp] * 5 + [_c_int, _vp, _c_int, ctypes.c_ulonglong, _vp, _vp,
+                                                                                  _c_int] + [_vp] * 8,
 }
 _OTHER = {
     "pn2_last_error": ([], ctypes.c_char_p),
