@@ -363,6 +363,7 @@ train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, floa
     using S = TileShape<NT>;
     extern __shared__ __align__(16) float smem[];
     __shared__ float cpart[2][TG_THREADS / 32][NT];  // per-warp partial sums of the tile's columns (sum, sum of squares)
+    __shared__ float tpiv[NT];                       // the tile's pivots (its first row of z)
     const int cout = w.n_total, cin = w.k_total;
     const int tid = threadIdx.x, tx = tid % S::TX, ty = tid / S::TX;
     const int ntn = (cout + NT - 1) / NT;
@@ -377,6 +378,20 @@ train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, floa
         float bv[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) bv[j] = col + j < cout ? __ldg(bias + col + j) : 0.f;
+        // The statistics are summed CENTRED on a pivot p per column, the tile's first row: s1 = sum (z - p), s2 =
+        // sum (z - p)^2, expanded to sum z = s1 + n p and sum z^2 = s2 + 2 p s1 + n p^2 in fp64.  An fp32 sum of z^2 loses
+        // (mean / std)^2 of its relative precision in var = E[z^2] - mean^2 (1e-4 relative at mean / std = 100); the
+        // centred sums lose nothing to the mean, and both expansions use the same s1, so the rounding of s1 cancels in var.
+        float pv[4] = {0.f, 0.f, 0.f, 0.f};
+        if constexpr (STATS) {
+            if (ty == 0) {  // row m0 (always valid) is row 0 of the ty == 0 threads
+#pragma unroll
+                for (int j = 0; j < 4; ++j) tpiv[tx * 4 + j] = acc[0][j] + bv[j];
+            }
+            __syncthreads();
+#pragma unroll
+            for (int j = 0; j < 4; ++j) pv[j] = tpiv[tx * 4 + j];
+        }
 #pragma unroll
         for (int i = 0; i < S::TM; ++i) {
             const long long r = m0 + ty * S::TM + i;
@@ -386,8 +401,9 @@ train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, floa
             for (int j = 0; j < 4; ++j) {
                 v[j] = acc[i][j] + bv[j];
                 if (STATS && col + j < cout) {
-                    s1[j] += v[j];
-                    s2[j] = fmaf(v[j], v[j], s2[j]);
+                    const float dv = v[j] - pv[j];
+                    s1[j] += dv;
+                    s2[j] = fmaf(dv, dv, s2[j]);
                 }
             }
             if (col + 3 < cout && (cout & 3) == 0) {
@@ -418,11 +434,16 @@ train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, floa
             }
         }
         __syncthreads();
-        if (tid < 2 * NT && n0 + (tid % NT) < cout) {
-            float t = 0.f;
+        if (tid < NT && n0 + tid < cout) {
+            float t1 = 0.f, t2 = 0.f;
 #pragma unroll
-            for (int w8 = 0; w8 < TG_THREADS / 32; ++w8) t += cpart[tid / NT][w8][tid % NT];
-            atomicAdd(stats + (size_t)(tid / NT) * cout + n0 + (tid % NT), (double)t);
+            for (int w8 = 0; w8 < TG_THREADS / 32; ++w8) {
+                t1 += cpart[0][w8][tid];
+                t2 += cpart[1][w8][tid];
+            }
+            const double p = (double)tpiv[tid], n = (double)min((long long)TG_M, xin.rows - m0);
+            atomicAdd(stats + n0 + tid, fma(n, p, (double)t1));
+            atomicAdd(stats + (size_t)cout + n0 + tid, (double)t2 + p * (2.0 * (double)t1 + n * p));
         }
         __syncthreads();
     }
@@ -432,29 +453,34 @@ train_linear_fwd_kernel(LX xin, WeightIn w, const float *__restrict__ bias, floa
 __global__ void __launch_bounds__(256)
 train_bn_bwd_reduce_kernel(long long rows, int c, const float *__restrict__ g, const float *__restrict__ z, const float *__restrict__ scale,
                            const float *__restrict__ shift, double *__restrict__ sums) {
-    // lanes along channels (coalesced rows), the 8 warps of a CTA and the CTAs of the grid along rows
+    // lanes along channels (coalesced rows), the 8 warps of a CTA and the CTAs of the grid along rows.
+    // Each lane reduces sum dy (z - p) about a pivot p = the first z of its row range and adds p sum dy back in fp64: the
+    // coefficients use S2 - mean S1, which an fp32 sum of dy z buries under its rounding once |mean| >> std.  S1 is
+    // combined across the warps in fp64 too, so S2 carries exactly the S1 its pivot terms were formed from.
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    __shared__ float red[2][8][32];
+    __shared__ double red[2][8][32];
+    const long long r0 = (long long)blockIdx.x * 8 + warp;
     for (int c0 = 0; c0 < c; c0 += 32) {
         const int ch = c0 + lane;
-        float s1 = 0.f, s2 = 0.f;
+        float s1 = 0.f, s2 = 0.f, p = 0.f;
         if (ch < c) {
             const float sc = __ldg(scale + ch), sh = __ldg(shift + ch);
-            for (long long r = (long long)blockIdx.x * 8 + warp; r < rows; r += (long long)gridDim.x * 8) {
+            if (r0 < rows) p = __ldg(z + r0 * c + ch);
+            for (long long r = r0; r < rows; r += (long long)gridDim.x * 8) {
                 const float zz = __ldg(z + r * c + ch), gg = __ldg(g + r * c + ch);
                 const float dy = fmaf(zz, sc, sh) > 0.f ? gg : 0.f;
                 s1 += dy;
-                s2 = fmaf(dy, zz, s2);
+                s2 = fmaf(dy, zz - p, s2);
             }
         }
-        red[0][warp][lane] = s1;
-        red[1][warp][lane] = s2;
+        red[0][warp][lane] = (double)s1;
+        red[1][warp][lane] = fma((double)p, (double)s1, (double)s2);
         __syncthreads();
         if (warp < 2 && ch < c) {
-            float t = 0.f;
+            double t = 0.0;
 #pragma unroll
             for (int w8 = 0; w8 < 8; ++w8) t += red[warp][w8][lane];
-            atomicAdd(sums + (size_t)warp * c + ch, (double)t);
+            atomicAdd(sums + (size_t)warp * c + ch, t);
         }
         __syncthreads();
     }
